@@ -18,6 +18,9 @@ The line also carries `large_scene`: BASELINE.json configs[4]'s geometry (the 10
 64 spp, run by ALL ranks (tiles interleaved, film reduced to rank 0) — the workload whose BVH cannot live in the caches,
 with its own clocks, roofline (algorithmic bytes next to the ncu-measured DRAM / L2 bytes per launch) and per-rank busy
 times. Films are checked against stored digests (tests/golden/bench_film_digests.json) outside the timed regions.
+
+`--dump-outputs DIR` writes the headline leg's film and counters of its last timed step as DIR/*.npy (dump_outputs()): the
+inputs are fixed, so two builds' dumps of the same command can be compared output for output.
 """
 import argparse
 import json
@@ -281,6 +284,28 @@ def check_digest(key, digest, update):
     return "ok"
 
 
+DUMP_COUNTERS = ("ray_count", "shadow_rays", "samples", "closest_nodes", "closest_tris", "any_nodes", "any_tris")
+DUMP_LIMIT = 64 << 20    # bytes, all files of one --dump-outputs together
+DUMP_SAMPLE_PIXELS = 1 << 20
+
+
+def dump_outputs(directory, film, counters):
+    """--dump-outputs: what the timed leg's caller receives after its last timed step, so that two builds' runs with the same
+    arguments can be compared output for output. film.npy is the (height, width, 3) float32 film; a film larger than the budget
+    (--workload c5) is replaced by film_sample.npy, the pixels at a fixed seeded choice of DUMP_SAMPLE_PIXELS flat pixel indices
+    (film_sample_index.npy). counters.npy holds the step's DUMP_COUNTERS in that order as float64 (exact below 2**53)."""
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, "counters.npy"), np.asarray(counters, np.float64))
+    film = np.asarray(film, np.float32)
+    if film.nbytes <= DUMP_LIMIT // 2:
+        np.save(os.path.join(directory, "film.npy"), film)
+        return
+    pixels = film.reshape(-1, 3)
+    idx = np.sort(np.random.default_rng(0).choice(len(pixels), DUMP_SAMPLE_PIXELS, replace=False))
+    np.save(os.path.join(directory, "film_sample.npy"), pixels[idx])
+    np.save(os.path.join(directory, "film_sample_index.npy"), idx.astype(np.float64))
+
+
 def shared_host_scene(api, scene, world, local, tag, big):
     """One host BVH build per node: local rank 0 builds and (for the 10 M-triangle scene, `big`) leaves the flattened arrays under
     /dev/shm; the other ranks map them (api.HostScene.save / load) instead of repeating the 6 s build N times on contended cores.
@@ -515,6 +540,12 @@ def run_ours(args):
             dist.all_reduce(counts, op=dist.ReduceOp.SUM)
         ms_total = float(ms.item())
         value = total_samples * args.steps / (ms_total / 1e3) / 1e6
+        if args.dump_outputs:  # d_film and st hold the last timed step's film and counters
+            last = torch.tensor([getattr(st, k) for k in DUMP_COUNTERS], dtype=torch.float64, device="cuda")
+            if world > 1:
+                dist.reduce(last, dst=0, op=dist.ReduceOp.SUM)
+            if rank == 0:
+                dump_outputs(args.dump_outputs, d_film.cpu().numpy().reshape(film.res[1], film.res[0], 3), last.tolist())
 
         # ---- e2e: public API with host buffers; scene upload + job upload + film read-back inside the timed region ----
         film_host = np.zeros((film.res[1], film.res[0], 3), np.float32)
@@ -656,6 +687,9 @@ def run_single_process(args):
                 rays += r.stats.ray_count; shadow += r.stats.shadow_rays; launches += r.stats.kernel_launches
             sec = time.perf_counter() - t0
             clk = clocks.stop()
+            if key == "c2" and args.dump_outputs:
+                dump_outputs(args.dump_outputs, d_film.cpu().numpy().reshape(film.res[1], film.res[0], 3),
+                             [getattr(r.stats, k) for k in DUMP_COUNTERS])
             film_host = np.zeros((film.res[1], film.res[0], 3), np.float32)
             e2e_steps = max(1, min(steps, 2))
             for k in range(e2e_steps + 1):  # the first pass warms up (pinned staging buffers of the upload, first touch of film_host)
@@ -696,7 +730,12 @@ def main():
     ap.add_argument("--write-digests", action="store_true", help="store the films' digests in tests/golden/bench_film_digests.json instead of checking them")
     ap.add_argument("--workload", default="c2", choices=["c2", "c5"], help="c2 = BASELINE.json configs[1] (default, the contract's line); c5 = configs[4]")
     ap.add_argument("--spp-side", type=int, default=0, help="override the stratified grid side (spp = side^2); the line's config says so")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the film and counters of the last timed step as DIR/*.npy (GPU arms)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU arm's outputs; the reference arm renders a sample of the tiles")
     global _REAL_STDOUT
     sys.stdout.flush()
     _REAL_STDOUT = os.dup(1)

@@ -187,8 +187,10 @@ inline RadianceResult path_li(const RenderCtx& c, Ray ray, Sampler& sampler, int
             break;
         }
         if (bounces > 3) {  // :163-169 Russian roulette
+            // Deviation: q == 1 (beta.g == 0) breaks even when the stratified draw rounds up to exactly 1.0f, where the
+            // reference goes on with beta * 1 / 0 and returns NaN for the pixel. The draw is still taken.
             float q = fmax_(1.0f - beta.g, 0.05f);
-            if (sampler.get_1d() < q) break;
+            if (sampler.get_1d() < q || q >= 1.0f) break;
             beta *= spec1(1.0f) / (1.0f - q);
         }
         bounces += 1;

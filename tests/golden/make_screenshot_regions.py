@@ -1,6 +1,6 @@
-"""Generates tests/golden/reference_screenshot_regions.json from the reference's only published render,
-/root/reference/screenshot.png (embedded by readme.md:3) — run in the build container, where /root/reference exists; the GPU
-box only sees the committed JSON. No pixels are copied: the fixture holds the mean colour of a few flat regions, two floor
+"""Generates tests/golden/reference_screenshot_regions.json from the reference's only published render, screenshot.png of a
+yuki checkout (embedded by readme.md:3): python tests/golden/make_screenshot_regions.py <yuki>/screenshot.png. The tests only
+read the committed JSON. No pixels are copied: the fixture holds the mean colour of a few flat regions, two floor
 profiles, the box opening's edges and the light quad's bounding box, i.e. measurements of the picture.
 
 What the screenshot shows (every setting is visible in its UI panel; window client area = 1920 x 1080 at (1, 38), so the film
@@ -15,7 +15,6 @@ import sys
 import numpy as np
 from PIL import Image
 
-SRC = "/root/reference/screenshot.png"
 OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "reference_screenshot_regions.json")
 CLIENT_X, CLIENT_Y, W, H = 1, 38, 1920, 1080
 
@@ -35,11 +34,11 @@ REGIONS = {
 }
 
 
-def main():
-    im = np.array(Image.open(SRC).convert("RGB")).astype(np.float64)
+def main(src):
+    im = np.array(Image.open(src).convert("RGB")).astype(np.float64)
     assert im.shape == (1119, 1922, 3), im.shape
     film = im[CLIENT_Y:CLIENT_Y + H, CLIENT_X:CLIENT_X + W]
-    out = {"source": "/root/reference/screenshot.png (readme.md:3)", "film": [W, H], "client_origin": [CLIENT_X, CLIENT_Y],
+    out = {"source": "screenshot.png (readme.md:3)", "film": [W, H], "client_origin": [CLIENT_X, CLIENT_Y],
            "settings": {"scene": "Scene::cornell()", "shapes": 37, "camera_position": [0.278, 0.273, 0.8], "camera_target": [0.278, 0.273, -0.26],
                         "fov_x_deg": 64.0, "tile_dim": 32, "sampler": "stratified 32x32 jittered", "integrator": "path", "max_depth": 10,
                         "indirect_clamp": 2.0, "tone_map": "filmic", "exposure": 1.0},
@@ -71,4 +70,4 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    main(sys.argv[1])

@@ -63,3 +63,30 @@ def test_reference_arm_prints_the_drivers_line():
     assert line["cpu_baseline"]["kind"] == "port" and line["cpu_baseline"]["cores"] >= 1 and line["cpu_baseline"]["value"] == line["value"] > 0
     assert line["e2e"] == {"value": line["value"], "unit": "Msamples/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     assert np.isfinite(line["ms_per_step"])
+
+
+def test_dump_outputs_fit_the_budget_and_sample_the_same_pixels_every_run(tmp_path):
+    """--dump-outputs: the 1024x1024 film is written whole; a 3840x2160 film (--workload c5) is replaced by the same seeded pixel
+    sample on every run, and one dump's files stay within the 64 MB budget."""
+    counters = [3.5e9, 1e9, 2 ** 30, 5, 6, 7, 8]
+    small = np.random.default_rng(1).random((1024, 1024, 3), dtype=np.float32)
+    bench.dump_outputs(str(tmp_path / "small"), small, counters)
+    assert np.array_equal(np.load(tmp_path / "small" / "film.npy"), small)
+    got = np.load(tmp_path / "small" / "counters.npy")
+    assert got.dtype == np.float64 and got.tolist() == counters
+    big = np.random.default_rng(2).random((2160, 3840, 3), dtype=np.float32)
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), big, counters)
+        files = sorted(os.listdir(tmp_path / run))
+        assert files == ["counters.npy", "film_sample.npy", "film_sample_index.npy"]
+        assert sum(os.path.getsize(tmp_path / run / f) for f in files) <= bench.DUMP_LIMIT
+    idx = np.load(tmp_path / "a" / "film_sample_index.npy")
+    assert np.array_equal(idx, np.load(tmp_path / "b" / "film_sample_index.npy"))
+    assert np.array_equal(np.load(tmp_path / "a" / "film_sample.npy"), big.reshape(-1, 3)[idx.astype(np.int64)])
+
+
+def test_bench_refuses_zero_steps_and_a_reference_dump(tmp_path):
+    for extra, msg in ((["--steps", "0"], "--steps must be at least 1"),
+                       (["--impl", "reference", "--dump-outputs", str(tmp_path)], "the reference arm renders a sample of the tiles")):
+        p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *extra], capture_output=True, text=True, cwd=ROOT, timeout=600)
+        assert p.returncode == 2 and msg in p.stderr, p.stderr

@@ -174,6 +174,18 @@ def test_gpu_matches_committed_golden_fixtures(gpu_ctx, xf):
         assert hashlib.sha256(r.film.tobytes()).hexdigest() == g["film_sha256"], name
 
 
+def test_roulette_with_zero_continuation_probability_matches_the_oracle(gpu_ctx, oracle, xf):
+    """The two benchmark samples whose roulette draw is exactly 1.0f at q == 1 (test_oracle_render.py): finite and bit-identical."""
+    from test_oracle_render import roulette_draw_of_one_case
+    scene, cam, film, smp, integ, tiles = roulette_draw_of_one_case(xf)
+    dev = api.Scene(gpu_ctx, scene)
+    r = api.Renderer(gpu_ctx).render(dev, cam, film, smp, integ, tiles=tiles)
+    dev.close()
+    o_img, _, o_st = oracle.OracleScene(scene).render(cam, film, smp, integ, tiles=tiles)
+    assert np.isfinite(r.film).all() and np.array_equal(r.film.view(np.uint32), o_img.view(np.uint32))
+    assert r.stats.ray_count == o_st.ray_count
+
+
 def test_path_is_bit_identical_to_the_oracle(gpu_ctx, oracle, xf):
     """Stronger than the RMSE gate: with un-fused IEEE arithmetic and glibc-exact sinf/cosf the Path film has no
     differing bit, for every material and light kind."""

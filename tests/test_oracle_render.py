@@ -34,6 +34,20 @@ def golden_cases(xf):
     }
 
 
+def roulette_draw_of_one_case(xf):
+    """Two samples of the benchmark render (Cornell box 1024x1024, Path 8, stratified 32x32) whose paths lose their green
+    throughput on the red wall, so that Russian roulette's q is 1 at the fifth vertex, and whose roulette draw rounds up to
+    exactly 1.0f: an accumulating one-pixel tile each. Found by rendering every sample of the pixels that were NaN in the
+    benchmark film one at a time. Returns (scene, camera, film, sampler, integrator, tiles)."""
+    from yuki_b200 import capi
+    scene, cam = scenes.cornell(xf, light="rect", tall_box="glass")
+    tiles = np.zeros(2, capi.TILE_DTYPE)
+    tiles[0] = (448, 246, 449, 247, 265, 0, 0)
+    tiles[1] = (630, 673, 631, 674, 424, 0, 1)
+    return (scene, cam, D.FilmSettings((1024, 1024), 16, accumulate=True), D.SamplerType.stratified(32, 32, jitter=True),
+            D.IntegratorType.path(8), tiles)
+
+
 def digest(img, ids, st):
     return {"film_sha256": hashlib.sha256(np.ascontiguousarray(img).tobytes()).hexdigest(),
             "ids_sha256": hashlib.sha256(np.ascontiguousarray(ids).tobytes()).hexdigest(),
@@ -101,3 +115,17 @@ def test_ray_counts(oracle, xf):
     assert st.ray_count == 16 * 16 * 2 and st.samples == 16 * 16 * 2
     _, _, st = osc.render(cam, D.FilmSettings((16, 16), 16), D.SamplerType.uniform(2), D.IntegratorType.path(0))
     assert st.ray_count == 0
+
+
+def test_roulette_ends_a_path_whose_continuation_probability_is_zero(oracle, xf):
+    """q == 1 ends the path whatever the draw: a draw of exactly 1.0f used to go on with beta * 1 / 0 and make the pixel NaN."""
+    scene, cam, film, smp, integ, tiles = roulette_draw_of_one_case(xf)
+    # draws up to the first roulette: the camera jitter, then per vertex one get_2d per light (one light) and the BSDF's
+    # get_2d, five vertices (bounces 0..4), then roulette's get_1d
+    assert len(scene.lights) == 1
+    for t in tiles:
+        draws = oracle.sampler_draws(smp, int(t["x0"]), int(t["y0"]), int(t["sample"]), [2] + [2, 2] * 5 + [1])
+        assert draws[-1] == np.float32(1.0)
+    img, _, st = oracle.OracleScene(scene).render(cam, film, smp, integ, tiles=tiles)
+    px = img[tiles["y0"], tiles["x0"]]
+    assert st.samples == 2 and np.isfinite(px).all() and (px >= 0).all()

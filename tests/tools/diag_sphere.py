@@ -1,4 +1,6 @@
-import sys; sys.path.insert(0,'/root/repo'); sys.path.insert(0,'/root/repo/tests')
+import os, sys
+TESTS = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, os.path.dirname(TESTS)); sys.path.insert(0, TESTS)
 import numpy as np
 from yuki_b200 import api, desc as D, scenes, transforms as xf
 from oracle import oracle as O

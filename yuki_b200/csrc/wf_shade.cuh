@@ -428,8 +428,10 @@ __device__ __forceinline__ void shade_item(const DevScene& sc, const Wave& w, co
             beta = beta * (s.f * fabsf(dotn(s.wi, si.sh_n)) / s.pdf);
             const Ray nr = spawn_ray(si.p, si.n, s.wi);
             if (depth > 3) {  // Russian roulette, path.rs:163-169
+                // q == 1 (beta.g == 0) ends the path even when the stratified draw rounds up to exactly 1.0f: path.rs would go on
+                // with beta * 1 / 0 and turn the pixel into NaN. The draw is still taken, as in the oracle.
                 const float q = fmaxf(1.0f - beta.g, 0.05f);
-                if (smp.get_1d(cfg.sampler) < q) alive = false;
+                if (smp.get_1d(cfg.sampler) < q || q >= 1.0f) alive = false;
                 else beta = beta * (gray(1.0f) / (1.0f - q));
             }
             const uint32_t bounces = depth + 1;
