@@ -7,6 +7,7 @@ source prescribes, the GPU tests compare `yk_debug_ray` with the oracle bit for 
 import numpy as np
 import pytest
 
+from test_render_limits import white_box
 from yuki_b200 import api, capi, desc as D, scenes
 
 DIRECT, REFLECTION, REFRACTION, NORMAL, SHADOW = range(5)
@@ -19,6 +20,9 @@ def _cases(xf):
     room = scenes.material_room(xf)
     point = scenes.cornell(xf, light="point")
     return [
+        # the deepest settings yk_render admits: Path's bounce counter full, Whitted's largest tree depth
+        ("white-box-path-255", *white_box(xf), D.SamplerType.uniform(8), D.IntegratorType.path(255)),
+        ("cornell-whitted-24", *cornell, D.SamplerType.stratified(2, 2), D.IntegratorType.whitted(24)),
         ("cornell-path", *cornell, D.SamplerType.stratified(4, 4), D.IntegratorType.path(8)),
         ("cornell-path-uniform", *cornell, D.SamplerType.uniform(16), D.IntegratorType.path(6)),
         ("room-path", *room, D.SamplerType.stratified(3, 3), D.IntegratorType.path(8)),

@@ -165,7 +165,9 @@ struct Wave {
     struct Stream {
         float4* ray_o;   // o.xyz, t_max
         float4* ray_d;   // d.xyz, -
-        float4* beta;    // throughput (path; 1 for whitted); w = flags | sampler dimension << kDimShift
+        // path: throughput, w = flags | sampler dimension << kDimShift. whitted: x = sampler dimension (uint bits), y, z = 1,
+        // w = flags: a Whitted sample draws 2 * lights dimensions per tree node, and its trees outgrow the 21 bits of w
+        float4* beta;
         unsigned long long* rng;
     } st[2];
     uint2* hit;         // per queue slot: t bits, shape slot (kMiss = none)
@@ -202,7 +204,7 @@ constexpr uint32_t kFlagSpecular = 0x100u;   // path: specular_bounce / whitted:
 constexpr uint32_t kFlagAlive = 0x200u;
 constexpr uint32_t kFlagTransmission = 0x400u;  // the ray left a TRANSMISSION lobe (ray type of li_debug, path.rs:146-153)
 constexpr uint32_t kDepthMask = 0xffu;       // path: bounces / whitted: depth
-constexpr uint32_t kDimShift = 11;           // sampler dimension (stratified.rs:40) in the upper 21 bits
+constexpr uint32_t kDimShift = 11;           // path: sampler dimension (stratified.rs:40) in the upper 21 bits
 constexpr uint32_t kFlagMask = (1u << kDimShift) - 1u;
 
 // Ray list of Integrator::li_debug (integrators/mod.rs:76-118), filled by k_debug_log for the one path of yk_debug_ray.

@@ -96,7 +96,8 @@ __global__ void k_raygen(Wave w, RenderCfg cfg, Batch bt, uint32_t first_sample,
     st_once(&w.st[0].ray_o[i], make_float4(o.x, o.y, o.z, __int_as_float(0x7f800000)));
     st_once(&w.st[0].ray_d[i], make_float4(d.x, d.y, d.z, 0.0f));
     st_once(&w.st[0].rng[i], (unsigned long long)s.rng.state);
-    st_once(&w.st[0].beta[i], make_float4(1.0f, 1.0f, 1.0f, __uint_as_float(kFlagAlive | (s.dim << kDimShift))));
+    if (cfg.integrator == YK_INTEGRATOR_WHITTED) st_once(&w.st[0].beta[i], make_float4(__uint_as_float(s.dim), 1.0f, 1.0f, __uint_as_float(kFlagAlive)));
+    else st_once(&w.st[0].beta[i], make_float4(1.0f, 1.0f, 1.0f, __uint_as_float(kFlagAlive | (s.dim << kDimShift))));
     st_once(&w.L[i], make_float4(0.0f, 0.0f, 0.0f, 0.0f));
 }
 

@@ -55,7 +55,7 @@ __device__ __forceinline__ bool tree_return(const Wave& w, uint32_t path, uint32
 __device__ __forceinline__ void stream_node(const Wave::Stream& st, uint32_t pos, const TreeRay& e, uint32_t dim, unsigned long long rng) {
     st.ray_o[pos] = make_float4(e.o.x, e.o.y, e.o.z, __int_as_float(0x7f800000));
     st.ray_d[pos] = make_float4(e.d.x, e.d.y, e.d.z, 0.0f);
-    st.beta[pos] = make_float4(1.0f, 1.0f, 1.0f, __uint_as_float(e.flags | kFlagAlive | (dim << kDimShift)));
+    st.beta[pos] = make_float4(__uint_as_float(dim), 1.0f, 1.0f, __uint_as_float(e.flags | kFlagAlive));
     st.rng[pos] = rng;
 }
 
@@ -98,7 +98,7 @@ __global__ void k_classify(DevScene sc, Wave w, RenderCfg cfg, Batch bt, const u
             } else if (first_iteration != 2) {  // (2 = debug integrators: their li() returns no background)
                 const float4 bw = w.st[b].beta[i];
                 if (WHITTED) {  // whitted.rs:174: this node's radiance is the background
-                    node_dim[WHITTED ? k : 0] = __float_as_uint(bw.w) >> kDimShift;
+                    node_dim[WHITTED ? k : 0] = __float_as_uint(bw.x);
                     const uint32_t depth = __float_as_uint(bw.w) & kDepthMask;
                     if (tree_return(w, path[k], depth, rgb(sc.background[0], sc.background[1], sc.background[2]), &node[WHITTED ? k : 0])) key[k] = 4;
                 } else {  // path.rs:155-160: background weighted by the throughput
@@ -375,7 +375,7 @@ __device__ __forceinline__ void shade_item(const DevScene& sc, const Wave& w, co
     SamplerState smp;
     smp.rng.state = ld_once(&w.st[b].rng[slot]);
     smp.rng.inc = job.rng_inc;
-    smp.dim = __float_as_uint(beta4.w) >> kDimShift;
+    smp.dim = PATH ? __float_as_uint(beta4.w) >> kDimShift : __float_as_uint(beta4.x);
     smp.px = job.x;
     smp.py = job.y;
     smp.index = job.sample_begin + bt.sample_off + sample_i;
@@ -482,7 +482,7 @@ __device__ __forceinline__ void shade_item(const DevScene& sc, const Wave& w, co
             const TreeRay& e = child[0];
             out->nx_o = make_float4(e.o.x, e.o.y, e.o.z, __int_as_float(0x7f800000));
             out->nx_d = make_float4(e.d.x, e.d.y, e.d.z, 0.0f);
-            out->nx_beta = make_float4(1.0f, 1.0f, 1.0f, __uint_as_float(e.flags | kFlagAlive | (smp.dim << kDimShift)));
+            out->nx_beta = make_float4(__uint_as_float(smp.dim), 1.0f, 1.0f, __uint_as_float(e.flags | kFlagAlive));
         } else {
             w.tree_rng[g] = smp.rng.state;  // the sampler goes on with whichever node the tree visits next
         }
@@ -609,7 +609,7 @@ __global__ void k_debug_log(DevScene sc, Wave w, RenderCfg cfg, Batch bt, int b,
     SamplerState smp;
     smp.rng.state = w.st[b].rng[0];
     smp.rng.inc = job.rng_inc;
-    smp.dim = word >> kDimShift;
+    smp.dim = cfg.integrator == YK_INTEGRATOR_WHITTED ? __float_as_uint(beta4.x) : word >> kDimShift;
     smp.px = job.x;
     smp.py = job.y;
     smp.index = job.sample_begin + bt.sample_off;
