@@ -260,6 +260,39 @@ int yk_trace(yk_context*, const yk_scene*, const float* o_xyz, const float* d_xy
  * o -> o + d (d unnormalised, cut at t_max = 0.9999 as interaction.rs:57-58 spawns every shadow ray):
  * occluded_out[i] = 1 when anything lies in between. */
 int yk_occluded(yk_context*, const yk_scene*, const float* o_xyz, const float* d_xyz, uint32_t n, uint8_t* occluded_out);
+/* Ray queries with the hit's surface (Scene::intersect's Hit { t, si, shape }), on host or device-resident arrays.
+ * Host arrays (opts NULL or flags 0) are staged through the context's buffers like yk_trace. With YK_QUERY_ON_DEVICE the
+ * rays and every output are device memory (cudaMalloc'd or managed) of the context's GPU, 4-byte aligned: the call reads and
+ * writes them in place, starts its device work after the work already queued on opts->stream and returns when its outputs
+ * are written. Buffer sizes are the caller's contract. A NaN t_max is refused (YK_ERR_INVALID); on the device path this is
+ * found by the kernel that reads t_max, and the outputs are then unspecified. */
+#define YK_QUERY_ON_DEVICE 1u   /* rays and every output array are device memory of the context's GPU */
+typedef struct {
+    uint32_t flags;             /* YK_QUERY_ON_DEVICE or 0 (host arrays) */
+    uint32_t _reserved;         /* must be 0 */
+    void* stream;               /* ON_DEVICE: the caller's cudaStream_t (NULL = legacy default stream). The call's device
+                                   work starts after the work already queued on it; the call returns when its outputs are
+                                   written (blocking, like yk_render). Ignored for host arrays. */
+} yk_query_opts;
+typedef struct {                /* each array optional: NULL = not produced */
+    float* t;                   /* n: hit distance, inf on a miss */
+    int32_t* orig_id;           /* n: original shape id, -1 on a miss */
+    uint32_t* counts;           /* 2n: (intersection_test_count, intersection_count), bvh.rs:177-179 */
+    int32_t* material;          /* n: material index of the hit shape, -1 on a miss */
+    int32_t* area_light;        /* n: SurfaceInteraction::area_light, -1 for none or a miss */
+    float* p;                   /* 3n: SurfaceInteraction::p */
+    float* n;                   /* 3n: geometric normal (after set_shading_geometry's faceforward) */
+    float* uv;                  /* 2n */
+    float* shading_n;           /* 3n: shading.n */
+    float* shading_dpdu;        /* 3n: shading.dpdu (what Bsdf::new normalises into its frame's s) */
+} yk_hits;                      /* on a miss p, n, uv, shading_n and shading_dpdu are 0 */
+/* BoundingVolumeHierarchy::intersect (bvh.rs:160-232) for n rays (t_max NULL = infinity), writing the requested fields of
+ * `out`. The geometric dpdu / dpdv and shading.dpdv are not produced. */
+int yk_query_intersect(yk_context*, const yk_scene*, const float* o_xyz, const float* d_xyz, const float* t_max,
+                       uint32_t n, const yk_query_opts* opts /* NULL = host arrays */, const yk_hits* out);
+/* yk_occluded's semantics (segments o -> o + d, cut at 0.9999, no target light) with yk_query_intersect's options. */
+int yk_query_occluded(yk_context*, const yk_scene*, const float* o_xyz, const float* d_xyz, uint32_t n,
+                      const yk_query_opts* opts, uint8_t* occluded_out);
 /* Sampler::{start_pixel_sample(p, index, 0), get_1d, get_2d} (sampling/mod.rs:46-57, uniform.rs:72-94, stratified.rs:90-143)
  * on the device, for n (pixel x, pixel y, sample index) triples: every triple starts a sampler the way Integrator::render
  * does (integrators/mod.rs:163) and performs the draws of `pattern` (1 = get_1d: one float, 2 = get_2d: two floats);

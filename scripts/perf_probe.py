@@ -96,18 +96,32 @@ if which == "jitter_hf4":
         t0 = time.time()
         r = rn.render(dev, c, D.FilmSettings((1920, 1080), 16), D.SamplerType.stratified(2, 2), D.IntegratorType.path(8))
         print(f"rep {i}: device {r.stats.device_ms:.1f} ms wall {1e3*(time.time()-t0):.1f} ms closest {r.stats.trace_closest_ms:.1f} any {r.stats.trace_any_ms:.1f} shade {r.stats.shade_ms:.1f} launches {r.stats.kernel_launches}", flush=True)
-if which == "query":  # yk_trace / yk_occluded through the ABI with host arrays (copies included): incoherent rays on the 1 M-triangle mesh
+if which == "query":  # the ray-query ABI on 8 Mi incoherent rays on the 1 M-triangle mesh: host arrays (copies included), then device arrays
+    import subprocess
+    print(subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv"], capture_output=True, text=True).stdout.strip(), flush=True)
     s, c = scenes.heightfield(xf, 708, 708)
     ctx = api.Context(0); dev = api.Scene(ctx, s)
     rng = np.random.default_rng(1)
     n = 1 << 23
     o = rng.uniform((-0.7, -0.4, -0.7), (0.7, 0.6, 0.7), (n, 3)).astype(np.float32)
     d = (rng.uniform((-0.7, -0.4, -0.7), (0.7, 0.6, 0.7), (n, 3)).astype(np.float32) - o)
-    for name, fn in (("yk_trace", lambda: dev.intersect(o, d)), ("yk_trace (no counters)", lambda: dev.intersect(o, d, counts=False)), ("yk_occluded", lambda: dev.occluded(o, d))):
+    def best_of(name, fn, where):  # host clock around the blocking call, best of 4 after a warm-up call
+        fn()
         best = 1e9
         for i in range(4):
             t0 = time.perf_counter(); r = fn(); best = min(best, time.perf_counter() - t0)
-        print(f"{name}: {n / best / 1e6:.1f} Mrays/s end to end ({n} incoherent rays, host arrays in and out)", flush=True)
+        print(f"{name}: {n / best / 1e6:.1f} Mrays/s end to end ({n} incoherent rays, {where}), {1e3 * best:.1f} ms", flush=True)
+    host = "host arrays in and out"
+    for name, fn in (("yk_trace", lambda: dev.intersect(o, d)), ("yk_trace (no counters)", lambda: dev.intersect(o, d, counts=False)), ("yk_occluded", lambda: dev.occluded(o, d)),
+                     ("yk_query_intersect surface", lambda: dev.surface(o, d))):
+        best_of(name, fn, host)
+    import torch
+    to, td = torch.from_numpy(o).cuda(), torch.from_numpy(d).cuda()
+    torch.cuda.synchronize()
+    dv = "torch CUDA tensors in and out"
+    for name, fn in (("yk_query_intersect t + id + counts", lambda: dev.intersect(to, td)), ("yk_query_intersect t + id", lambda: dev.intersect(to, td, counts=False)),
+                     ("yk_query_intersect surface", lambda: dev.surface(to, td)), ("yk_query_occluded", lambda: dev.occluded(to, td))):
+        best_of(name + " (device)", fn, dv)
     dev.close(); ctx.close()
 if which == "whitted":  # config 1 (Cornell 512^2, Whitted depth 3, 16 spp) and a deeper tree
     s, c = scenes.cornell(xf, light="point", tall_box="glass")

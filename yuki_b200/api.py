@@ -167,6 +167,68 @@ class HostScene:
             pass
 
 
+HIT_FIELDS = ("t", "orig_id", "material", "area_light", "p", "n", "uv", "shading_n", "shading_dpdu")
+_HIT_SHAPES = {"t": ((), np.float32), "orig_id": ((), np.int32), "material": ((), np.int32), "area_light": ((), np.int32),
+               "p": ((3,), np.float32), "n": ((3,), np.float32), "uv": ((2,), np.float32), "shading_n": ((3,), np.float32),
+               "shading_dpdu": ((3,), np.float32)}
+
+
+@dataclass
+class Hits:
+    """`Scene::intersect`'s Hit for a batch of rays (numpy arrays, or torch tensors on the GPU when the rays were): hit distance
+    (inf on a miss), original shape id and material index (-1 on a miss), and the SurfaceInteraction's area light (-1 for
+    none), p, geometric normal n, uv, shading normal and shading dpdu (0 on a miss)."""
+    t: object
+    orig_id: object
+    material: object
+    area_light: object
+    p: object
+    n: object
+    uv: object
+    shading_n: object
+    shading_dpdu: object
+
+
+def _cuda_rays(ctx, arrays):
+    """The torch module when any of `arrays` is a CUDA tensor (then all must be float32 CUDA tensors on the context's device),
+    else None: host input keeps the numpy path. torch is only imported by callers that already hold tensors."""
+    import sys
+    torch = sys.modules.get("torch")
+    if torch is None:
+        return None
+    given = [a for a in arrays if a is not None]
+    if not any(isinstance(a, torch.Tensor) and a.is_cuda for a in given):
+        return None
+    for a in given:
+        if not (isinstance(a, torch.Tensor) and a.is_cuda):
+            raise TypeError(f"rays mix CUDA tensors with {type(a).__name__} ({getattr(a, 'device', 'host')}): pass o, d and t_max "
+                            "all as CUDA tensors or all as host arrays")
+        if a.dtype != torch.float32:
+            raise TypeError(f"ray tensors must be float32, got {a.dtype}")
+        if a.device.index != ctx.device_id:
+            raise ValueError(f"ray tensor on {a.device}, but the scene's context is on cuda:{ctx.device_id}")
+    return torch
+
+
+def _device_rays(torch, o, d, t_max):
+    if o.dim() != 2 or o.shape[1] != 3 or d.shape != o.shape:
+        raise ValueError(f"o and d must have shape (n, 3), got {tuple(o.shape)} and {tuple(d.shape)}")
+    n = o.shape[0]
+    if t_max is not None and tuple(t_max.shape) != (n,):
+        raise ValueError(f"t_max must have shape ({n},), got {tuple(t_max.shape)}")
+    return o.contiguous(), d.contiguous(), None if t_max is None else t_max.contiguous(), n
+
+
+def _device_opts(torch, ctx):
+    return capi.QueryOpts(capi.QUERY_ON_DEVICE, 0, torch.cuda.current_stream(ctx.device_id).cuda_stream)
+
+
+def _ptr(a):
+    if a is None:
+        return None
+    return a.data_ptr() if hasattr(a, "data_ptr") else a.ctypes.data
+
+
 class Scene:
     """Device-resident scene (`yk_scene`): SoA node / triangle / material / light / texture buffers in HBM."""
 
@@ -178,7 +240,19 @@ class Scene:
 
     def intersect(self, o, d, t_max=None, counts: bool = True):
         """`BoundingVolumeHierarchy::intersect` (bvh.rs:160-232) for a batch of rays: (t, original shape id, (tests, hits)
-        node counters); t = inf and id = -1 on a miss."""
+        node counters); t = inf and id = -1 on a miss. Rays held as float32 CUDA tensors on the context's device are traced
+        in place, ordered after the current torch stream's work, and the results are tensors on that device."""
+        torch = _cuda_rays(self.ctx, (o, d, t_max))
+        if torch is not None:
+            o, d, t_max, n = _device_rays(torch, o, d, t_max)
+            dev = o.device
+            t = torch.empty(n, dtype=torch.float32, device=dev)
+            ids = torch.empty(n, dtype=torch.int32, device=dev)
+            cnt = (torch.empty if counts else torch.zeros)((n, 2), dtype=torch.int32, device=dev).view(torch.uint32)
+            hits = capi.Hits(t=_ptr(t), orig_id=_ptr(ids), counts=_ptr(cnt) if counts else None)
+            capi.check(capi.lib().yk_query_intersect(self.ctx._h, self._h, _ptr(o), _ptr(d), _ptr(t_max), n,
+                                                     C.byref(_device_opts(torch, self.ctx)), C.byref(hits)))
+            return t, ids, cnt
         o = np.ascontiguousarray(o, np.float32).reshape(-1, 3)
         d = np.ascontiguousarray(d, np.float32).reshape(-1, 3)
         n = o.shape[0]
@@ -196,7 +270,15 @@ class Scene:
         return t, ids, cnt
 
     def occluded(self, o, d):
-        """`VisibilityTester::unoccluded` negated (visibility.rs:6-23) for a batch of segments o -> o + d."""
+        """`VisibilityTester::unoccluded` negated (visibility.rs:6-23) for a batch of segments o -> o + d (numpy, or CUDA
+        tensors as in `intersect`)."""
+        torch = _cuda_rays(self.ctx, (o, d))
+        if torch is not None:
+            o, d, _, n = _device_rays(torch, o, d, None)
+            out = torch.empty(n, dtype=torch.uint8, device=o.device)
+            capi.check(capi.lib().yk_query_occluded(self.ctx._h, self._h, _ptr(o), _ptr(d), n, C.byref(_device_opts(torch, self.ctx)),
+                                                    _ptr(out)))
+            return out
         o = np.ascontiguousarray(o, np.float32).reshape(-1, 3)
         d = np.ascontiguousarray(d, np.float32).reshape(-1, 3)
         n = o.shape[0]
@@ -204,6 +286,30 @@ class Scene:
         out = np.zeros(n, np.uint8)
         capi.check(capi.lib().yk_occluded(self.ctx._h, self._h, capi.fptr(o), capi.fptr(d), n, out.ctypes.data))
         return out
+
+    def surface(self, o, d, t_max=None) -> Hits:
+        """`Scene::intersect` (scene/mod.rs) for a batch of rays: the hit with its SurfaceInteraction, as a `Hits` record of
+        numpy arrays, or of tensors on the GPU when the rays are CUDA tensors (see `intersect`)."""
+        torch = _cuda_rays(self.ctx, (o, d, t_max))
+        if torch is not None:
+            o, d, t_max, n = _device_rays(torch, o, d, t_max)
+            out = {k: torch.empty((n,) + shape, dtype=getattr(torch, np.dtype(dt).name), device=o.device) for k, (shape, dt) in _HIT_SHAPES.items()}
+            opts = C.byref(_device_opts(torch, self.ctx))
+        else:
+            o = np.ascontiguousarray(o, np.float32).reshape(-1, 3)
+            d = np.ascontiguousarray(d, np.float32).reshape(-1, 3)
+            n = o.shape[0]
+            if d.shape[0] != n:
+                raise ValueError(f"o and d must have the same number of rays, got {n} and {d.shape[0]}")
+            if t_max is not None:
+                t_max = np.ascontiguousarray(t_max, np.float32).reshape(-1)
+                if t_max.shape[0] != n:
+                    raise ValueError(f"t_max must have {n} entries, got {t_max.shape[0]}")
+            out = {k: np.zeros((n,) + shape, dt) for k, (shape, dt) in _HIT_SHAPES.items()}
+            opts = None
+        hits = capi.Hits(**{k: _ptr(v) for k, v in out.items()})
+        capi.check(capi.lib().yk_query_intersect(self.ctx._h, self._h, _ptr(o), _ptr(d), _ptr(t_max), n, opts, C.byref(hits)))
+        return Hits(**out)
 
     def close(self):
         if self._h:

@@ -157,6 +157,18 @@ class Stats(C.Structure):
 
 
 RENDER_FILM_ON_DEVICE = 1
+QUERY_ON_DEVICE = 1
+
+
+class QueryOpts(C.Structure):
+    _fields_ = [("flags", C.c_uint32), ("_reserved", C.c_uint32), ("stream", C.c_void_p)]
+
+
+class Hits(C.Structure):
+    """yk_hits: output pointers of yk_query_intersect (NULL = not produced)."""
+    _fields_ = [("t", C.c_void_p), ("orig_id", C.c_void_p), ("counts", C.c_void_p), ("material", C.c_void_p),
+                ("area_light", C.c_void_p), ("p", C.c_void_p), ("n", C.c_void_p), ("uv", C.c_void_p), ("shading_n", C.c_void_p),
+                ("shading_dpdu", C.c_void_p)]
 
 # Every symbol include/yuki_gpu.h declares (checked by tests/test_abi.py).
 EXPORTS = [
@@ -164,7 +176,7 @@ EXPORTS = [
     "yk_context_stream", "yk_bvh_build", "yk_host_scene_build", "yk_host_scene_destroy", "yk_host_scene_flat", "yk_camera_make",
     "yk_film_tiles", "yk_xf_identity", "yk_xf_translation", "yk_xf_scale", "yk_xf_rotation", "yk_xf_new", "yk_xf_look_at",
     "yk_xf_mul", "yk_xf_inverted", "yk_xf_point", "yk_xf_vec", "yk_xf_normal", "yk_light_make", "yk_selftest_fastdiv", "yk_ply_load", "yk_ply_view", "yk_ply_destroy", "yk_write_exr", "yk_tonemap_filmic", "yk_heatmap", "yk_pbrt_load", "yk_pbrt_view", "yk_pbrt_destroy", "yk_mitsuba_load",
-    "yk_debug_ray", "yk_trace", "yk_occluded", "yk_sampler_draws",
+    "yk_debug_ray", "yk_trace", "yk_occluded", "yk_query_intersect", "yk_query_occluded", "yk_sampler_draws",
     "yk_multi_create", "yk_multi_destroy", "yk_multi_device_count", "yk_multi_context", "yk_multi_peer_stores",
     "yk_multi_scene_create", "yk_multi_scene_destroy", "yk_multi_render",
 ]
@@ -196,6 +208,8 @@ def lib():
                                C.POINTER(u32), fp, C.POINTER(C.c_uint64)]
     L.yk_trace.argtypes = [vp, vp, fp, fp, fp, u32, fp, vp, vp]
     L.yk_occluded.argtypes = [vp, vp, fp, fp, u32, vp]
+    L.yk_query_intersect.argtypes = [vp, vp, vp, vp, vp, u32, C.POINTER(QueryOpts), C.POINTER(Hits)]
+    L.yk_query_occluded.argtypes = [vp, vp, vp, vp, u32, C.POINTER(QueryOpts), vp]
     L.yk_sampler_draws.argtypes = [vp, C.POINTER(Sampler), vp, u32, C.c_char_p, u32, fp]
     L.yk_bvh_build.argtypes = [fp, u32, u32, u32, vp, C.POINTER(u32), C.POINTER(u32)]
     L.yk_host_scene_build.argtypes = [C.POINTER(HostSceneDesc), C.POINTER(vp)]

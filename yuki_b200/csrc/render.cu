@@ -27,6 +27,7 @@
 #include <string>
 #include <thread>
 #include <type_traits>
+#include <utility>
 #include <vector>
 
 #include "wf_common.cuh"
@@ -104,6 +105,12 @@ struct yk_context {
     int32_t* q_id = nullptr;
     uint32_t* q_cnt = nullptr;
     uint8_t* q_occ = nullptr;
+    std::vector<void*> query_surface_allocs;  // yk_query_intersect staging of the surface fields (host arrays), kept too
+    uint32_t query_surface_cap = 0;
+    int32_t *q_mat = nullptr, *q_al = nullptr;
+    float *q_p = nullptr, *q_n = nullptr, *q_uv = nullptr, *q_sh_n = nullptr, *q_sh_dpdu = nullptr;
+    std::vector<void*> query_flag_alloc;
+    int* q_nan = nullptr;  // device-resident rays: set by k_query_pack when a t_max is NaN
     // Ray sort between bounces (wf_sort.cuh). key: 0 = off, 1 = leaf slot of the shape the ray leaves + octant, 2 = Morton cell of
     // the origin + octant, -1 = by scene size (render_impl). order: 1 = closest-hit kernel only, 2 = material sort too.
     // Environment: YK_SORT_KEY, YK_SORT_ORDER; yk_render_opts.ray_sort overrides the key per render.
@@ -651,6 +658,8 @@ void yk_context_destroy(yk_context* c) {
         if (p.owns_stream) cudaStreamDestroy(p.stream);
     }
     free_bag(c->query_allocs);
+    free_bag(c->query_surface_allocs);
+    free_bag(c->query_flag_alloc);
     cudaFree(c->d_tiles);
     cudaFree(c->d_tile_off);
     cudaFree(c->d_accum);
@@ -1381,13 +1390,27 @@ int yk_debug_ray(yk_context* c, const yk_scene* sc, const yk_camera* cam, const 
 
 
 // ---- ray-batch queries ------------------------------------------------------------------------------------
+// yk_trace / yk_occluded / yk_query_intersect / yk_query_occluded share one chunk loop (query_run). Host arrays go through
+// the context's staging buffers, one synchronise per chunk; device arrays are read and written in place, and the host waits
+// once, at the end of the call.
 namespace {
-int query_prepare(yk_context* c, const yk_scene* sc, uint32_t n, const char* who, uint32_t* chunk) {
-    if (sc->ctx != c) return yk_set_error(YK_ERR_INVALID, std::string(who) + ": scene belongs to another context");
-    CUDA_TRY(cudaSetDevice(c->device));
-    (void)cudaGetLastError();
+struct QueryCall {
+    const char* who;
+    const float *o, *d, *t_max;
+    uint32_t n;
+    bool on_device;
+    cudaStream_t caller;    // on_device: the pipe's work starts after what is queued here
+    const yk_hits* hits;    // closest-hit query: the outputs wanted
+    uint8_t* occluded;      // any-hit query (hits == nullptr)
+};
+
+bool wants_surface(const yk_hits& h) {
+    return h.material || h.area_light || h.p || h.n || h.uv || h.shading_n || h.shading_dpdu;
+}
+
+int query_prepare(yk_context* c, const yk_scene* sc, uint32_t n, bool staged, bool staged_surface, uint32_t* chunk) {
     *chunk = std::min<uint32_t>(std::max<uint32_t>(n, 32u), 1u << 22);
-    if (c->query_cap < *chunk) {  // staging grows to the largest chunk asked for and stays
+    if (staged && c->query_cap < *chunk) {  // staging grows to the largest chunk asked for and stays
         free_bag(c->query_allocs);
         c->query_cap = 0;
         std::vector<void*>& bag = c->query_allocs;
@@ -1401,9 +1424,166 @@ int query_prepare(yk_context* c, const yk_scene* sc, uint32_t n, const char* who
         }
         c->query_cap = *chunk;
     }
+    if (staged_surface && c->query_surface_cap < *chunk) {
+        free_bag(c->query_surface_allocs);
+        c->query_surface_cap = 0;
+        std::vector<void*>& bag = c->query_surface_allocs;
+        int rc = YK_OK;
+        if ((rc = dev_alloc(bag, &c->q_mat, *chunk)) != YK_OK || (rc = dev_alloc(bag, &c->q_al, *chunk)) != YK_OK ||
+            (rc = dev_alloc(bag, &c->q_p, (size_t)3 * *chunk)) != YK_OK || (rc = dev_alloc(bag, &c->q_n, (size_t)3 * *chunk)) != YK_OK ||
+            (rc = dev_alloc(bag, &c->q_uv, (size_t)2 * *chunk)) != YK_OK || (rc = dev_alloc(bag, &c->q_sh_n, (size_t)3 * *chunk)) != YK_OK ||
+            (rc = dev_alloc(bag, &c->q_sh_dpdu, (size_t)3 * *chunk)) != YK_OK) {
+            free_bag(bag);
+            return rc;
+        }
+        c->query_surface_cap = *chunk;
+    }
+    if (!staged && !c->q_nan) {
+        int rc = dev_alloc(c->query_flag_alloc, &c->q_nan, 1);
+        if (rc != YK_OK) return rc;
+    }
     Pipe& p = c->pipe[0];
     if (p.wave_cap >= *chunk && p.wave_lights == sc->dev.n_lights) return YK_OK;  // a render's (larger) wavefront state is reused
     return ensure_wave(&p, *chunk, sc->dev.n_lights, 0);
+}
+
+// YK_QUERY_ON_DEVICE: every array must be device (or managed) memory of the context's GPU, 4-byte aligned
+int check_device_array(const yk_context* c, const void* ptr, const char* who, const char* name) {
+    if (!ptr) return YK_OK;
+    if ((uintptr_t)ptr % 4u != 0)
+        return yk_set_error(YK_ERR_INVALID, std::string(who) + ": " + name + " is not 4-byte aligned");
+    cudaPointerAttributes a{};
+    const cudaError_t e = cudaPointerGetAttributes(&a, ptr);
+    if (e != cudaSuccess) (void)cudaGetLastError();
+    if (e != cudaSuccess || (a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged) || a.device != c->device)
+        return yk_set_error(YK_ERR_INVALID, std::string(who) + ": " + name + " is not device memory of the context's GPU (device " +
+                                                std::to_string(c->device) + ") although YK_QUERY_ON_DEVICE is set");
+    return YK_OK;
+}
+
+int query_run(yk_context* c, const yk_scene* sc, const QueryCall& q) {
+    std::lock_guard<std::recursive_mutex> guard(c->mu);
+    if (sc->ctx != c) return yk_set_error(YK_ERR_INVALID, std::string(q.who) + ": scene belongs to another context");
+    CUDA_TRY(cudaSetDevice(c->device));
+    (void)cudaGetLastError();
+    const yk_hits none{};
+    const yk_hits& h = q.hits ? *q.hits : none;
+    if (q.on_device) {
+        const std::pair<const void*, const char*> arrays[] = {
+            {q.o, "o_xyz"}, {q.d, "d_xyz"}, {q.t_max, "t_max"}, {q.occluded, "occluded_out"}, {h.t, "t"}, {h.orig_id, "orig_id"},
+            {h.counts, "counts"}, {h.material, "material"}, {h.area_light, "area_light"}, {h.p, "p"}, {h.n, "n"}, {h.uv, "uv"},
+            {h.shading_n, "shading_n"}, {h.shading_dpdu, "shading_dpdu"}};
+        for (const auto& a : arrays) {
+            const int rc = check_device_array(c, a.first, q.who, a.second);
+            if (rc != YK_OK) return rc;
+        }
+    }
+    const bool surface = q.hits && wants_surface(h);
+    uint32_t chunk = 0;
+    int rc = query_prepare(c, sc, q.n, !q.on_device, !q.on_device && surface, &chunk);
+    if (rc != YK_OK) return rc;
+    Pipe& p = c->pipe[0];
+    cudaStream_t s = p.stream;
+    const bool check_nan = q.on_device && q.t_max;
+    if (q.on_device) {
+        // The pipe's stream is non-blocking: without this event it would not order after the caller's queued work.
+        // (ev[1] is otherwise unused; the context mutex serialises its users.)
+        CUDA_TRY(cudaEventRecord(c->ev[1], q.caller));
+        CUDA_TRY(cudaStreamWaitEvent(s, c->ev[1], 0));
+        if (check_nan) CUDA_TRY(cudaMemsetAsync(c->q_nan, 0, sizeof(int), s));
+    }
+    const bool generic = sc->dev.spheres != nullptr || sc->dev.leaf_table != nullptr;
+    RenderCfg cfg{};
+    cfg.integrator = YK_INTEGRATOR_PATH;
+    const int T = 256;
+    for (size_t first = 0; first < q.n; first += chunk) {
+        const uint32_t m = (uint32_t)std::min<size_t>(chunk, q.n - first);
+        const float *o = q.o + 3 * first, *d = q.d + 3 * first, *tm = q.t_max ? q.t_max + first : nullptr;
+        if (!q.on_device) {
+            CUDA_TRY(cudaMemcpyAsync(c->q_o, o, (size_t)3 * m * sizeof(float), cudaMemcpyHostToDevice, s));
+            CUDA_TRY(cudaMemcpyAsync(c->q_d, d, (size_t)3 * m * sizeof(float), cudaMemcpyHostToDevice, s));
+            if (tm) CUDA_TRY(cudaMemcpyAsync(c->q_tm, tm, (size_t)m * sizeof(float), cudaMemcpyHostToDevice, s));
+            o = c->q_o;
+            d = c->q_d;
+            tm = tm ? c->q_tm : nullptr;
+        }
+        IterCounters ctr{};
+        if (q.hits) ctr.n_active = m;
+        else ctr.mat[0] = m;  // all segments in the first material queue's range of shading positions
+        CUDA_TRY(cudaMemcpyAsync(&p.d_ctr[0], &ctr, sizeof(ctr), cudaMemcpyHostToDevice, s));
+        CUDA_TRY(cudaMemsetAsync(p.wave.totals, 0, sizeof(Totals), s));
+        // where an output of this chunk goes: the caller's array itself, or the staging buffer it is copied back from
+        auto out = [&](auto* caller, auto* staged, size_t per) -> decltype(caller) {
+            if (!caller) return nullptr;
+            return q.on_device ? caller + per * first : staged;
+        };
+        auto back = [&](auto* caller, const void* staged, size_t per) -> int {
+            if (!q.on_device && caller)
+                CUDA_TRY(cudaMemcpyAsync(caller + per * first, staged, per * m * sizeof(*caller), cudaMemcpyDeviceToHost, s));
+            return YK_OK;
+        };
+        if (q.hits) {
+            k_query_pack<<<(m + T - 1) / T, T, 0, s>>>(p.wave, o, d, tm, m, check_nan ? c->q_nan : nullptr);
+            const int blocks = grid_for(m, kTraceThreads, c->sm_count * std::max(1, c->occ_trace_closest));
+            if (generic) k_trace_closest<true, true><<<blocks, kTraceThreads, 0, s>>>(sc->dev, p.wave, 0, &p.d_ctr[0], nullptr);
+            else k_trace_closest<true, false><<<blocks, kTraceThreads, 0, s>>>(sc->dev, p.wave, 0, &p.d_ctr[0], nullptr);
+            if (h.t || h.orig_id || h.counts)
+                k_query_unpack<<<(m + T - 1) / T, T, 0, s>>>(sc->dev, p.wave, m, out(h.t, c->q_t, 1), out(h.orig_id, c->q_id, 1),
+                                                             out(h.counts, c->q_cnt, 2));
+            if (surface) {
+                QuerySurfaceOut so;
+                so.material = out(h.material, c->q_mat, 1);
+                so.area_light = out(h.area_light, c->q_al, 1);
+                so.p = out(h.p, c->q_p, 3);
+                so.n = out(h.n, c->q_n, 3);
+                so.uv = out(h.uv, c->q_uv, 2);
+                so.sh_n = out(h.shading_n, c->q_sh_n, 3);
+                so.sh_dpdu = out(h.shading_dpdu, c->q_sh_dpdu, 3);
+                k_query_surface<<<(m + T - 1) / T, T, 0, s>>>(sc->dev, p.wave, m, so);
+            }
+            if ((rc = back(h.t, c->q_t, 1)) != YK_OK || (rc = back(h.orig_id, c->q_id, 1)) != YK_OK ||
+                (rc = back(h.counts, c->q_cnt, 2)) != YK_OK || (rc = back(h.material, c->q_mat, 1)) != YK_OK ||
+                (rc = back(h.area_light, c->q_al, 1)) != YK_OK || (rc = back(h.p, c->q_p, 3)) != YK_OK ||
+                (rc = back(h.n, c->q_n, 3)) != YK_OK || (rc = back(h.uv, c->q_uv, 2)) != YK_OK ||
+                (rc = back(h.shading_n, c->q_sh_n, 3)) != YK_OK || (rc = back(h.shading_dpdu, c->q_sh_dpdu, 3)) != YK_OK)
+                return rc;
+        } else {
+            k_query_pack_segments<<<(m + T - 1) / T, T, 0, s>>>(p.wave, o, d, m);
+            const bool per_ray = c->shadow_mode != 0;  // one segment per lane either way; the per-ray kernel needs no fold
+            if (per_ray) {
+                const int blocks = grid_for(m, kTraceThreads, c->sm_count * std::max(1, c->occ_trace_rays));
+                if (generic) k_trace_shadow_rays<true><<<blocks, kTraceThreads, 0, s>>>(sc->dev, p.wave, 1u, &p.d_ctr[0]);
+                else k_trace_shadow_rays<false><<<blocks, kTraceThreads, 0, s>>>(sc->dev, p.wave, 1u, &p.d_ctr[0]);
+            } else {
+                const int blocks = grid_for(m, kTraceThreads, c->sm_count * std::max(1, c->occ_trace_any));
+                if (generic) k_trace_shadow<true><<<blocks, kTraceThreads, 0, s>>>(sc->dev, p.wave, cfg, &p.d_ctr[0]);
+                else k_trace_shadow<false><<<blocks, kTraceThreads, 0, s>>>(sc->dev, p.wave, cfg, &p.d_ctr[0]);
+            }
+            k_query_unpack_segments<<<(m + T - 1) / T, T, 0, s>>>(p.wave, m, per_ray ? 1 : 0, out(q.occluded, c->q_occ, 1));
+            if ((rc = back(q.occluded, c->q_occ, 1)) != YK_OK) return rc;
+        }
+        if (!q.on_device) CUDA_TRY(cudaStreamSynchronize(s));
+    }
+    if (q.on_device) {
+        int nan_seen = 0;
+        if (check_nan) CUDA_TRY(cudaMemcpyAsync(&nan_seen, c->q_nan, sizeof(int), cudaMemcpyDeviceToHost, s));
+        CUDA_TRY(cudaStreamSynchronize(s));
+        if (nan_seen) return yk_set_error(YK_ERR_INVALID, std::string(q.who) + ": NaN t_max (Ray::new, math/ray.rs)");
+    }
+    CUDA_TRY(cudaGetLastError());
+    return YK_OK;
+}
+
+// opts of yk_query_intersect / yk_query_occluded -> (on_device, caller stream)
+int query_options(const yk_query_opts* opts, const char* who, bool* on_device, cudaStream_t* stream) {
+    *on_device = false;
+    *stream = nullptr;
+    if (!opts) return YK_OK;
+    if (opts->flags & ~YK_QUERY_ON_DEVICE) return yk_set_error(YK_ERR_INVALID, std::string(who) + ": unknown flag bits");
+    if (opts->_reserved != 0) return yk_set_error(YK_ERR_INVALID, std::string(who) + ": _reserved must be 0");
+    *on_device = (opts->flags & YK_QUERY_ON_DEVICE) != 0;
+    *stream = *on_device ? (cudaStream_t)opts->stream : nullptr;
+    return YK_OK;
 }
 }  // namespace
 
@@ -1415,38 +1595,11 @@ int yk_trace(yk_context* c, const yk_scene* sc, const float* o_xyz, const float*
     if (n == 0) return YK_OK;
     for (size_t i = 0; t_max && i < n; ++i)
         if (t_max[i] != t_max[i]) return yk_set_error(YK_ERR_INVALID, "yk_trace: NaN t_max (Ray::new, math/ray.rs)");
-    std::lock_guard<std::recursive_mutex> guard(c->mu);
-    uint32_t chunk = 0;
-    int rc = query_prepare(c, sc, n, "yk_trace", &chunk);
-    if (rc != YK_OK) return rc;
-    Pipe& p = c->pipe[0];
-    cudaStream_t s = p.stream;
-    float *d_o = c->q_o, *d_d = c->q_d, *d_tm = c->q_tm, *d_t = c->q_t;
-    int32_t* d_id = c->q_id;
-    uint32_t* d_cnt = c->q_cnt;
-    const bool generic = sc->dev.spheres != nullptr || sc->dev.leaf_table != nullptr;
-    const int T = 256;
-    for (size_t first = 0; first < n; first += chunk) {
-        const uint32_t m = (uint32_t)std::min<size_t>(chunk, n - first);
-        CUDA_TRY(cudaMemcpyAsync(d_o, o_xyz + 3 * first, (size_t)3 * m * sizeof(float), cudaMemcpyHostToDevice, s));
-        CUDA_TRY(cudaMemcpyAsync(d_d, d_xyz + 3 * first, (size_t)3 * m * sizeof(float), cudaMemcpyHostToDevice, s));
-        if (t_max) CUDA_TRY(cudaMemcpyAsync(d_tm, t_max + first, (size_t)m * sizeof(float), cudaMemcpyHostToDevice, s));
-        IterCounters ctr{};
-        ctr.n_active = m;
-        CUDA_TRY(cudaMemcpyAsync(&p.d_ctr[0], &ctr, sizeof(ctr), cudaMemcpyHostToDevice, s));
-        CUDA_TRY(cudaMemsetAsync(p.wave.totals, 0, sizeof(Totals), s));
-        k_query_pack<<<(m + T - 1) / T, T, 0, s>>>(p.wave, d_o, d_d, t_max ? d_tm : nullptr, m);
-        const int blocks = grid_for(m, kTraceThreads, c->sm_count * std::max(1, c->occ_trace_closest));
-        if (generic) k_trace_closest<true, true><<<blocks, kTraceThreads, 0, s>>>(sc->dev, p.wave, 0, &p.d_ctr[0], nullptr);
-        else k_trace_closest<true, false><<<blocks, kTraceThreads, 0, s>>>(sc->dev, p.wave, 0, &p.d_ctr[0], nullptr);
-        k_query_unpack<<<(m + T - 1) / T, T, 0, s>>>(sc->dev, p.wave, m, d_t, d_id, counts_out ? d_cnt : nullptr);
-        CUDA_TRY(cudaMemcpyAsync(t_out + first, d_t, (size_t)m * sizeof(float), cudaMemcpyDeviceToHost, s));
-        CUDA_TRY(cudaMemcpyAsync(orig_id_out + first, d_id, (size_t)m * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
-        if (counts_out) CUDA_TRY(cudaMemcpyAsync(counts_out + 2 * first, d_cnt, (size_t)2 * m * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
-        CUDA_TRY(cudaStreamSynchronize(s));
-    }
-    CUDA_TRY(cudaGetLastError());
-    return YK_OK;
+    yk_hits hits{};
+    hits.t = t_out;
+    hits.orig_id = orig_id_out;
+    hits.counts = counts_out;
+    return query_run(c, sc, QueryCall{"yk_trace", o_xyz, d_xyz, t_max, n, false, nullptr, &hits, nullptr});
     });
 }
 
@@ -1456,43 +1609,35 @@ int yk_occluded(yk_context* c, const yk_scene* sc, const float* o_xyz, const flo
     return yk_guard("yk_occluded", [&]() -> int {
     if (!c || !sc || (n && (!o_xyz || !d_xyz || !occluded_out))) return yk_set_error(YK_ERR_INVALID, "yk_occluded: null argument");
     if (n == 0) return YK_OK;
-    std::lock_guard<std::recursive_mutex> guard(c->mu);
-    uint32_t chunk = 0;
-    int rc = query_prepare(c, sc, n, "yk_occluded", &chunk);
-    if (rc != YK_OK) return rc;
-    Pipe& p = c->pipe[0];
-    cudaStream_t s = p.stream;
-    float *d_o = c->q_o, *d_d = c->q_d;
-    uint8_t* d_out = c->q_occ;
-    const bool generic = sc->dev.spheres != nullptr || sc->dev.leaf_table != nullptr;
-    RenderCfg cfg{};
-    cfg.integrator = YK_INTEGRATOR_PATH;
-    const int T = 256;
-    for (size_t first = 0; first < n; first += chunk) {
-        const uint32_t m = (uint32_t)std::min<size_t>(chunk, n - first);
-        CUDA_TRY(cudaMemcpyAsync(d_o, o_xyz + 3 * first, (size_t)3 * m * sizeof(float), cudaMemcpyHostToDevice, s));
-        CUDA_TRY(cudaMemcpyAsync(d_d, d_xyz + 3 * first, (size_t)3 * m * sizeof(float), cudaMemcpyHostToDevice, s));
-        IterCounters ctr{};
-        ctr.mat[0] = m;  // all segments in the first material queue's range of shading positions
-        CUDA_TRY(cudaMemcpyAsync(&p.d_ctr[0], &ctr, sizeof(ctr), cudaMemcpyHostToDevice, s));
-        CUDA_TRY(cudaMemsetAsync(p.wave.totals, 0, sizeof(Totals), s));
-        k_query_pack_segments<<<(m + T - 1) / T, T, 0, s>>>(p.wave, d_o, d_d, m);
-        const bool per_ray = c->shadow_mode != 0;  // one segment per lane either way; the per-ray kernel needs no fold
-        if (per_ray) {
-            const int blocks = grid_for(m, kTraceThreads, c->sm_count * std::max(1, c->occ_trace_rays));
-            if (generic) k_trace_shadow_rays<true><<<blocks, kTraceThreads, 0, s>>>(sc->dev, p.wave, 1u, &p.d_ctr[0]);
-            else k_trace_shadow_rays<false><<<blocks, kTraceThreads, 0, s>>>(sc->dev, p.wave, 1u, &p.d_ctr[0]);
-        } else {
-            const int blocks = grid_for(m, kTraceThreads, c->sm_count * std::max(1, c->occ_trace_any));
-            if (generic) k_trace_shadow<true><<<blocks, kTraceThreads, 0, s>>>(sc->dev, p.wave, cfg, &p.d_ctr[0]);
-            else k_trace_shadow<false><<<blocks, kTraceThreads, 0, s>>>(sc->dev, p.wave, cfg, &p.d_ctr[0]);
-        }
-        k_query_unpack_segments<<<(m + T - 1) / T, T, 0, s>>>(p.wave, m, per_ray ? 1 : 0, d_out);
-        CUDA_TRY(cudaMemcpyAsync(occluded_out + first, d_out, m, cudaMemcpyDeviceToHost, s));
-        CUDA_TRY(cudaStreamSynchronize(s));
-    }
-    CUDA_TRY(cudaGetLastError());
-    return YK_OK;
+    return query_run(c, sc, QueryCall{"yk_occluded", o_xyz, d_xyz, nullptr, n, false, nullptr, nullptr, occluded_out});
+    });
+}
+
+// Scene::intersect (bvh.rs:160-232 + the hit's SurfaceInteraction) for n caller rays, on host or device arrays.
+int yk_query_intersect(yk_context* c, const yk_scene* sc, const float* o_xyz, const float* d_xyz, const float* t_max, uint32_t n,
+                       const yk_query_opts* opts, const yk_hits* out) {
+    return yk_guard("yk_query_intersect", [&]() -> int {
+    if (!c || !sc || !out || (n && (!o_xyz || !d_xyz))) return yk_set_error(YK_ERR_INVALID, "yk_query_intersect: null argument");
+    bool on_device = false;
+    cudaStream_t stream = nullptr;
+    int rc = query_options(opts, "yk_query_intersect", &on_device, &stream);
+    if (rc != YK_OK || n == 0) return rc;
+    for (size_t i = 0; !on_device && t_max && i < n; ++i)  // device arrays: k_query_pack raises c->q_nan instead
+        if (t_max[i] != t_max[i]) return yk_set_error(YK_ERR_INVALID, "yk_query_intersect: NaN t_max (Ray::new, math/ray.rs)");
+    return query_run(c, sc, QueryCall{"yk_query_intersect", o_xyz, d_xyz, t_max, n, on_device, stream, out, nullptr});
+    });
+}
+
+// yk_occluded on host or device arrays.
+int yk_query_occluded(yk_context* c, const yk_scene* sc, const float* o_xyz, const float* d_xyz, uint32_t n, const yk_query_opts* opts,
+                      uint8_t* occluded_out) {
+    return yk_guard("yk_query_occluded", [&]() -> int {
+    if (!c || !sc || (n && (!o_xyz || !d_xyz || !occluded_out))) return yk_set_error(YK_ERR_INVALID, "yk_query_occluded: null argument");
+    bool on_device = false;
+    cudaStream_t stream = nullptr;
+    int rc = query_options(opts, "yk_query_occluded", &on_device, &stream);
+    if (rc != YK_OK || n == 0) return rc;
+    return query_run(c, sc, QueryCall{"yk_query_occluded", o_xyz, d_xyz, nullptr, n, on_device, stream, nullptr, occluded_out});
     });
 }
 
