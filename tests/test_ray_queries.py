@@ -97,11 +97,8 @@ def _grid_scene(xf, n=6):
     return s
 
 
-@pytest.mark.gpu
-def test_corner_case_rays(gpu_ctx, oracle, xf):
-    n = 6
-    scene = _grid_scene(xf, n)
-    dev, osc = api.Scene(gpu_ctx, scene), oracle.OracleScene(scene)
+def corner_case_rays(n=6):
+    """Rays at _grid_scene(xf, n)'s vertices, shared edges and box planes: (o, d, t_max) as float32 arrays."""
     o, d, tm = [], [], []
     inf = np.inf
 
@@ -130,7 +127,15 @@ def test_corner_case_rays(gpu_ctx, oracle, xf):
     add((n, 1.0, 3.0), (0.0, 0.0, 1.0))                   # inside the wall's plane
     add((n, 1.0, 3.0), (1.0, 0.0, 0.0))                   # starts on the wall
     add((n, 1.0, 3.0), (-1.0, 0.0, 0.0))
-    o, d, tm = np.array(o, np.float32), np.array(d, np.float32), np.array(tm, np.float32)
+    return np.array(o, np.float32), np.array(d, np.float32), np.array(tm, np.float32)
+
+
+@pytest.mark.gpu
+def test_corner_case_rays(gpu_ctx, oracle, xf):
+    n = 6
+    scene = _grid_scene(xf, n)
+    dev, osc = api.Scene(gpu_ctx, scene), oracle.OracleScene(scene)
+    o, d, tm = corner_case_rays(n)
     t, ids = _same(dev, osc, o, d, tm)
     assert (ids >= 0).sum() > 100
     _same_occluded(dev, osc, o, d)
