@@ -184,8 +184,22 @@ typedef struct {
 /* ---- render options / statistics ------------------------------------------------------------ */
 #define YK_RENDER_FILM_ON_DEVICE 1u  /* film_rgb (and opts.hit_ids) are device pointers on the context's GPU */
 #define YK_RENDER_KEEP_FILM 2u       /* non-accumulating render: pixels outside `tiles` are left untouched (default) */
+#define YK_RENDER_AOVS 4u            /* read opts.aovs: companion films of the same render (Path / Whitted only; not yk_multi_render) */
 #define YK_RAY_SORT_TRACE_ONLY 16u   /* yk_render_opts.ray_sort flag: only the closest-hit kernel walks the sorted order (default: the
                                         material sort does too, so shading and shadow rays run in the same order) */
+
+/* Companion films of a Path or Whitted render (YK_RENDER_AOVS). Each pointer is optional (NULL = not produced) and, like film_rgb,
+ * res_y*res_x*3 f32 on the host, or on the device with YK_RENDER_FILM_ON_DEVICE. They follow film_rgb's semantics: the mean
+ * over the samples summed in ascending sample order, or (accumulating films) one add per tile sample in tile-list order;
+ * pixels outside `tiles` are left untouched. The four views are the films of the debug integrators from the same camera rays:
+ * each equals, bit for bit, what yk_render returns with that integrator. */
+typedef struct {
+    float* bvh_intersections;  /* BVHIntersections film (bvh_heatmap.rs): (tests, hits, hits if the ray hit, else 0) */
+    float* geometry_normals;   /* GeometryNormals film (geometry_normals.rs): n / 2 + 0.5, 0 on a miss */
+    float* shading_normals;    /* ShadingNormals film (shading_normals.rs) */
+    float* shading_uvs;        /* ShadingUVs film (shading_uvs.rs): (u, v, 0) */
+    float* radiance_sq;        /* per pixel and channel: the sum of li * li over the samples, in the film's order, / spp */
+} yk_aov_films;
 
 typedef int (*yk_progress_fn)(void* user, uint64_t samples_done, uint64_t samples_total); /* return !=0 to cancel */
 
@@ -203,6 +217,7 @@ typedef struct {
                                    leaves + direction octant, 3 = key = Morton cell of the ray origin + direction octant. The film does
                                    not depend on it (bit-identical either way). */
     uint32_t _reserved;
+    const yk_aov_films* aovs;   /* read only when flags & YK_RENDER_AOVS (callers built against the shorter struct never set it) */
 } yk_render_opts;
 
 typedef struct {
@@ -237,7 +252,10 @@ void yk_scene_destroy(yk_scene*);
  * Replaces Integrator::render + Film::update_tile for every tile in the list. Non-accumulating:
  * film[pixel] = mean over all samples_per_pixel (integrators/mod.rs:152-175). Accumulating
  * (film_settings.accumulate): each tile renders the single sample `tile.sample` and is ADDED to the
- * film (film.rs:260-272). `film_rgb` is res_y*res_x*3 f32, row-major (film.rs:72,95). */
+ * film (film.rs:260-272). `film_rgb` is res_y*res_x*3 f32, row-major (film.rs:72,95).
+ * With YK_RENDER_AOVS the same render also writes opts->aovs' films. Refused (YK_ERR_INVALID, nothing launched) when
+ * opts->aovs is NULL, for the debug integrators (they are the views themselves) and for Path with max_depth 0 (no primary
+ * ray is traced); yk_multi_render refuses the flag. An all-NULL yk_aov_films is a plain render. */
 int yk_render(yk_context*, const yk_scene*, const yk_camera*, const yk_film_settings*, const yk_sampler*,
               const yk_integrator*, const yk_tile* tiles, uint32_t n_tiles, const yk_render_opts* opts,
               float* film_rgb, yk_stats* stats);

@@ -172,3 +172,32 @@ if which == "terrain16":  # the render of bench.py's large_scene leg (one pipe),
 if which == "c64":
     s, c = scenes.cornell(xf, light="rect", tall_box="glass")
     probe("cornell 1024^2 path8 64spp", s, c, D.FilmSettings((1024, 1024), 16), D.SamplerType.stratified(8, 8), D.IntegratorType.path(8), reps=3)
+if which == "aov":  # companion films: Path alone, Path + each view, Path + all five, and each debug integrator on its own
+    import subprocess
+    print(subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv"], capture_output=True, text=True).stdout.strip(), flush=True)
+    from yuki_b200 import capi
+    views = ("bvh_intersections", "geometry_normals", "shading_normals", "shading_uvs")
+    debug = {"bvh_intersections": D.IntegratorType.bvh_intersections(), "geometry_normals": D.IntegratorType.debug(D.INTEGRATOR_GEOMETRY_NORMALS),
+             "shading_normals": D.IntegratorType.debug(D.INTEGRATOR_SHADING_NORMALS), "shading_uvs": D.IntegratorType.debug(D.INTEGRATOR_SHADING_UVS)}
+    def aov_table(name, s, c, film, smp, reps=5):
+        ctx = api.Context(0); dev = api.Scene(ctx, s); rn = api.Renderer(ctx)
+        path = D.IntegratorType.path(8)
+        runs = [("path", path, ())] + [(f"path + {v}", path, (v,)) for v in capi.AOV_NAMES] + [("path + all five", path, capi.AOV_NAMES),
+                ("path + four views", path, views)] + [(f"debug {v} alone", debug[v], ()) for v in views]
+        best = {}
+        for rep in range(reps + 1):  # round-robin over the configurations; rep 0 warms up; best device time of the rest
+            for label, integ, aovs in runs:
+                r = rn.render(dev, c, film, smp, integ, aovs=aovs)
+                if rep and (label not in best or r.stats.device_ms < best[label][0]):
+                    best[label] = (r.stats.device_ms, r.stats.seconds)
+        base = best["path"][0]
+        for label, _, _ in runs:
+            ms, wall = best[label]
+            print(f"{name} | {label:28s}: device {ms:8.2f} ms ({ms - base:+7.2f} ms vs path), lib wall {1e3 * wall:8.2f} ms", flush=True)
+        four = sum(best[f"debug {v} alone"][0] for v in views)
+        print(f"{name} | path + four views {best['path + four views'][0]:.2f} ms vs path + four debug renders {base + four:.2f} ms", flush=True)
+        dev.close(); ctx.close()
+    s, c = scenes.cornell(xf, light="rect", tall_box="glass")
+    aov_table("cornell 1024^2 path8 64spp", s, c, D.FilmSettings((1024, 1024), 16), D.SamplerType.stratified(8, 8))
+    s, c = scenes.heightfield(xf, 708, 708)
+    aov_table("heightfield 1M 1080p path8 16spp", s, c, D.FilmSettings((1920, 1080), 16), D.SamplerType.stratified(4, 4))

@@ -647,10 +647,21 @@ class RenderFinished:        # RenderStatus::Finished, renderer/mod.rs:29-31
 
 
 class RenderResult:
-    def __init__(self, film, hit_ids, stats):
+    def __init__(self, film, hit_ids, stats, aovs=None):
         self.film = film
         self.hit_ids = hit_ids
         self.stats = stats
+        self.aovs = aovs if aovs is not None else {}   # companion films by name (Renderer.render's `aovs`)
+
+
+def aov_names(aovs=None, aov_out=None) -> tuple:
+    """The companion films a render asks for: the names in `aovs` and the keys of `aov_out`, in capi.AOV_NAMES order.
+    An unknown name raises ValueError."""
+    names = set(aovs or ()) | set(aov_out or {})
+    unknown = sorted(n for n in names if n not in capi.AOV_NAMES)
+    if unknown:
+        raise ValueError(f"unknown companion film(s) {unknown}; known: {list(capi.AOV_NAMES)}")
+    return tuple(n for n in capi.AOV_NAMES if n in names)
 
 
 class Renderer:
@@ -677,6 +688,7 @@ class Renderer:
         """Starts a render into `film` on a background thread, overriding a running one (renderer/mod.rs:131-177).
         Accumulating film settings render one tile list per sample index, in order (render_manager.rs:135-143) and add
         into the film; otherwise the film's tiles are overwritten with the per-pixel mean."""
+        aov_names(render_kw.get("aovs"), render_kw.get("aov_out"))   # an unknown name fails here, not on the worker
         self.kill()
         fs = film_settings or film.settings
         assert tuple(fs.res) == tuple(film.settings.res), "Film does not match settings"   # film.rs:421
@@ -742,6 +754,7 @@ class Renderer:
         `film.samples` and (optionally) rewrites the checkpoint. Returns the number of sample indices the film now holds.
         `render_fn(tiles, film_out)` defaults to this renderer's `render`; tests on CPU pass the oracle's."""
         fs = film.settings
+        aov_names(render_kw.get("aovs"), render_kw.get("aov_out"))
         if not fs.accumulate or film.samples is None:
             raise ValueError("render_progressive needs an accumulating film (FilmSettings.accumulate)")
         spp = sampler.samples_per_pixel()
@@ -829,7 +842,12 @@ class Renderer:
     def render(self, scene: Scene, camera_params: D.CameraParameters, film: D.FilmSettings, sampler: D.SamplerType,
                integrator: D.IntegratorType, tiles: Optional[np.ndarray] = None, want_hit_ids: bool = False,
                aux_sample: int = 0, wavefront_paths: int = 0, film_out: Optional[np.ndarray] = None,
-               device_film_ptr: Optional[int] = None, progress=None, pipes: int = 0, ray_sort: int = 0) -> RenderResult:
+               device_film_ptr: Optional[int] = None, progress=None, pipes: int = 0, ray_sort: int = 0, aovs=None,
+               aov_out: Optional[dict] = None) -> RenderResult:
+        """`aovs`: names of companion films (capi.AOV_NAMES) rendered from the same camera rays, returned in
+        RenderResult.aovs as (res_y, res_x, 3) float32 arrays. `aov_out` maps names to the arrays to render into (accumulating
+        or keep-film renders, like `film_out`), or, with `device_film_ptr`, to device pointers; its names are requested too."""
+        names = aov_names(aovs, aov_out)
         cam = make_camera(camera_params, film)
         if tiles is None:
             tiles = film_tiles(film)
@@ -851,6 +869,21 @@ class Renderer:
             if want_hit_ids:
                 hit_ids = np.full((res_y, res_x), -1, dtype=np.int32)
                 opts.hit_ids = hit_ids.ctypes.data
+        views, aov_films = {}, capi.AovFilms()
+        for n in names:
+            if device_film_ptr is not None:
+                if aov_out is None or n not in aov_out:
+                    raise ValueError(f"device films: aov_out must give a device pointer for '{n}'")
+                views[n] = int(aov_out[n])
+                setattr(aov_films, n, views[n])
+            else:
+                a = aov_out[n] if aov_out is not None and n in aov_out else np.zeros((res_y, res_x, 3), dtype=np.float32)
+                assert a.dtype == np.float32 and a.flags["C_CONTIGUOUS"] and a.size == res_x * res_y * 3
+                views[n] = a
+                setattr(aov_films, n, a.ctypes.data)
+        if names:
+            opts.flags |= capi.RENDER_AOVS
+            opts.aovs = C.pointer(aov_films)
         cb = None
         if progress is not None:
             cb = capi.PROGRESS_FN(lambda user, done, total: int(bool(progress(done, total))))
@@ -859,4 +892,4 @@ class Renderer:
         stats = capi.Stats()
         capi.check(capi.lib().yk_render(self.ctx._h, scene._h, C.byref(cam), C.byref(fs), C.byref(sm), C.byref(ig),
                                         C.c_void_p(tiles.ctypes.data), len(tiles), C.byref(opts), film_ptr, C.byref(stats)))
-        return RenderResult(film_arr, hit_ids, stats)
+        return RenderResult(film_arr, hit_ids, stats, views)

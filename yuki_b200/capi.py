@@ -139,10 +139,19 @@ class PlyData(C.Structure):
                 ("normals", C.POINTER(C.c_float)), ("uvs", C.POINTER(C.c_float)), ("indices", C.POINTER(C.c_uint32))]
 
 
+class AovFilms(C.Structure):
+    """yk_aov_films: the companion films of a Path / Whitted render (NULL = not produced), in AOV_NAMES order."""
+    _fields_ = [("bvh_intersections", C.c_void_p), ("geometry_normals", C.c_void_p), ("shading_normals", C.c_void_p),
+                ("shading_uvs", C.c_void_p), ("radiance_sq", C.c_void_p)]
+
+
+AOV_NAMES = tuple(n for n, _ in AovFilms._fields_)
+
+
 class RenderOpts(C.Structure):
     _fields_ = [("flags", C.c_uint32), ("wavefront_paths", C.c_uint32), ("hit_ids", C.c_void_p), ("aux_sample", C.c_uint32),
                 ("pipes", C.c_uint32), ("progress", PROGRESS_FN), ("progress_user", C.c_void_p), ("ray_sort", C.c_uint32),
-                ("_reserved", C.c_uint32)]
+                ("_reserved", C.c_uint32), ("aovs", C.POINTER(AovFilms))]
 
 
 class Stats(C.Structure):
@@ -157,6 +166,7 @@ class Stats(C.Structure):
 
 
 RENDER_FILM_ON_DEVICE = 1
+RENDER_AOVS = 4
 QUERY_ON_DEVICE = 1
 
 

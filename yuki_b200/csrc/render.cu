@@ -18,6 +18,7 @@
 #include <chrono>
 #include <memory>
 #include <mutex>
+#include <cstddef>
 #include <cstdio>
 #include <cmath>
 #include <cstdlib>
@@ -35,6 +36,7 @@
 #include "wf_trace.cuh"
 #include "wf_shade.cuh"
 #include "wf_film.cuh"
+#include "wf_aov.cuh"
 #include "wf_query.cuh"
 #include "wf_scene_pack.cuh"
 
@@ -95,6 +97,9 @@ struct yk_context {
     float* d_film = nullptr;
     int32_t* d_hit_ids = nullptr;
     size_t film_cap = 0;
+    float* d_aov_sums[kAovViews] = {};  // per-pixel sums of the requested companion films (yk_render_opts.aovs), like d_accum
+    float* d_aov_film[kAovViews] = {};  // device copies of the companion films given as host buffers
+    size_t aov_sums_cap[kAovViews] = {}, aov_film_cap[kAovViews] = {};
     int occ_trace_closest = 0, occ_trace_any = 0, occ_trace_rays = 0;
     int wide_per_sm = 16;  // grid cap of the grid-stride kernels, blocks per SM (development override: YK_WIDE_PER_SM)
     int n_pipes_env = 0;  // YK_PIPES override (development)
@@ -389,8 +394,9 @@ int retire_slot(Pipe* p, int k, Timers* tm, uint64_t* done_paths) {
 // One batch on one pipe: raygen, the bounce loop, and the per-batch film step, all asynchronous on the pipe's stream.
 // Path tracing runs exactly max_depth bounces (every queue length stays on the device); Whitted's tree walk has no
 // such bound, so it reads the next bounce's ray count back once per bounce.
+// `aov`: the companion films' sums (AovSums; all null = none requested).
 int run_batch(yk_context* c, Pipe* p, const yk_scene* sc, const RenderCfg& cfg, const Batch& bt, uint32_t first_sample, bool accumulate_film,
-              float* d_film, Timers* tm, uint64_t* done_paths) {
+              float* d_film, const AovSums& aov, Timers* tm, uint64_t* done_paths) {
     cudaStream_t s = p->stream;
     Wave& w = p->wave;
     const int k = (int)(p->n_batches % kRing);
@@ -460,7 +466,8 @@ int run_batch(yk_context* c, Pipe* p, const yk_scene* sc, const RenderCfg& cfg, 
         if (c->stage_timing > 0) CUDA_TRY(cudaEventRecord(stage_event(iter, 0), s));
         const bool spheres = sc->dev.spheres != nullptr || sc->dev.leaf_table != nullptr;  // the generic instantiations: sphere slots, leaf table
         nvtxRangePushA("yk closest hit");
-        if (cfg.integrator == YK_INTEGRATOR_BVH_INTERSECTIONS) {
+        // the BVH view needs bounce 0's per-ray counters: the counting instantiation traces the same hits
+        if (cfg.integrator == YK_INTEGRATOR_BVH_INTERSECTIONS || (iter == 0 && aov.v[0])) {
             if (spheres) k_trace_closest<true, true><<<closest_blocks, kTraceThreads, 0, s>>>(sc->dev, w, b, cur, perm_trace);
             else k_trace_closest<true, false><<<closest_blocks, kTraceThreads, 0, s>>>(sc->dev, w, b, cur, perm_trace);
         } else {
@@ -471,6 +478,11 @@ int run_batch(yk_context* c, Pipe* p, const yk_scene* sc, const RenderCfg& cfg, 
         if (c->stage_timing > 0) CUDA_TRY(cudaEventRecord(stage_event(iter, 1), s));
         tm->launches += 1;
         tm->closest_launches += 1;
+        // before bounce 1 overwrites the first hits; between stage events 1 and 2, which no yk_stats stage time sums (device_ms holds it)
+        if (iter == 0 && (aov.v[0] || aov.v[1] || aov.v[2] || aov.v[3])) {
+            k_aov_first_hit<<<(bt.n_jobs + T - 1) / T, T, 0, s>>>(sc->dev, w, bt, aov, cfg.res_x, accumulate_film ? 1u : 0u);
+            tm->launches += 1;
+        }
         if (cfg.debug_log) {  // yk_debug_ray: log this bounce of the single path before it is shaded
             k_debug_log<<<1, 32, 0, s>>>(sc->dev, w, cfg, bt, b, cur);
             tm->launches += 1;
@@ -566,6 +578,10 @@ int run_batch(yk_context* c, Pipe* p, const yk_scene* sc, const RenderCfg& cfg, 
     }
     nvtxRangePop();
     tm->launches += 1;
+    if (aov.v[kAovRadianceSq]) {  // (accumulating films: one sample per pixel per batch, added into the view itself)
+        k_film_accumulate_sq<<<(bt.n_jobs + T - 1) / T, T, 0, s>>>(w, bt, aov.v[kAovRadianceSq], cfg.res_x, accumulate_film ? 1u : 0u);
+        tm->launches += 1;
+    }
     CUDA_TRY(cudaEventRecord(sl.done, s));
     CUDA_TRY(cudaGetLastError());
     sl.busy = true;
@@ -665,6 +681,7 @@ void yk_context_destroy(yk_context* c) {
     cudaFree(c->d_accum);
     cudaFree(c->d_film);
     cudaFree(c->d_hit_ids);
+    for (int k = 0; k < kAovViews; ++k) { cudaFree(c->d_aov_sums[k]); cudaFree(c->d_aov_film[k]); }
     for (auto& ev : c->ev) cudaEventDestroy(ev);
     cudaStreamDestroy(c->stream);
     delete c;
@@ -986,6 +1003,11 @@ void yk_scene_destroy(yk_scene* s) {
 // Internal yk_render_opts.flags bit (yk_multi_render's workers): the caller initialised the hit-id image, do not refill it.
 constexpr uint32_t kRenderAuxInitialised = 0x100u;
 
+// yk_aov_films' buffers in AovSums order
+static void aov_views(const yk_aov_films* a, float* (&v)[kAovViews]) {
+    v[0] = a->bvh_intersections; v[1] = a->geometry_normals; v[2] = a->shading_normals; v[3] = a->shading_uvs; v[4] = a->radiance_sq;
+}
+
 // yk_render, and yk_debug_ray's single path (`debug_log` = device ray list, `debug_px` = the film pixel of its camera sample).
 static int render_impl(yk_context* c, const yk_scene* sc, const yk_camera* cam, const yk_film_settings* fs, const yk_sampler* sm,
                        const yk_integrator* in, const yk_tile* tiles, uint32_t n_tiles, const yk_render_opts* opts, float* film_rgb,
@@ -1003,6 +1025,15 @@ static int render_impl(yk_context* c, const yk_scene* sc, const yk_camera* cam, 
     if (in->kind == YK_INTEGRATOR_WHITTED && in->max_depth > 24)
         return yk_set_error(YK_ERR_INVALID, "yk_render: whitted max_depth above 24 is not supported");
     if (n_tiles && !tiles) return yk_set_error(YK_ERR_INVALID, "yk_render: null tile list");
+    const yk_aov_films* aovs = nullptr;
+    if (opts && (opts->flags & YK_RENDER_AOVS)) {
+        if (!opts->aovs) return yk_set_error(YK_ERR_INVALID, "yk_render: YK_RENDER_AOVS without opts->aovs");
+        if (in->kind >= YK_INTEGRATOR_BVH_INTERSECTIONS)
+            return yk_set_error(YK_ERR_INVALID, "yk_render: companion films need the Path or Whitted integrator (the debug integrators are the views)");
+        if (in->kind == YK_INTEGRATOR_PATH && in->max_depth == 0)
+            return yk_set_error(YK_ERR_INVALID, "yk_render: companion films need a traced primary ray (Path max_depth 0 traces none)");
+        aovs = opts->aovs;
+    }
     std::lock_guard<std::recursive_mutex> guard(c->mu);
     CUDA_TRY(cudaSetDevice(c->device));
     (void)cudaGetLastError();  // do not inherit a stale error from an unrelated earlier call
@@ -1085,6 +1116,39 @@ static int render_impl(yk_context* c, const yk_scene* sc, const yk_camera* cam, 
         if (!(flags & kRenderAuxInitialised)) k_fill_i32<<<(unsigned)((n_pixels + 255) / 256), 256, 0, s>>>(d_ids, n_pixels, -1);
     }
     cfg.hit_ids = d_ids;
+    // Companion films: each requested view on the device (the caller's buffer, or a copy of the host buffer made like d_film's),
+    // and the per-pixel sums its kernels add into (accumulating films: the view itself).
+    float* d_aov[kAovViews] = {};
+    AovSums aov_sums{};
+    if (aovs) {
+        float* views[kAovViews];
+        aov_views(aovs, views);
+        auto ensure = [&](float** buf, size_t* cap) -> int {
+            if (*cap >= n_pixels) return YK_OK;
+            cudaFree(*buf);
+            *buf = nullptr;
+            *cap = 0;
+            CUDA_TRY(cudaMalloc((void**)buf, n_pixels * 3 * sizeof(float)));
+            *cap = n_pixels;
+            return YK_OK;
+        };
+        for (int k = 0; k < kAovViews; ++k) {
+            if (!views[k]) continue;
+            int rc = YK_OK;
+            if (on_device) d_aov[k] = views[k];
+            else {
+                if ((rc = ensure(&c->d_aov_film[k], &c->aov_film_cap[k])) != YK_OK) return rc;
+                d_aov[k] = c->d_aov_film[k];
+                if (full_cover) CUDA_TRY(cudaMemsetAsync(d_aov[k], 0, n_pixels * 3 * sizeof(float), s));
+                else CUDA_TRY(cudaMemcpyAsync(d_aov[k], views[k], n_pixels * 3 * sizeof(float), cudaMemcpyHostToDevice, s));
+            }
+            if (accumulate) aov_sums.v[k] = d_aov[k];
+            else {
+                if ((rc = ensure(&c->d_aov_sums[k], &c->aov_sums_cap[k])) != YK_OK) return rc;
+                aov_sums.v[k] = c->d_aov_sums[k];
+            }
+        }
+    }
 
     yk_stats st{};
     Timers tm;
@@ -1213,6 +1277,11 @@ static int render_impl(yk_context* c, const yk_scene* sc, const yk_camera* cam, 
                         if (!accumulate) {
                             k_zero_jobs<<<(nj + 255) / 256, 256, 0, p.stream>>>(p.d_jobs, nj, c->d_accum, fs->res_x);
                             tm.launches += 1;
+                            for (float* sums : aov_sums.v) {
+                                if (!sums) continue;
+                                k_zero_jobs<<<(nj + 255) / 256, 256, 0, p.stream>>>(p.d_jobs, nj, sums, fs->res_x);
+                                tm.launches += 1;
+                            }
                         }
                         if (debug_log) {
                             k_debug_job<<<1, 1, 0, p.stream>>>(p.d_jobs);
@@ -1255,7 +1324,7 @@ static int render_impl(yk_context* c, const yk_scene* sc, const yk_camera* cam, 
                     bt.n_paths = nj * bt.n_samples;
                     // the batch's first sample index: s0, or the sample of the group's tiles (accumulating films: one per group)
                     const uint32_t first_sample = accumulate ? (uint32_t)tiles[groups[group].t_lo].sample : s0;
-                    rc = run_batch(c, &p, sc, gcfg, bt, first_sample, accumulate, d_film, &tm, &done);
+                    rc = run_batch(c, &p, sc, gcfg, bt, first_sample, accumulate, d_film, aov_sums, &tm, &done);
                     if (rc != YK_OK) {  // nothing may stay in flight or marked busy behind an error return
                         cudaDeviceSynchronize();
                         for (Pipe& q : c->pipe)
@@ -1266,6 +1335,11 @@ static int render_impl(yk_context* c, const yk_scene* sc, const yk_camera* cam, 
                         // the group's last samples are queued: `color /= sample_count` + Film::update_tile for its pixels
                         k_film_store<<<(nj + 255) / 256, 256, 0, p.stream>>>(p.d_jobs, nj, c->d_accum, d_film, fs->res_x, (float)spp);
                         tm.launches += 1;
+                        for (int k = 0; k < kAovViews; ++k) {
+                            if (!d_aov[k]) continue;
+                            k_film_store<<<(nj + 255) / 256, 256, 0, p.stream>>>(p.d_jobs, nj, aov_sums.v[k], d_aov[k], fs->res_x, (float)spp);
+                            tm.launches += 1;
+                        }
                     }
                     if (opts && opts->progress && opts->progress(opts->progress_user, done, total_paths)) cancelled = true;
                 }
@@ -1291,6 +1365,12 @@ static int render_impl(yk_context* c, const yk_scene* sc, const yk_camera* cam, 
         CUDA_TRY(cudaMemcpyAsync(film_rgb, d_film, n_pixels * 3 * sizeof(float), cudaMemcpyDeviceToHost, s));
         if (opts && opts->hit_ids)
             CUDA_TRY(cudaMemcpyAsync(opts->hit_ids, d_ids, n_pixels * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+        if (aovs) {
+            float* views[kAovViews];
+            aov_views(aovs, views);
+            for (int k = 0; k < kAovViews; ++k)
+                if (views[k]) CUDA_TRY(cudaMemcpyAsync(views[k], d_aov[k], n_pixels * 3 * sizeof(float), cudaMemcpyDeviceToHost, s));
+        }
     }
     CUDA_TRY(cudaStreamSynchronize(s));
     CUDA_TRY(cudaGetLastError());

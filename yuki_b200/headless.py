@@ -16,7 +16,7 @@ import time
 
 import numpy as np
 
-from . import api, desc as D, scenes, transforms as xf
+from . import api, capi, desc as D, scenes, transforms as xf
 
 INTEGRATORS = {"whitted": D.INTEGRATOR_WHITTED, "path": D.INTEGRATOR_PATH, "bvh-intersections": D.INTEGRATOR_BVH_INTERSECTIONS,
                "geometry-normals": D.INTEGRATOR_GEOMETRY_NORMALS, "shading-normals": D.INTEGRATOR_SHADING_NORMALS,
@@ -64,7 +64,20 @@ def parse_args(argv=None):
     ap.add_argument("--exposure", type=float, default=1.0)
     ap.add_argument("--heatmap-channel", type=int, default=0, help="0 R, 1 G, 2 B, 3 luminance")
     ap.add_argument("--device", type=int, default=0)
+    ap.add_argument("--aov", type=aov_arg, action="append", default=[], metavar="NAME=PATH",
+                    help=f"also write a companion film of the same render as a raw EXR (Path / Whitted); NAME is one of "
+                         f"{', '.join(capi.AOV_NAMES)}; repeatable")
     return ap.parse_args(argv)
+
+
+def aov_arg(text):
+    """--aov NAME=PATH -> (name, path)."""
+    name, sep, path = text.partition("=")
+    if not sep or not path:
+        raise argparse.ArgumentTypeError(f"expected NAME=PATH, got '{text}'")
+    if name not in capi.AOV_NAMES:
+        raise argparse.ArgumentTypeError(f"unknown companion film '{name}' (one of {', '.join(capi.AOV_NAMES)})")
+    return name, path
 
 
 def settings_from_args(args):
@@ -101,7 +114,7 @@ def render(args, out=sys.stdout) -> np.ndarray:
     film = api.Film(film_settings)
     rn = api.Renderer(ctx)
     start = time.perf_counter()
-    rn.launch(dev, cam, film, sampler, integrator)
+    rn.launch(dev, cam, film, sampler, integrator, aovs=[name for name, _ in args.aov])
     width = 0
     while True:   # headless.rs:51-110
         st = rn.check_status()
@@ -125,6 +138,9 @@ def render(args, out=sys.stdout) -> np.ndarray:
         pixels, bounds = api.heatmap(ctx, pixels, args.heatmap_channel)
         print(f"Heatmap bounds {bounds[0]:g} .. {bounds[1]:g}", file=out)
     api.write_exr(args.out, pixels)
+    for name, path in args.aov:
+        api.write_exr(path, rn.last_result.aovs[name])
+        print(f"wrote {name} to {path}", file=out)
     st = rn.last_result.stats
     print(f"{st.samples / max(st.device_ms, 1e-9) * 1e-3:.1f} Msamples/s, {st.ray_count / max(st.device_ms, 1e-9) * 1e-3:.1f} Mrays/s on the device; "
           f"wrote {args.out}", file=out)
