@@ -185,6 +185,8 @@ typedef struct {
 #define YK_RENDER_FILM_ON_DEVICE 1u  /* film_rgb (and opts.hit_ids) are device pointers on the context's GPU */
 #define YK_RENDER_KEEP_FILM 2u       /* non-accumulating render: pixels outside `tiles` are left untouched (default) */
 #define YK_RENDER_AOVS 4u            /* read opts.aovs: companion films of the same render (Path / Whitted only; not yk_multi_render) */
+#define YK_RENDER_ADAPTIVE 8u        /* read opts.adaptive: stop each pixel once its mean is precise enough (Path / Whitted, averaging
+                                        films only; not yk_multi_render) */
 #define YK_RAY_SORT_TRACE_ONLY 16u   /* yk_render_opts.ray_sort flag: only the closest-hit kernel walks the sorted order (default: the
                                         material sort does too, so shading and shadow rays run in the same order) */
 
@@ -200,6 +202,19 @@ typedef struct {
     float* shading_uvs;        /* ShadingUVs film (shading_uvs.rs): (u, v, 0) */
     float* radiance_sq;        /* per pixel and channel: the sum of li * li over the samples, in the film's order, / spp */
 } yk_aov_films;
+
+/* Adaptive sampling (YK_RENDER_ADAPTIVE). The sampler's samples_per_pixel becomes each pixel's maximum. After n = min_samples,
+ * min_samples + step, ... samples (every such n below spp), a pixel stops when, for all three channels, with its float32 sums
+ * S = sum li and Q = sum li * li in ascending sample order and n as a float:
+ *     m = S / n;  v = Q / n - m * m;  v = max(v, 0);  e2 = v / (n - 1);  t = rel_error * m + abs_error;  e2 <= t * t
+ * (the squared standard error of the mean within the tolerance; every op un-fused IEEE float32, so a NaN never stops). A pixel
+ * that stops, or reaches spp, gets film = S / n and the companion films their sums / n. */
+typedef struct {
+    uint32_t min_samples;      /* first convergence check after this many samples; >= 2 */
+    uint32_t step;             /* then a check every `step` samples; >= 1 */
+    float rel_error, abs_error;  /* >= 0, finite */
+    uint32_t* sample_counts;   /* optional res_y*res_x out: samples taken per pixel; host, or device with YK_RENDER_FILM_ON_DEVICE */
+} yk_adaptive;
 
 typedef int (*yk_progress_fn)(void* user, uint64_t samples_done, uint64_t samples_total); /* return !=0 to cancel */
 
@@ -218,6 +233,7 @@ typedef struct {
                                    not depend on it (bit-identical either way). */
     uint32_t _reserved;
     const yk_aov_films* aovs;   /* read only when flags & YK_RENDER_AOVS (callers built against the shorter struct never set it) */
+    const yk_adaptive* adaptive;  /* read only when flags & YK_RENDER_ADAPTIVE */
 } yk_render_opts;
 
 typedef struct {
@@ -255,7 +271,13 @@ void yk_scene_destroy(yk_scene*);
  * film (film.rs:260-272). `film_rgb` is res_y*res_x*3 f32, row-major (film.rs:72,95).
  * With YK_RENDER_AOVS the same render also writes opts->aovs' films. Refused (YK_ERR_INVALID, nothing launched) when
  * opts->aovs is NULL, for the debug integrators (they are the views themselves) and for Path with max_depth 0 (no primary
- * ray is traced); yk_multi_render refuses the flag. An all-NULL yk_aov_films is a plain render. */
+ * ray is traced); yk_multi_render refuses the flag. An all-NULL yk_aov_films is a plain render.
+ * With YK_RENDER_ADAPTIVE each pixel takes between min_samples and spp samples (yk_adaptive); the film, companion films and
+ * counts do not depend on the batch shape, pipes, ray sort or shadow mode. stats.samples is the sum of the counts, the ray and
+ * traversal counters count the samples traced, the progress callback reports (done, spp * pixels) and at the end (total,
+ * total), and hit_ids holds -1 for a pixel that stopped before `aux_sample`. Refused (YK_ERR_INVALID, nothing launched)
+ * when opts->adaptive is NULL, min_samples < 2, step is 0, a tolerance is negative or not finite, the film accumulates or
+ * the integrator is a debug one; yk_multi_render refuses the flag. min_samples >= spp is the plain render. */
 int yk_render(yk_context*, const yk_scene*, const yk_camera*, const yk_film_settings*, const yk_sampler*,
               const yk_integrator*, const yk_tile* tiles, uint32_t n_tiles, const yk_render_opts* opts,
               float* film_rgb, yk_stats* stats);

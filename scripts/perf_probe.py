@@ -201,3 +201,28 @@ if which == "aov":  # companion films: Path alone, Path + each view, Path + all 
     aov_table("cornell 1024^2 path8 64spp", s, c, D.FilmSettings((1024, 1024), 16), D.SamplerType.stratified(8, 8))
     s, c = scenes.heightfield(xf, 708, 708)
     aov_table("heightfield 1M 1080p path8 16spp", s, c, D.FilmSettings((1920, 1080), 16), D.SamplerType.stratified(4, 4))
+if which == "adaptive":  # adaptive sampling against uniform spp: device time, samples taken and RMSE against a 4096-spp render
+    import subprocess
+    print(subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv"], capture_output=True, text=True).stdout.strip(), flush=True)
+    def adaptive_table(name, s, c, film, reps=2):
+        ctx = api.Context(0); dev = api.Scene(ctx, s); rn = api.Renderer(ctx)
+        path = D.IntegratorType.path(8)
+        # the reference draws from another seed: the renders under test must not share its samples
+        ref = rn.render(dev, c, film, D.SamplerType.uniform(4096, seed=12345), path).film.astype(np.float64)
+        runs = [(f"uniform {n:4d} spp", D.SamplerType.uniform(n), None) for n in (64, 128, 256, 512, 1024)]
+        runs += [(f"adaptive rel {rel:<5g} (16/16, max 1024)", D.SamplerType.uniform(1024), D.Adaptive(16, 16, rel, 0.0)) for rel in (0.1, 0.05, 0.02)]
+        best = {}
+        for rep in range(reps + 1):  # round-robin; rep 0 warms up; best device time of the rest (the films are identical)
+            for label, smp, ad in runs:
+                r = rn.render(dev, c, film, smp, path, adaptive=ad)
+                if rep and (label not in best or r.stats.device_ms < best[label][0]):
+                    best[label] = (r.stats.device_ms, r.stats.samples, float(np.sqrt(np.mean((r.film - ref) ** 2))))
+        for label, _, _ in runs:
+            ms, n, rmse = best[label]
+            print(f"{name} | {label:34s}: device {ms:9.2f} ms, {n:11d} samples ({n / (film.res[0] * film.res[1]):7.1f} per pixel), "
+                  f"{n / ms / 1e3:7.1f} Msamples/s, RMSE {rmse:.5f}", flush=True)
+        dev.close(); ctx.close()
+    s, c = scenes.cornell(xf, light="rect", tall_box="glass")
+    adaptive_table("cornell 1024^2 path8", s, c, D.FilmSettings((1024, 1024), 16))
+    s, c = scenes.heightfield(xf, 708, 708)
+    adaptive_table("heightfield 1M 1080p path8", s, c, D.FilmSettings((1920, 1080), 16))

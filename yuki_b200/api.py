@@ -647,11 +647,12 @@ class RenderFinished:        # RenderStatus::Finished, renderer/mod.rs:29-31
 
 
 class RenderResult:
-    def __init__(self, film, hit_ids, stats, aovs=None):
+    def __init__(self, film, hit_ids, stats, aovs=None, sample_counts=None):
         self.film = film
         self.hit_ids = hit_ids
         self.stats = stats
         self.aovs = aovs if aovs is not None else {}   # companion films by name (Renderer.render's `aovs`)
+        self.sample_counts = sample_counts             # adaptive renders: (res_y, res_x) uint32 samples per pixel, or the device pointer
 
 
 def aov_names(aovs=None, aov_out=None) -> tuple:
@@ -662,6 +663,23 @@ def aov_names(aovs=None, aov_out=None) -> tuple:
     if unknown:
         raise ValueError(f"unknown companion film(s) {unknown}; known: {list(capi.AOV_NAMES)}")
     return tuple(n for n in capi.AOV_NAMES if n in names)
+
+
+def check_adaptive(adaptive: Optional[D.Adaptive], film: D.FilmSettings, integrator: D.IntegratorType) -> None:
+    """Raises ValueError for what yk_render refuses under adaptive sampling: min_samples < 2, step < 1, a negative or
+    non-finite tolerance, an accumulating film, a debug integrator."""
+    if adaptive is None:
+        return
+    if int(adaptive.min_samples) < 2 or int(adaptive.step) < 1:
+        raise ValueError(f"adaptive sampling needs min_samples >= 2 and step >= 1, got {adaptive}")
+    for name in ("rel_error", "abs_error"):
+        v = float(getattr(adaptive, name))
+        if not 0.0 <= v <= float(np.finfo(np.float32).max):   # (NaN fails the comparison)
+            raise ValueError(f"adaptive sampling: {name} must be finite and >= 0, got {v}")
+    if film.accumulate:
+        raise ValueError("adaptive sampling needs an averaging film (FilmSettings.accumulate is set)")
+    if integrator.kind not in (D.INTEGRATOR_PATH, D.INTEGRATOR_WHITTED):
+        raise ValueError("adaptive sampling needs the Path or Whitted integrator")
 
 
 class Renderer:
@@ -689,8 +707,9 @@ class Renderer:
         Accumulating film settings render one tile list per sample index, in order (render_manager.rs:135-143) and add
         into the film; otherwise the film's tiles are overwritten with the per-pixel mean."""
         aov_names(render_kw.get("aovs"), render_kw.get("aov_out"))   # an unknown name fails here, not on the worker
-        self.kill()
         fs = film_settings or film.settings
+        check_adaptive(render_kw.get("adaptive"), fs, integrator)
+        self.kill()
         assert tuple(fs.res) == tuple(film.settings.res), "Film does not match settings"   # film.rs:421
         if force_single_sample:   # SamplerType::instantiate(force_single_sample), sampling/mod.rs:21-42
             sampler = D.SamplerType(kind=sampler.kind, nx=1, ny=1, jitter=sampler.jitter, seed=sampler.seed)
@@ -755,6 +774,8 @@ class Renderer:
         `render_fn(tiles, film_out)` defaults to this renderer's `render`; tests on CPU pass the oracle's."""
         fs = film.settings
         aov_names(render_kw.get("aovs"), render_kw.get("aov_out"))
+        if render_kw.get("adaptive") is not None or render_kw.get("sample_counts_out") is not None:
+            raise ValueError("render_progressive: adaptive sampling needs an averaging film, not an accumulating one")
         if not fs.accumulate or film.samples is None:
             raise ValueError("render_progressive needs an accumulating film (FilmSettings.accumulate)")
         spp = sampler.samples_per_pixel()
@@ -843,11 +864,17 @@ class Renderer:
                integrator: D.IntegratorType, tiles: Optional[np.ndarray] = None, want_hit_ids: bool = False,
                aux_sample: int = 0, wavefront_paths: int = 0, film_out: Optional[np.ndarray] = None,
                device_film_ptr: Optional[int] = None, progress=None, pipes: int = 0, ray_sort: int = 0, aovs=None,
-               aov_out: Optional[dict] = None) -> RenderResult:
+               aov_out: Optional[dict] = None, adaptive: Optional[D.Adaptive] = None, sample_counts_out=None) -> RenderResult:
         """`aovs`: names of companion films (capi.AOV_NAMES) rendered from the same camera rays, returned in
         RenderResult.aovs as (res_y, res_x, 3) float32 arrays. `aov_out` maps names to the arrays to render into (accumulating
-        or keep-film renders, like `film_out`), or, with `device_film_ptr`, to device pointers; its names are requested too."""
+        or keep-film renders, like `film_out`), or, with `device_film_ptr`, to device pointers; its names are requested too.
+        `adaptive` (D.Adaptive): stop each pixel once its mean is precise enough; RenderResult.sample_counts is then the
+        (res_y, res_x) uint32 array of samples per pixel: `sample_counts_out` if given (pixels outside `tiles` keep their
+        values), or, with `device_film_ptr`, the device pointer `sample_counts_out` (None: no counts)."""
         names = aov_names(aovs, aov_out)
+        check_adaptive(adaptive, film, integrator)
+        if sample_counts_out is not None and adaptive is None:
+            raise ValueError("sample_counts_out needs adaptive sampling (adaptive=D.Adaptive(...))")
         cam = make_camera(camera_params, film)
         if tiles is None:
             tiles = film_tiles(film)
@@ -884,6 +911,18 @@ class Renderer:
         if names:
             opts.flags |= capi.RENDER_AOVS
             opts.aovs = C.pointer(aov_films)
+        counts = None
+        if adaptive is not None:
+            ad = capi.Adaptive(int(adaptive.min_samples), int(adaptive.step), float(adaptive.rel_error), float(adaptive.abs_error))
+            if device_film_ptr is not None:
+                counts = None if sample_counts_out is None else int(sample_counts_out)
+                ad.sample_counts = counts
+            else:
+                counts = sample_counts_out if sample_counts_out is not None else np.zeros((res_y, res_x), dtype=np.uint32)
+                assert counts.dtype == np.uint32 and counts.flags["C_CONTIGUOUS"] and counts.size == res_x * res_y
+                ad.sample_counts = counts.ctypes.data
+            opts.flags |= capi.RENDER_ADAPTIVE
+            opts.adaptive = C.pointer(ad)
         cb = None
         if progress is not None:
             cb = capi.PROGRESS_FN(lambda user, done, total: int(bool(progress(done, total))))
@@ -892,4 +931,4 @@ class Renderer:
         stats = capi.Stats()
         capi.check(capi.lib().yk_render(self.ctx._h, scene._h, C.byref(cam), C.byref(fs), C.byref(sm), C.byref(ig),
                                         C.c_void_p(tiles.ctypes.data), len(tiles), C.byref(opts), film_ptr, C.byref(stats)))
-        return RenderResult(film_arr, hit_ids, stats, views)
+        return RenderResult(film_arr, hit_ids, stats, views, counts)

@@ -148,10 +148,16 @@ class AovFilms(C.Structure):
 AOV_NAMES = tuple(n for n, _ in AovFilms._fields_)
 
 
+class Adaptive(C.Structure):
+    """yk_adaptive: adaptive sampling's parameters and the optional per-pixel sample counts (YK_RENDER_ADAPTIVE)."""
+    _fields_ = [("min_samples", C.c_uint32), ("step", C.c_uint32), ("rel_error", C.c_float), ("abs_error", C.c_float),
+                ("sample_counts", C.c_void_p)]
+
+
 class RenderOpts(C.Structure):
     _fields_ = [("flags", C.c_uint32), ("wavefront_paths", C.c_uint32), ("hit_ids", C.c_void_p), ("aux_sample", C.c_uint32),
                 ("pipes", C.c_uint32), ("progress", PROGRESS_FN), ("progress_user", C.c_void_p), ("ray_sort", C.c_uint32),
-                ("_reserved", C.c_uint32), ("aovs", C.POINTER(AovFilms))]
+                ("_reserved", C.c_uint32), ("aovs", C.POINTER(AovFilms)), ("adaptive", C.POINTER(Adaptive))]
 
 
 class Stats(C.Structure):
@@ -167,6 +173,7 @@ class Stats(C.Structure):
 
 RENDER_FILM_ON_DEVICE = 1
 RENDER_AOVS = 4
+RENDER_ADAPTIVE = 8
 QUERY_ON_DEVICE = 1
 
 

@@ -37,6 +37,7 @@
 #include "wf_shade.cuh"
 #include "wf_film.cuh"
 #include "wf_aov.cuh"
+#include "wf_adaptive.cuh"
 #include "wf_query.cuh"
 #include "wf_scene_pack.cuh"
 
@@ -72,6 +73,16 @@ struct Pipe {
     uint32_t* d_dim_hash = nullptr;  // SamplerCfg::hash_table of the pipe's current pixel group
     size_t dim_hash_cap = 0;
     size_t hash_group = (size_t)-1;
+    // adaptive sampling (wf_adaptive.cuh): the job list a check compacts into, its per-job keep flags and per-block survivor
+    // counts, and the survivor count read back for the next batch's size
+    Job* d_jobs_next = nullptr;
+    size_t jobs_next_cap = 0;
+    uint8_t* d_keep = nullptr;
+    uint32_t* d_block_keep = nullptr;  // + 1 entry: the total
+    size_t keep_cap = 0;
+    uint32_t* h_survivors = nullptr;   // pinned
+    bool survivors_pending = false;    // a check's count is on its way to h_survivors
+    bool rehash = false;               // the job list was compacted: SamplerCfg::hash_table is indexed by the old job slots
     struct Slot {
         cudaEvent_t done = nullptr;
         std::vector<cudaEvent_t> ev;  // kTimedStages per bounce
@@ -100,6 +111,9 @@ struct yk_context {
     float* d_aov_sums[kAovViews] = {};  // per-pixel sums of the requested companion films (yk_render_opts.aovs), like d_accum
     float* d_aov_film[kAovViews] = {};  // device copies of the companion films given as host buffers
     size_t aov_sums_cap[kAovViews] = {}, aov_film_cap[kAovViews] = {};
+    float* d_adaptive_sq = nullptr;  // adaptive renders without radiance_sq: the per-pixel sums of li * li the stopping rule reads
+    uint32_t* d_counts = nullptr;    // device copy of yk_adaptive::sample_counts given as a host buffer
+    size_t adaptive_sq_cap = 0, counts_cap = 0;
     int occ_trace_closest = 0, occ_trace_any = 0, occ_trace_rays = 0;
     int wide_per_sm = 16;  // grid cap of the grid-stride kernels, blocks per SM (development override: YK_WIDE_PER_SM)
     int n_pipes_env = 0;  // YK_PIPES override (development)
@@ -589,6 +603,49 @@ int run_batch(yk_context* c, Pipe* p, const yk_scene* sc, const RenderCfg& cfg, 
     return YK_OK;
 }
 
+// Adaptive sampling after the first `count` samples of every job of the pipe's list (nj jobs): the pixels that stop get their
+// films and counts (k_adaptive_check); unless `last` (every pixel stops), the survivors are compacted in order into the other
+// job list, which becomes the pipe's, and their number is copied to p->h_survivors (read once the stream has reached it).
+int adaptive_check(Pipe* p, uint32_t nj, uint32_t count, bool last, const yk_adaptive& a, uint32_t res_x, const float* accum,
+                   const AovSums& sums, const AovSums& views, float* film, uint32_t* counts, Timers* tm) {
+    cudaStream_t s = p->stream;
+    const uint32_t nb = (nj + kAdaptiveThreads - 1) / kAdaptiveThreads;
+    if (!last) {
+        if (p->jobs_next_cap < p->jobs_cap) {  // (cudaFree waits for the device: nothing in flight still reads the old buffer)
+            cudaFree(p->d_jobs_next);
+            p->d_jobs_next = nullptr;
+            p->jobs_next_cap = 0;
+            CUDA_TRY(cudaMalloc((void**)&p->d_jobs_next, p->jobs_cap * sizeof(Job)));
+            p->jobs_next_cap = p->jobs_cap;
+        }
+        if (p->keep_cap < nj) {
+            cudaFree(p->d_keep);
+            cudaFree(p->d_block_keep);
+            p->d_keep = nullptr;
+            p->d_block_keep = nullptr;
+            p->keep_cap = 0;
+            CUDA_TRY(cudaMalloc((void**)&p->d_keep, nj));
+            CUDA_TRY(cudaMalloc((void**)&p->d_block_keep, ((size_t)nb + 1) * sizeof(uint32_t)));
+            p->keep_cap = nj;
+        }
+        if (!p->h_survivors) CUDA_TRY(cudaMallocHost((void**)&p->h_survivors, sizeof(uint32_t)));
+    }
+    k_adaptive_check<<<nb, kAdaptiveThreads, 0, s>>>(p->d_jobs, nj, res_x, count, last ? 1u : 0u, a.rel_error, a.abs_error, accum, sums,
+                                                      views, film, counts, last ? nullptr : p->d_keep, last ? nullptr : p->d_block_keep);
+    tm->launches += 1;
+    if (last) return YK_OK;
+    uint32_t* d_total = p->d_block_keep + (p->keep_cap + kAdaptiveThreads - 1) / kAdaptiveThreads;
+    k_adaptive_scan<<<1, kAdaptiveScanThreads, 0, s>>>(p->d_block_keep, nb, d_total);
+    k_adaptive_compact<<<nb, kAdaptiveThreads, 0, s>>>(p->d_jobs, nj, p->d_keep, p->d_block_keep, p->d_jobs_next);
+    CUDA_TRY(cudaMemcpyAsync(p->h_survivors, d_total, sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+    tm->launches += 2;
+    std::swap(p->d_jobs, p->d_jobs_next);
+    std::swap(p->jobs_cap, p->jobs_next_cap);
+    p->survivors_pending = true;
+    p->rehash = true;
+    return YK_OK;
+}
+
 }  // namespace
 
 // Makes the context's device current on the calling thread (post.cu: the display passes may be called from any thread).
@@ -664,6 +721,10 @@ void yk_context_destroy(yk_context* c) {
         cudaFree(p.d_ctr);
         cudaFree(p.d_dim_hash);
         cudaFree(p.d_jobs);
+        cudaFree(p.d_jobs_next);
+        cudaFree(p.d_keep);
+        cudaFree(p.d_block_keep);
+        cudaFreeHost(p.h_survivors);
         cudaFree(p.d_jumps);
         cudaFreeHost(p.h_ctr);
         cudaFreeHost(p.h_totals);
@@ -682,6 +743,8 @@ void yk_context_destroy(yk_context* c) {
     cudaFree(c->d_film);
     cudaFree(c->d_hit_ids);
     for (int k = 0; k < kAovViews; ++k) { cudaFree(c->d_aov_sums[k]); cudaFree(c->d_aov_film[k]); }
+    cudaFree(c->d_adaptive_sq);
+    cudaFree(c->d_counts);
     for (auto& ev : c->ev) cudaEventDestroy(ev);
     cudaStreamDestroy(c->stream);
     delete c;
@@ -1034,6 +1097,19 @@ static int render_impl(yk_context* c, const yk_scene* sc, const yk_camera* cam, 
             return yk_set_error(YK_ERR_INVALID, "yk_render: companion films need a traced primary ray (Path max_depth 0 traces none)");
         aovs = opts->aovs;
     }
+    const yk_adaptive* adaptive = nullptr;
+    if (opts && (opts->flags & YK_RENDER_ADAPTIVE)) {
+        const yk_adaptive* a = opts->adaptive;
+        if (!a) return yk_set_error(YK_ERR_INVALID, "yk_render: YK_RENDER_ADAPTIVE without opts->adaptive");
+        if (a->min_samples < 2 || a->step == 0)
+            return yk_set_error(YK_ERR_INVALID, "yk_render: adaptive sampling needs min_samples >= 2 and step >= 1");
+        if (!std::isfinite(a->rel_error) || !std::isfinite(a->abs_error) || !(a->rel_error >= 0.0f) || !(a->abs_error >= 0.0f))
+            return yk_set_error(YK_ERR_INVALID, "yk_render: adaptive tolerances must be finite and >= 0");
+        if (fs->accumulate) return yk_set_error(YK_ERR_INVALID, "yk_render: adaptive sampling needs an averaging film (not accumulate)");
+        if (in->kind >= YK_INTEGRATOR_BVH_INTERSECTIONS)
+            return yk_set_error(YK_ERR_INVALID, "yk_render: adaptive sampling needs the Path or Whitted integrator");
+        adaptive = a;
+    }
     std::lock_guard<std::recursive_mutex> guard(c->mu);
     CUDA_TRY(cudaSetDevice(c->device));
     (void)cudaGetLastError();  // do not inherit a stale error from an unrelated earlier call
@@ -1120,18 +1196,18 @@ static int render_impl(yk_context* c, const yk_scene* sc, const yk_camera* cam, 
     // and the per-pixel sums its kernels add into (accumulating films: the view itself).
     float* d_aov[kAovViews] = {};
     AovSums aov_sums{};
+    auto ensure = [&](float** buf, size_t* cap) -> int {
+        if (*cap >= n_pixels) return YK_OK;
+        cudaFree(*buf);
+        *buf = nullptr;
+        *cap = 0;
+        CUDA_TRY(cudaMalloc((void**)buf, n_pixels * 3 * sizeof(float)));
+        *cap = n_pixels;
+        return YK_OK;
+    };
     if (aovs) {
         float* views[kAovViews];
         aov_views(aovs, views);
-        auto ensure = [&](float** buf, size_t* cap) -> int {
-            if (*cap >= n_pixels) return YK_OK;
-            cudaFree(*buf);
-            *buf = nullptr;
-            *cap = 0;
-            CUDA_TRY(cudaMalloc((void**)buf, n_pixels * 3 * sizeof(float)));
-            *cap = n_pixels;
-            return YK_OK;
-        };
         for (int k = 0; k < kAovViews; ++k) {
             if (!views[k]) continue;
             int rc = YK_OK;
@@ -1146,6 +1222,33 @@ static int render_impl(yk_context* c, const yk_scene* sc, const yk_camera* cam, 
             else {
                 if ((rc = ensure(&c->d_aov_sums[k], &c->aov_sums_cap[k])) != YK_OK) return rc;
                 aov_sums.v[k] = c->d_aov_sums[k];
+            }
+        }
+    }
+    // Adaptive sampling: the sums of li * li the stopping rule reads (radiance_sq's, else a scratch accumulator that the
+    // render zeroes and sums like a companion film), and the per-pixel counts on the device (kept outside `tiles`, like d_film).
+    uint32_t* d_counts = nullptr;
+    AovSums adaptive_views{};
+    if (adaptive) {
+        if (!aov_sums.v[kAovRadianceSq]) {
+            int rc = ensure(&c->d_adaptive_sq, &c->adaptive_sq_cap);
+            if (rc != YK_OK) return rc;
+            aov_sums.v[kAovRadianceSq] = c->d_adaptive_sq;
+        }
+        for (int k = 0; k < kAovViews; ++k) adaptive_views.v[k] = d_aov[k];
+        if (adaptive->sample_counts) {
+            if (on_device) d_counts = adaptive->sample_counts;
+            else {
+                if (c->counts_cap < n_pixels) {
+                    cudaFree(c->d_counts);
+                    c->d_counts = nullptr;
+                    c->counts_cap = 0;
+                    CUDA_TRY(cudaMalloc((void**)&c->d_counts, n_pixels * sizeof(uint32_t)));
+                    c->counts_cap = n_pixels;
+                }
+                d_counts = c->d_counts;
+                if (full_cover) CUDA_TRY(cudaMemsetAsync(d_counts, 0, n_pixels * sizeof(uint32_t), s));
+                else CUDA_TRY(cudaMemcpyAsync(d_counts, adaptive->sample_counts, n_pixels * sizeof(uint32_t), cudaMemcpyHostToDevice, s));
             }
         }
     }
@@ -1228,6 +1331,8 @@ static int render_impl(yk_context* c, const yk_scene* sc, const yk_camera* cam, 
             if (pi > 0) CUDA_TRY(cudaStreamWaitEvent(p.stream, c->ev[0], 0));
             CUDA_TRY(cudaMemsetAsync(p.wave.totals, 0, sizeof(Totals), p.stream));
             p.hash_group = (size_t)-1;
+            p.survivors_pending = false;
+            p.rehash = false;
         }
         // Pixel groups: consecutive runs of at most jobs_per_batch jobs. The accumulating film adds every batch into the
         // film in stream order, so a group never spans a change of `tile.sample`: within one sample index the reference's
@@ -1256,12 +1361,37 @@ static int render_impl(yk_context* c, const yk_scene* sc, const yk_camera* cam, 
         const size_t n_groups = groups.size();
         uint64_t done = 0;
         bool cancelled = false;
+        // The samples [s0, s1) of a batch: at most m, and, with adaptive sampling, never past the next check point (min_samples,
+        // min_samples + step, ...), so that the stopping decisions do not depend on the batch shape.
+        auto batch_end = [&](uint32_t s0) -> uint32_t {
+            uint32_t s1 = std::min(samples_per_job, s0 + m);
+            if (adaptive) {
+                const uint32_t lo = adaptive->min_samples, st_ = adaptive->step;
+                const uint64_t check = s0 < lo ? lo : lo + ((uint64_t)(s0 - lo) / st_ + 1) * st_;
+                s1 = (uint32_t)std::min<uint64_t>(s1, check);
+            }
+            return s1;
+        };
         for (size_t g0 = 0; g0 < n_groups && !cancelled; g0 += n_pipes) {
-            for (uint32_t s0 = 0; s0 < samples_per_job && !cancelled; s0 += m) {
+            uint32_t active[kMaxPipes] = {};  // adaptive: the jobs of each pipe's group still sampling (its job list's length)
+            for (uint32_t s0 = 0, s1 = 0; s0 < samples_per_job && !cancelled; s0 = s1) {
+                s1 = batch_end(s0);
+                bool any = false;
                 for (int pi = 0; pi < n_pipes && g0 + pi < n_groups && !cancelled; ++pi) {
                     Pipe& p = c->pipe[pi];
                     const size_t group = g0 + pi;
-                    const uint32_t nj = groups[group].count;
+                    uint32_t nj = groups[group].count;
+                    if (adaptive && p.hash_group == group) {
+                        if (p.survivors_pending) {  // the last check's survivors: the other pipe keeps running meanwhile
+                            CUDA_TRY(cudaStreamSynchronize(p.stream));
+                            active[pi] = *p.h_survivors;
+                            p.survivors_pending = false;
+                        }
+                        nj = active[pi];
+                        if (!nj) continue;  // every pixel of the group has stopped
+                    }
+                    any = true;
+                    active[pi] = nj;
                     if (p.hash_group != group) {  // a new pixel group on this pipe: its jobs, and a zeroed accumulator
                         if (p.jobs_cap < nj) {
                             CUDA_TRY(cudaStreamSynchronize(p.stream));
@@ -1296,7 +1426,7 @@ static int render_impl(yk_context* c, const yk_scene* sc, const yk_camera* cam, 
                         else if (in->kind == YK_INTEGRATOR_WHITTED)
                             dims = 2 + 2ull * sc->dev.n_lights * ((1ull << std::min(in->max_depth, 8u)) - 1);
                         dims = std::min<uint64_t>(dims, std::min<uint64_t>(4096, (256ull << 20) / (4ull * nj)));  // the rest is hashed on the fly
-                        if (p.hash_group != group) {
+                        if (p.hash_group != group || p.rehash) {
                             const size_t need = (size_t)dims * nj;
                             if (p.dim_hash_cap < need) {
                                 CUDA_TRY(cudaStreamSynchronize(p.stream));
@@ -1315,12 +1445,13 @@ static int render_impl(yk_context* c, const yk_scene* sc, const yk_camera* cam, 
                         gcfg.sampler.hash_stride = nj;
                     }
                     p.hash_group = group;
+                    p.rehash = false;
                     Batch bt;
                     bt.jobs = p.d_jobs;
                     bt.n_jobs = nj;
                     bt.div_jobs = FastDiv::make(nj);
                     bt.sample_off = s0;
-                    bt.n_samples = std::min(m, samples_per_job - s0);
+                    bt.n_samples = s1 - s0;
                     bt.n_paths = nj * bt.n_samples;
                     // the batch's first sample index: s0, or the sample of the group's tiles (accumulating films: one per group)
                     const uint32_t first_sample = accumulate ? (uint32_t)tiles[groups[group].t_lo].sample : s0;
@@ -1331,7 +1462,18 @@ static int render_impl(yk_context* c, const yk_scene* sc, const yk_camera* cam, 
                             for (auto& slot : q.slot) slot.busy = false;
                         return rc;
                     }
-                    if (!accumulate && s0 + m >= samples_per_job) {
+                    if (adaptive) {
+                        const bool last = s1 >= samples_per_job;
+                        if (last || (s1 >= adaptive->min_samples && (s1 - adaptive->min_samples) % adaptive->step == 0)) {
+                            rc = adaptive_check(&p, nj, s1, last, *adaptive, fs->res_x, c->d_accum, aov_sums, adaptive_views, d_film, d_counts, &tm);
+                            if (rc != YK_OK) {
+                                cudaDeviceSynchronize();
+                                for (Pipe& q : c->pipe)
+                                    for (auto& slot : q.slot) slot.busy = false;
+                                return rc;
+                            }
+                        }
+                    } else if (!accumulate && s1 >= samples_per_job) {
                         // the group's last samples are queued: `color /= sample_count` + Film::update_tile for its pixels
                         k_film_store<<<(nj + 255) / 256, 256, 0, p.stream>>>(p.d_jobs, nj, c->d_accum, d_film, fs->res_x, (float)spp);
                         tm.launches += 1;
@@ -1343,6 +1485,7 @@ static int render_impl(yk_context* c, const yk_scene* sc, const yk_camera* cam, 
                     }
                     if (opts && opts->progress && opts->progress(opts->progress_user, done, total_paths)) cancelled = true;
                 }
+                if (!any) break;
             }
         }
         for (int pi = 0; pi < n_pipes; ++pi) {
@@ -1357,8 +1500,10 @@ static int render_impl(yk_context* c, const yk_scene* sc, const yk_camera* cam, 
             totals.hit_hash += t.hit_hash; totals.shadow_rays += t.shadow_rays; totals.closest_rays += t.closest_rays;
         }
         if (cancelled) return yk_set_error(YK_ERR_CANCELLED, "yk_render: cancelled by the progress callback");
-        if (opts && opts->progress) opts->progress(opts->progress_user, done, total_paths);
-        st.samples = total_paths;
+        // (adaptive: the samples taken, each pixel's count, of at most total_paths)
+        const uint64_t taken = adaptive ? done : total_paths;
+        if (opts && opts->progress) opts->progress(opts->progress_user, taken, taken);
+        st.samples = taken;
     }
     CUDA_TRY(cudaEventRecord(c->ev[3], s));
     if (!on_device) {
@@ -1371,6 +1516,7 @@ static int render_impl(yk_context* c, const yk_scene* sc, const yk_camera* cam, 
             for (int k = 0; k < kAovViews; ++k)
                 if (views[k]) CUDA_TRY(cudaMemcpyAsync(views[k], d_aov[k], n_pixels * 3 * sizeof(float), cudaMemcpyDeviceToHost, s));
         }
+        if (d_counts) CUDA_TRY(cudaMemcpyAsync(adaptive->sample_counts, d_counts, n_pixels * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
     }
     CUDA_TRY(cudaStreamSynchronize(s));
     CUDA_TRY(cudaGetLastError());

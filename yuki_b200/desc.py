@@ -166,3 +166,14 @@ class IntegratorType:                       # integrators/mod.rs:33-40
     @staticmethod
     def debug(kind) -> "IntegratorType":
         return IntegratorType(kind, 0)
+
+
+@dataclass
+class Adaptive:                             # yk_adaptive (include/yuki_gpu.h): no counterpart in the reference
+    """Adaptive sampling: the sampler's samples per pixel become each pixel's maximum. After `min_samples` samples and then
+    every `step`, a pixel stops once, in every channel, the squared standard error of its mean is at most
+    (rel_error * mean + abs_error)^2."""
+    min_samples: int = 16
+    step: int = 16
+    rel_error: float = 0.05
+    abs_error: float = 0.0

@@ -67,7 +67,25 @@ def parse_args(argv=None):
     ap.add_argument("--aov", type=aov_arg, action="append", default=[], metavar="NAME=PATH",
                     help=f"also write a companion film of the same render as a raw EXR (Path / Whitted); NAME is one of "
                          f"{', '.join(capi.AOV_NAMES)}; repeatable")
-    return ap.parse_args(argv)
+    ap.add_argument("--adaptive", type=float, default=None, metavar="REL",
+                    help="adaptive sampling (Path / Whitted): stop a pixel once the standard error of its mean is at most "
+                         "REL * mean + --adaptive-abs in every channel; the sampler's spp is each pixel's maximum")
+    ap.add_argument("--adaptive-abs", type=float, default=0.0, metavar="A")
+    ap.add_argument("--adaptive-min", type=int, default=16, metavar="N", help="first check after N samples (>= 2)")
+    ap.add_argument("--adaptive-step", type=int, default=16, metavar="N", help="then a check every N samples")
+    ap.add_argument("--sample-counts", default=None, metavar="PATH",
+                    help="with --adaptive: write each pixel's sample count (in all three channels) as a raw EXR")
+    args = ap.parse_args(argv)
+    if args.sample_counts is not None and args.adaptive is None:
+        ap.error("--sample-counts needs --adaptive")
+    return args
+
+
+def adaptive_from_args(args):
+    """--adaptive REL [--adaptive-abs A --adaptive-min N --adaptive-step N] -> D.Adaptive, or None."""
+    if args.adaptive is None:
+        return None
+    return D.Adaptive(args.adaptive_min, args.adaptive_step, args.adaptive, args.adaptive_abs)
 
 
 def aov_arg(text):
@@ -114,7 +132,7 @@ def render(args, out=sys.stdout) -> np.ndarray:
     film = api.Film(film_settings)
     rn = api.Renderer(ctx)
     start = time.perf_counter()
-    rn.launch(dev, cam, film, sampler, integrator, aovs=[name for name, _ in args.aov])
+    rn.launch(dev, cam, film, sampler, integrator, aovs=[name for name, _ in args.aov], adaptive=adaptive_from_args(args))
     width = 0
     while True:   # headless.rs:51-110
         st = rn.check_status()
@@ -141,6 +159,10 @@ def render(args, out=sys.stdout) -> np.ndarray:
     for name, path in args.aov:
         api.write_exr(path, rn.last_result.aovs[name])
         print(f"wrote {name} to {path}", file=out)
+    if args.sample_counts is not None:
+        counts = rn.last_result.sample_counts.astype(np.float32)
+        api.write_exr(args.sample_counts, np.repeat(counts[:, :, None], 3, axis=2))
+        print(f"wrote sample counts to {args.sample_counts} ({int(rn.last_result.stats.samples)} samples)", file=out)
     st = rn.last_result.stats
     print(f"{st.samples / max(st.device_ms, 1e-9) * 1e-3:.1f} Msamples/s, {st.ray_count / max(st.device_ms, 1e-9) * 1e-3:.1f} Mrays/s on the device; "
           f"wrote {args.out}", file=out)
