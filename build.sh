@@ -9,6 +9,6 @@ $NVCC -std=c++17 -O3 -gencode arch=compute_100a,code=sm_100a -lineinfo \
   --fmad=false -prec-div=true -prec-sqrt=true -ftz=false \
   -Xcompiler -fPIC,-ffp-contract=off,-fno-fast-math,-pthread,-Wall \
   -Iinclude -I$SRC -shared -o $OUT \
-  $SRC/render.cu $SRC/host_scene.cpp $SRC/host_bvh.cpp $SRC/host_ply.cpp $SRC/host_exr.cpp $SRC/host_pbrt.cpp $SRC/host_mitsuba.cpp $SRC/post.cu -lz ${YK_NVCC_EXTRA}
+  $SRC/render.cu $SRC/host_scene.cpp $SRC/host_bvh.cpp $SRC/host_ply.cpp $SRC/host_exr.cpp $SRC/host_pbrt.cpp $SRC/host_mitsuba.cpp $SRC/post.cu $SRC/denoise.cu -lz ${YK_NVCC_EXTRA}
 make -s -C oracle
 echo "built $OUT and oracle/liboracle.so"

@@ -411,6 +411,37 @@ int yk_tonemap_filmic(yk_context*, const float* film_rgb, uint32_t res_x, uint32
  * are written back; otherwise the given values are used. */
 int yk_heatmap(yk_context*, const float* film_rgb, uint32_t res_x, uint32_t res_y, uint32_t channel, int auto_range, float* min_val,
                float* max_val, float* out_rgb);
+/* Denoising of an averaging Path / Whitted film (no counterpart in the reference): an edge-avoiding a-trous wavelet filter
+ * (Dammertz et al., HPG 2010) whose colour weights are scaled by each pixel's variance (SVGF, Schied et al., HPG 2017), from
+ * the render's own companion films. Per pixel with n >= 2 samples (n = sample_counts[p], or samples_per_pixel), every op
+ * un-fused IEEE float32 in the order written:
+ *     v = sq - c * c; if (v < 0) v = 0; v = v / (n - 1)  (per channel);   var = (v.r + v.g) + v.b
+ *     guide: d = g * 2 - 1;  l2 = (d.x * d.x + d.y * d.y) + d.z * d.z;  nh = l2 > 0 ? d / sqrtf(l2) : 0
+ * Iteration i = 0 .. iterations-1 (step s = 2^i) visits the 5x5 taps q = p + s * (kx - 2, ky - 2), ky outer, skipping taps
+ * outside the film or with n < 2. With h = (1/16, 1/4, 3/8, 1/4, 1/16): the centre tap weighs h[2] * h[2]; another tap
+ *     num = (dr * dr + dg * dg) + db * db  (d = c_i(p) - c_i(q));   den = (sigma * sigma) * (var_i(p) + var_i(q)) + eps
+ *     wc = den / (den + num); wc = wc * wc;   wn = 1, or with a guide t = nh(p) . nh(q), wn = max(t, 0)^128 (7 squarings)
+ *     w = ((h[ky] * h[kx]) * wn) * wc
+ * and a tap counts only when w > 0 (a NaN or infinite neighbour is skipped): W += w, C += w * c_i(q), V += (w * w) * var_i(q).
+ * Then c_i+1 = C / W and var_i+1 = V / (W * W). Pixels with n < 2 are copied through unchanged and are never a tap. The
+ * output is c_iterations. Refused (YK_ERR_INVALID, nothing launched): a NULL context, film_rgb, radiance_sq or out_rgb, a zero
+ * resolution, unknown flags, iterations outside 1 .. 10, a sigma or eps that is not > 0 and finite, no sample_counts and samples_per_pixel
+ * < 2. Host arrays are staged through the device; with YK_DENOISE_ON_DEVICE every array is device memory of the context's
+ * GPU and the call's work starts after the work already queued on `stream`. Returns when out_rgb is written. */
+#define YK_DENOISE_ON_DEVICE 1u
+typedef struct {
+    uint32_t flags;                 /* YK_DENOISE_ON_DEVICE or 0 (host arrays) */
+    uint32_t iterations;            /* 1 ... 10 */
+    float sigma, eps;               /* > 0 and finite */
+    uint32_t samples_per_pixel;     /* every pixel's n when sample_counts is NULL; >= 2 */
+    uint32_t _reserved;
+    const uint32_t* sample_counts;  /* optional res_y*res_x: yk_adaptive.sample_counts of the render */
+    const float* normals;           /* optional guide: a geometry_normals / shading_normals companion film */
+    void* stream;                   /* ON_DEVICE: the caller's cudaStream_t, as yk_query_opts.stream */
+} yk_denoise_params;
+/* film_rgb, radiance_sq, normals and out_rgb are res_y*res_x*3 f32; out_rgb may equal film_rgb. */
+int yk_denoise(yk_context*, uint32_t res_x, uint32_t res_y, const float* film_rgb, const float* radiance_sq,
+               const yk_denoise_params*, float* out_rgb);
 
 /* pbrt-v3 scene file -> host scene description, camera parameters and film resolution: the subset and defaults of
  * scene/pbrt/{lexer,mod,param_set,cie}.rs (see csrc/host_pbrt.cpp for the directive list and the kept quirks).

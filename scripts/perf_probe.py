@@ -226,3 +226,47 @@ if which == "adaptive":  # adaptive sampling against uniform spp: device time, s
     adaptive_table("cornell 1024^2 path8", s, c, D.FilmSettings((1024, 1024), 16))
     s, c = scenes.heightfield(xf, 708, 708)
     adaptive_table("heightfield 1M 1080p path8", s, c, D.FilmSettings((1920, 1080), 16))
+if which == "denoise":  # yk_denoise at 1080p and 4K next to the 16-spp renders whose films it would clean
+    import subprocess, torch
+    print(subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv"], capture_output=True, text=True).stdout.strip(), flush=True)
+
+    def denoise_table(name, s, c, film, reps=20):
+        ctx = api.Context(0); dev = api.Scene(ctx, s); rn = api.Renderer(ctx)
+        smp, path = D.SamplerType.stratified(4, 4), D.IntegratorType.path(8)
+        best = None
+        for _ in range(3):  # the first render allocates: report the fastest
+            r = rn.render(dev, c, film, smp, path, aovs=["radiance_sq", "shading_normals"])
+            best = r.stats.device_ms if best is None else min(best, r.stats.device_ms)
+        plain = min(rn.render(dev, c, film, smp, path).stats.device_ms for _ in range(2))
+        print(f"{name} | render Path 8, 16 spp: device {plain:8.2f} ms; with radiance_sq + shading_normals {best:8.2f} ms", flush=True)
+        gpu = torch.device("cuda", 0)
+        f, sq, nrm = (torch.from_numpy(a).to(gpu) for a in (r.film, r.aovs["radiance_sq"], r.aovs["shading_normals"]))
+        out = torch.empty_like(f)
+        stream = torch.cuda.current_stream(gpu)
+        for k in (5, 3, 1):
+            for guide in (None, nrm):
+                prm = D.Denoise(k)
+                api.denoise(ctx, f, sq, spp=16, normals=guide, params=prm, out=out)  # warm-up (pool allocation, module load)
+                times = []
+                for _ in range(reps):  # CUDA events on the caller's stream around the blocking call: device work + call overhead
+                    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+                    e0.record(stream)
+                    api.denoise(ctx, f, sq, spp=16, normals=guide, params=prm, out=out)
+                    e1.record(stream)
+                    e1.synchronize()
+                    times.append(e0.elapsed_time(e1))
+                host = []
+                hf, hsq, hn = r.film, r.aovs["radiance_sq"], (None if guide is None else r.aovs["shading_normals"])
+                for _ in range(5):  # host arrays: pageable copies both ways inside the call
+                    t0 = time.perf_counter()
+                    api.denoise(ctx, hf, hsq, spp=16, normals=hn, params=prm)
+                    host.append(1e3 * (time.perf_counter() - t0))
+                med = sorted(times)[len(times) // 2]
+                print(f"{name} | denoise {k} it, {'shading-normal guide' if guide is not None else 'no guide          '}: device tensors "
+                      f"best {min(times):6.3f} ms median {med:6.3f} ms ({min(times) / best * 100:5.2f} % of the render); host arrays best "
+                      f"{min(host):7.2f} ms", flush=True)
+        dev.close(); ctx.close()
+    s, c = scenes.material_room(xf)
+    denoise_table("C4 material room 1920x1080", s, c, D.FilmSettings((1920, 1080), 16))
+    s, c = scenes.terrain_room(xf)
+    denoise_table("C5 terrain 10M 3840x2160", s, c, D.FilmSettings((3840, 2160), 16))

@@ -471,6 +471,66 @@ def heatmap(ctx: Context, film: np.ndarray, channel: int = 0, value_range=None):
     return out, (lo.value, hi.value)
 
 
+def denoise(ctx: Context, film, radiance_sq, *, spp: Optional[int] = None, sample_counts=None, normals=None,
+            params: D.Denoise = D.Denoise(), out=None):
+    """`yk_denoise`: the edge-avoiding a-trous filter over an averaging Path / Whitted film, from the render's own
+    `radiance_sq` companion film and sample counts (`sample_counts`, an adaptive render's (H, W) counts, or `spp` for every
+    pixel), optionally guided by a `geometry_normals` / `shading_normals` companion film. Films are (H, W, 3) float32.
+    Takes numpy arrays, or CUDA tensors on the context's device, which are read and written in place after the current
+    torch stream's work; the result (`out` when given, which may be `film` itself) is of the same kind."""
+    if spp is None and sample_counts is None:
+        raise ValueError("denoise needs the samples per pixel: pass spp or sample_counts")
+    if sample_counts is None and int(spp) < 2:
+        raise ValueError(f"denoise needs at least 2 samples per pixel, got spp={spp}")
+    if not isinstance(params, D.Denoise):
+        raise ValueError(f"params must be a desc.Denoise, got {type(params).__name__}")
+    given = {"film": film, "radiance_sq": radiance_sq, "sample_counts": sample_counts, "normals": normals, "out": out}
+    given = {k: v for k, v in given.items() if v is not None}
+    import sys
+    torch = sys.modules.get("torch")   # only callers that already hold tensors have imported it
+    on_device = {k: torch is not None and isinstance(v, torch.Tensor) and v.is_cuda for k, v in given.items()}
+    if any(on_device.values()) and not all(on_device.values()):
+        raise ValueError("denoise mixes CUDA tensors and host arrays: "
+                         + ", ".join(f"{k} on {'device' if d else 'host'}" for k, d in on_device.items()))
+    shape = tuple(film.shape)
+    if len(shape) != 3 or shape[2] != 3 or shape[0] == 0 or shape[1] == 0:
+        raise ValueError(f"film must have shape (H, W, 3), got {shape}")
+    for k in ("radiance_sq", "normals", "out"):
+        if k in given and tuple(given[k].shape) != shape:
+            raise ValueError(f"{k} must have the film's shape {shape}, got {tuple(given[k].shape)}")
+    if sample_counts is not None and tuple(sample_counts.shape) != shape[:2]:
+        raise ValueError(f"sample_counts must have shape {shape[:2]}, got {tuple(sample_counts.shape)}")
+    prm = capi.DenoiseParams(0, int(params.iterations), float(params.sigma), float(params.eps), int(spp or 0), 0)
+    if all(on_device.values()):
+        for k, v in given.items():
+            if v.device.index != ctx.device_id:
+                raise ValueError(f"{k} is on {v.device}, but the context is on cuda:{ctx.device_id}")
+            want = (torch.int32, torch.uint32) if k == "sample_counts" else (torch.float32,)
+            if v.dtype not in want:
+                raise ValueError(f"{k} must be a {' or '.join(map(str, want))} tensor, got {v.dtype}")
+        if out is None:
+            out = torch.empty(shape, dtype=torch.float32, device=film.device)
+        elif not out.is_contiguous():
+            raise ValueError("out must be contiguous")
+        film, radiance_sq = film.contiguous(), radiance_sq.contiguous()
+        normals = None if normals is None else normals.contiguous()
+        sample_counts = None if sample_counts is None else sample_counts.contiguous()
+        prm.flags = capi.DENOISE_ON_DEVICE
+        prm.stream = torch.cuda.current_stream(ctx.device_id).cuda_stream
+    else:
+        film = np.ascontiguousarray(film, np.float32)
+        radiance_sq = np.ascontiguousarray(radiance_sq, np.float32)
+        normals = None if normals is None else np.ascontiguousarray(normals, np.float32)
+        sample_counts = None if sample_counts is None else np.ascontiguousarray(sample_counts, np.uint32)
+        if out is None:
+            out = np.empty(shape, np.float32)
+        elif not (isinstance(out, np.ndarray) and out.dtype == np.float32 and out.flags.c_contiguous):
+            raise ValueError("out must be a C-contiguous float32 numpy array")
+    prm.sample_counts, prm.normals = _ptr(sample_counts), _ptr(normals)
+    capi.check(capi.lib().yk_denoise(ctx._h, shape[1], shape[0], _ptr(film), _ptr(radiance_sq), C.byref(prm), _ptr(out)))
+    return out
+
+
 def load_pbrt(path: str, max_shapes_in_node: int = 1, split_method: int = D.SPLIT_SAH):
     """scene/pbrt/mod.rs `load`: pbrt-v3 file -> (SceneDesc, CameraParameters, FilmSettings), parsed by the C++ loader
     (csrc/host_pbrt.cpp). The description is copied out of the loader's storage, so it feeds the CUDA backend and the

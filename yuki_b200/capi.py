@@ -175,6 +175,14 @@ RENDER_FILM_ON_DEVICE = 1
 RENDER_AOVS = 4
 RENDER_ADAPTIVE = 8
 QUERY_ON_DEVICE = 1
+DENOISE_ON_DEVICE = 1
+
+
+class DenoiseParams(C.Structure):
+    """yk_denoise_params: the filter's settings, the per-pixel sample counts (or one count for all) and the optional guide."""
+    _fields_ = [("flags", C.c_uint32), ("iterations", C.c_uint32), ("sigma", C.c_float), ("eps", C.c_float),
+                ("samples_per_pixel", C.c_uint32), ("_reserved", C.c_uint32), ("sample_counts", C.c_void_p), ("normals", C.c_void_p),
+                ("stream", C.c_void_p)]
 
 
 class QueryOpts(C.Structure):
@@ -192,7 +200,7 @@ EXPORTS = [
     "yk_last_error", "yk_context_create", "yk_context_destroy", "yk_scene_create", "yk_scene_destroy", "yk_render",
     "yk_context_stream", "yk_bvh_build", "yk_host_scene_build", "yk_host_scene_destroy", "yk_host_scene_flat", "yk_camera_make",
     "yk_film_tiles", "yk_xf_identity", "yk_xf_translation", "yk_xf_scale", "yk_xf_rotation", "yk_xf_new", "yk_xf_look_at",
-    "yk_xf_mul", "yk_xf_inverted", "yk_xf_point", "yk_xf_vec", "yk_xf_normal", "yk_light_make", "yk_selftest_fastdiv", "yk_ply_load", "yk_ply_view", "yk_ply_destroy", "yk_write_exr", "yk_tonemap_filmic", "yk_heatmap", "yk_pbrt_load", "yk_pbrt_view", "yk_pbrt_destroy", "yk_mitsuba_load",
+    "yk_xf_mul", "yk_xf_inverted", "yk_xf_point", "yk_xf_vec", "yk_xf_normal", "yk_light_make", "yk_selftest_fastdiv", "yk_ply_load", "yk_ply_view", "yk_ply_destroy", "yk_write_exr", "yk_tonemap_filmic", "yk_heatmap", "yk_denoise", "yk_pbrt_load", "yk_pbrt_view", "yk_pbrt_destroy", "yk_mitsuba_load",
     "yk_debug_ray", "yk_trace", "yk_occluded", "yk_query_intersect", "yk_query_occluded", "yk_sampler_draws",
     "yk_multi_create", "yk_multi_destroy", "yk_multi_device_count", "yk_multi_context", "yk_multi_peer_stores",
     "yk_multi_scene_create", "yk_multi_scene_destroy", "yk_multi_render",
@@ -240,6 +248,7 @@ def lib():
     L.yk_write_exr.argtypes = [C.c_char_p, u32, u32, fp]
     L.yk_tonemap_filmic.argtypes = [vp, fp, u32, u32, fp, u32, u32, C.c_float, fp]
     L.yk_heatmap.argtypes = [vp, fp, u32, u32, u32, C.c_int, C.POINTER(C.c_float), C.POINTER(C.c_float), fp]
+    L.yk_denoise.argtypes = [vp, u32, u32, vp, vp, C.POINTER(DenoiseParams), vp]
     L.yk_pbrt_load.argtypes = [C.c_char_p, u32, u32, C.POINTER(vp)]
     L.yk_mitsuba_load.argtypes = [C.c_char_p, u32, u32, C.POINTER(vp)]
     L.yk_pbrt_view.argtypes = [vp]

@@ -654,6 +654,17 @@ int yk_context_activate(yk_context* c) {
     return YK_OK;
 }
 
+// denoise.cu: calls that use the context's stream hold its mutex
+std::recursive_mutex& yk_context_mutex(yk_context* c) { return c->mu; }
+
+// denoise.cu, device arrays: the context's stream is non-blocking, so without this event it would not order after the work
+// already queued on the caller's stream (as query_run does; ev[1] is only used under the context mutex)
+int yk_context_follow(yk_context* c, void* caller_stream) {
+    CUDA_TRY(cudaEventRecord(c->ev[1], (cudaStream_t)caller_stream));
+    CUDA_TRY(cudaStreamWaitEvent(c->stream, c->ev[1], 0));
+    return YK_OK;
+}
+
 extern "C" {
 
 int yk_context_create(int device_id, yk_context** out) {

@@ -177,3 +177,22 @@ class Adaptive:                             # yk_adaptive (include/yuki_gpu.h): 
     step: int = 16
     rel_error: float = 0.05
     abs_error: float = 0.0
+
+
+@dataclass(frozen=True)
+class Denoise:                              # yk_denoise_params (include/yuki_gpu.h): no counterpart in the reference
+    """The a-trous denoiser's settings: `iterations` passes (1 ... 10) at steps 1, 2, 4, ...; colour weights
+    (1 + |dc|^2 / (sigma^2 (var_p + var_q) + eps))^-2."""
+    iterations: int = 5
+    sigma: float = 2.0
+    eps: float = 1e-4
+
+    def __post_init__(self):
+        if isinstance(self.iterations, bool) or int(self.iterations) != self.iterations or not 1 <= int(self.iterations) <= 10:
+            raise ValueError(f"Denoise.iterations must be an integer in 1 ... 10, got {self.iterations!r}")
+        for name in ("sigma", "eps"):
+            v = float(getattr(self, name))
+            with np.errstate(over="ignore"):
+                f = float(np.float32(v))
+            if not 0.0 < f <= float(np.finfo(np.float32).max):   # (NaN fails the comparison)
+                raise ValueError(f"Denoise.{name} must be > 0 and finite in float32, got {v}")

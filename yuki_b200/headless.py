@@ -75,10 +75,32 @@ def parse_args(argv=None):
     ap.add_argument("--adaptive-step", type=int, default=16, metavar="N", help="then a check every N samples")
     ap.add_argument("--sample-counts", default=None, metavar="PATH",
                     help="with --adaptive: write each pixel's sample count (in all three channels) as a raw EXR")
+    ap.add_argument("--denoise", action="store_true",
+                    help="denoise the film before the tone map (Path / Whitted): an a-trous filter guided by the render's own "
+                         "radiance_sq and shading_normals companion films and, with --adaptive, its sample counts")
+    ap.add_argument("--denoise-sigma", type=float, default=D.Denoise.sigma, metavar="S")
+    ap.add_argument("--denoise-iterations", type=int, default=D.Denoise.iterations, metavar="K", help="1 ... 10")
     args = ap.parse_args(argv)
     if args.sample_counts is not None and args.adaptive is None:
         ap.error("--sample-counts needs --adaptive")
+    if args.denoise:
+        if args.integrator not in ("path", "whitted"):
+            ap.error("--denoise needs the Path or Whitted integrator")
+        try:
+            denoise_from_args(args)
+            sampler, _ = settings_from_args(args)
+        except ValueError as e:
+            ap.error(str(e))
+        if args.adaptive is None and sampler.samples_per_pixel() < 2:
+            ap.error("--denoise needs at least 2 samples per pixel")
     return args
+
+
+def denoise_from_args(args):
+    """--denoise [--denoise-sigma S --denoise-iterations K] -> D.Denoise, or None."""
+    if not args.denoise:
+        return None
+    return D.Denoise(args.denoise_iterations, args.denoise_sigma)
 
 
 def adaptive_from_args(args):
@@ -132,7 +154,9 @@ def render(args, out=sys.stdout) -> np.ndarray:
     film = api.Film(film_settings)
     rn = api.Renderer(ctx)
     start = time.perf_counter()
-    rn.launch(dev, cam, film, sampler, integrator, aovs=[name for name, _ in args.aov], adaptive=adaptive_from_args(args))
+    denoise = denoise_from_args(args)
+    aovs = [name for name, _ in args.aov] + (["radiance_sq", "shading_normals"] if denoise else [])
+    rn.launch(dev, cam, film, sampler, integrator, aovs=aovs, adaptive=adaptive_from_args(args))
     width = 0
     while True:   # headless.rs:51-110
         st = rn.check_status()
@@ -150,6 +174,11 @@ def render(args, out=sys.stdout) -> np.ndarray:
             print(f"\r{line:<{width}}", end="", file=out, flush=True)
         time.sleep(0.01)
     pixels = film.pixels
+    if denoise is not None:
+        res = rn.last_result
+        pixels = api.denoise(ctx, pixels, res.aovs["radiance_sq"], spp=sampler.samples_per_pixel(), sample_counts=res.sample_counts,
+                             normals=res.aovs["shading_normals"], params=denoise)
+        print(f"Denoised: {denoise.iterations} iterations, sigma {denoise.sigma:g}", file=out)
     if args.tone_map == "filmic":
         pixels = api.tonemap_filmic(ctx, pixels, args.exposure)
     elif args.tone_map == "heatmap":
