@@ -187,6 +187,7 @@ typedef struct {
 #define YK_RENDER_AOVS 4u            /* read opts.aovs: companion films of the same render (Path / Whitted only; not yk_multi_render) */
 #define YK_RENDER_ADAPTIVE 8u        /* read opts.adaptive: stop each pixel once its mean is precise enough (Path / Whitted, averaging
                                         films only; not yk_multi_render) */
+#define YK_RENDER_THIN_LENS 32u      /* read opts.lens: depth of field through a thin lens (yk_thin_lens) */
 #define YK_RAY_SORT_TRACE_ONLY 16u   /* yk_render_opts.ray_sort flag: only the closest-hit kernel walks the sorted order (default: the
                                         material sort does too, so shading and shadow rays run in the same order) */
 
@@ -216,6 +217,23 @@ typedef struct {
     uint32_t* sample_counts;   /* optional res_y*res_x out: samples taken per pixel; host, or device with YK_RENDER_FILM_ON_DEVICE */
 } yk_adaptive;
 
+/* Thin-lens camera (YK_RENDER_THIN_LENS): pbrt-v3's PerspectiveCamera::GenerateRay with lensradius R and focaldistance F. Camera
+ * space looks down +z. With R > 0 a camera sample draws the film jitter j = get_2d() (dimensions 0-1) and then the lens sample
+ * u = get_2d() (dimensions 2-3), so every later draw of the integrator moves up by 2 dimensions; every op un-fused IEEE float32,
+ * in this order:
+ *     p_cam = xf_point(raster_to_camera, (x + j.x, y + j.y, 0));  d = unit(p_cam)
+ *     l = concentric_sample_disk(u);  lx = R * l.x;  ly = R * l.y      (sampling/mod.rs:68-87, glibc-exact sinf / cosf)
+ *     ft = F / d.z;  f = d * ft                                        (the point on the plane of focus)
+ *     o_cam = (lx, ly, 0);  d_cam = unit(f - o_cam)
+ *     ray = (xf_point(camera_to_world, o_cam), xf_vec(camera_to_world, d_cam)), t_max = inf
+ * Points at depth F are sharp; a point at depth z is spread over a disk of radius R * |1 - z / F| around its pinhole image.
+ * R = 0 is the pinhole: no lens sample is drawn and the render is the plain one, bit for bit. Works with every integrator,
+ * accumulating films, YK_RENDER_AOVS, YK_RENDER_ADAPTIVE and yk_multi_render. yk_debug_ray has no options and stays pinhole. */
+typedef struct {
+    float lens_radius;         /* >= 0 and finite */
+    float focal_distance;      /* > 0 and finite (pbrt-v3's default: 1e6) */
+} yk_thin_lens;
+
 typedef int (*yk_progress_fn)(void* user, uint64_t samples_done, uint64_t samples_total); /* return !=0 to cancel */
 
 typedef struct {
@@ -234,6 +252,7 @@ typedef struct {
     uint32_t _reserved;
     const yk_aov_films* aovs;   /* read only when flags & YK_RENDER_AOVS (callers built against the shorter struct never set it) */
     const yk_adaptive* adaptive;  /* read only when flags & YK_RENDER_ADAPTIVE */
+    const yk_thin_lens* lens;     /* read only when flags & YK_RENDER_THIN_LENS */
 } yk_render_opts;
 
 typedef struct {
@@ -277,7 +296,9 @@ void yk_scene_destroy(yk_scene*);
  * traversal counters count the samples traced, the progress callback reports (done, spp * pixels) and at the end (total,
  * total), and hit_ids holds -1 for a pixel that stopped before `aux_sample`. Refused (YK_ERR_INVALID, nothing launched)
  * when opts->adaptive is NULL, min_samples < 2, step is 0, a tolerance is negative or not finite, the film accumulates or
- * the integrator is a debug one; yk_multi_render refuses the flag. min_samples >= spp is the plain render. */
+ * the integrator is a debug one; yk_multi_render refuses the flag. min_samples >= spp is the plain render.
+ * With YK_RENDER_THIN_LENS the camera rays leave through opts->lens (yk_thin_lens). Refused (YK_ERR_INVALID, nothing launched)
+ * when opts->lens is NULL, the radius is negative or not finite, or the focal distance is not > 0 and finite. */
 int yk_render(yk_context*, const yk_scene*, const yk_camera*, const yk_film_settings*, const yk_sampler*,
               const yk_integrator*, const yk_tile* tiles, uint32_t n_tiles, const yk_render_opts* opts,
               float* film_rgb, yk_stats* stats);
@@ -286,7 +307,7 @@ int yk_render(yk_context*, const yk_scene*, const yk_camera*, const yk_film_sett
  * window.rs:884) and returns the rays the integrator collects for the ray visualisation (path.rs:71-153,
  * whitted.rs:89-170), in the reference's order. Writes at most `cap` rays; *n_rays is the number collected. `li_rgb`
  * (3 floats) and `ray_count` are li_debug's RadianceResult. The debug integrators keep the trait's default: no rays, zero
- * radiance, zero ray count. */
+ * radiance, zero ray count. The camera is the pinhole: yk_debug_ray takes no yk_render_opts, hence no yk_thin_lens. */
 int yk_debug_ray(yk_context*, const yk_scene*, const yk_camera*, const yk_sampler*, const yk_integrator*,
                  uint32_t film_px_x, uint32_t film_px_y, yk_integrator_ray* rays, uint32_t cap, uint32_t* n_rays,
                  float* li_rgb, uint64_t* ray_count);
@@ -451,6 +472,7 @@ typedef struct {
     yk_host_scene_desc scene;
     yk_camera_params camera;
     uint32_t res_x, res_y;
+    float lens_radius, focal_distance;  /* Camera "perspective" lensradius (default 0) / focaldistance (default 1e6); Mitsuba: 0 / 1e6 */
 } yk_pbrt_result;
 int yk_pbrt_load(const char* path, uint32_t max_shapes_in_node, uint32_t split_method, yk_pbrt_scene** out);
 /* Mitsuba 2.1.0 XML scene file -> the same result type (read with yk_pbrt_view, freed with yk_pbrt_destroy): the

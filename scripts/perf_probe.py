@@ -270,3 +270,33 @@ if which == "denoise":  # yk_denoise at 1080p and 4K next to the 16-spp renders 
     denoise_table("C4 material room 1920x1080", s, c, D.FilmSettings((1920, 1080), 16))
     s, c = scenes.terrain_room(xf)
     denoise_table("C5 terrain 10M 3840x2160", s, c, D.FilmSettings((3840, 2160), 16))
+if which == "lens":  # thin lens (depth of field) against the pinhole: device time of C2 and C4 with a small and a large blur
+    import subprocess
+    print(subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv"], capture_output=True, text=True).stdout.strip(), flush=True)
+
+    def lens_table(name, s, c, film, smp, reps=3):
+        """The plane of focus through the surface at the film centre (depth z_c); radii chosen so that a point at 1.25 z_c is
+        blurred over a disk of about 4 and about 40 pixels (diameter R * 0.2 * 2 / its pixel footprint)."""
+        ctx = api.Context(0); dev = api.Scene(ctx, s); rn = api.Renderer(ctx)
+        pos, tgt = np.array(c.position, np.float64), np.array(c.target, np.float64)
+        fwd = (tgt - pos) / np.linalg.norm(tgt - pos)
+        t, _, _ = dev.intersect(pos[None].astype(np.float32), fwd[None].astype(np.float32))
+        z_c = float(t[0])
+        px = 1.25 * z_c * 2.0 * np.tan(np.radians(c.fov_deg) / 2.0) / film.res[0]
+        runs = [("pinhole", None)] + [(f"{d:>2d} px blur (R {d * px / 0.4:.4f}, F {z_c:.3f})", D.ThinLens(d * px / 0.4, z_c)) for d in (4, 40)]
+        best = {}
+        for rep in range(reps + 1):  # round-robin; the first round warms up
+            for label, lens in runs:
+                st = rn.render(dev, c, film, smp, D.IntegratorType.path(8), lens=lens).stats
+                if rep and (label not in best or st.device_ms < best[label].device_ms):
+                    best[label] = st
+        base = best["pinhole"].device_ms
+        for label, _ in runs:
+            st = best[label]
+            print(f"{name} | {label:<38}: device {st.device_ms:8.2f} ms ({st.device_ms / base:5.3f}x), closest-hit {st.trace_closest_ms:7.2f} ms, "
+                  f"{st.samples / st.device_ms * 1e-3:7.1f} Msamples/s, closest nodes/ray {st.closest_nodes / max(st.ray_count, 1):5.1f}", flush=True)
+        dev.close(); ctx.close()
+    s, c = scenes.cornell(xf, light="rect", tall_box="glass")
+    lens_table("C2 cornell 1024^2 path8 64spp", s, c, D.FilmSettings((1024, 1024), 16), D.SamplerType.stratified(8, 8))
+    s, c = scenes.material_room(xf)
+    lens_table("C4 material room 1920x1080 path8 16spp", s, c, D.FilmSettings((1920, 1080), 16), D.SamplerType.stratified(4, 4))

@@ -378,9 +378,10 @@ class MultiScene:
 def multi_render(mctx: MultiContext, scene: MultiScene, camera_params: D.CameraParameters, film: D.FilmSettings, sampler: D.SamplerType,
                  integrator: D.IntegratorType, tiles: Optional[np.ndarray] = None, want_hit_ids: bool = False, aux_sample: int = 0,
                  film_out: Optional[np.ndarray] = None, device_film_ptr: Optional[int] = None, pipes: int = 0, ray_sort: int = 0,
-                 wavefront_paths: int = 0):
+                 wavefront_paths: int = 0, lens: Optional[D.ThinLens] = None):
     """`yk_multi_render`: the tile list rendered by all devices of the group, popped from one shared cursor; the film is
-    assembled on the first device by peer stores. Returns (RenderResult with the summed stats, per-device stats list)."""
+    assembled on the first device by peer stores. `lens` (D.ThinLens): depth of field, as in `Renderer.render`.
+    Returns (RenderResult with the summed stats, per-device stats list)."""
     cam = make_camera(camera_params, film)
     if tiles is None:
         tiles = film_tiles(film)
@@ -391,6 +392,7 @@ def multi_render(mctx: MultiContext, scene: MultiScene, camera_params: D.CameraP
     opts.pipes = pipes
     opts.ray_sort = ray_sort
     opts.wavefront_paths = wavefront_paths
+    _set_lens(opts, lens)
     hit_ids = None
     if device_film_ptr is not None:
         opts.flags |= capi.RENDER_FILM_ON_DEVICE
@@ -408,6 +410,16 @@ def multi_render(mctx: MultiContext, scene: MultiScene, camera_params: D.CameraP
     capi.check(capi.lib().yk_multi_render(mctx._h, scene._h, C.byref(cam), C.byref(fs), C.byref(sm), C.byref(ig),
                                           C.c_void_p(tiles.ctypes.data), len(tiles), C.byref(opts), film_ptr, C.byref(stats), per))
     return RenderResult(film_arr, hit_ids, stats), list(per)
+
+
+def _set_lens(opts: capi.RenderOpts, lens: Optional[D.ThinLens]) -> None:
+    """Points `opts` at a yk_thin_lens for `lens` (None: the pinhole, and the flag stays clear)."""
+    if lens is None:
+        return
+    if not isinstance(lens, D.ThinLens):
+        raise TypeError(f"lens must be a desc.ThinLens, got {type(lens).__name__}")
+    opts.flags |= capi.RENDER_THIN_LENS
+    opts.lens = C.pointer(capi.ThinLens(float(lens.radius), float(lens.focal_distance)))
 
 
 def sampler_draws(ctx: Context, sampler: D.SamplerType, pixel_index, pattern) -> np.ndarray:
@@ -531,11 +543,12 @@ def denoise(ctx: Context, film, radiance_sq, *, spp: Optional[int] = None, sampl
     return out
 
 
-def load_pbrt(path: str, max_shapes_in_node: int = 1, split_method: int = D.SPLIT_SAH):
+def load_pbrt(path: str, max_shapes_in_node: int = 1, split_method: int = D.SPLIT_SAH, with_lens: bool = False):
     """scene/pbrt/mod.rs `load`: pbrt-v3 file -> (SceneDesc, CameraParameters, FilmSettings), parsed by the C++ loader
     (csrc/host_pbrt.cpp). The description is copied out of the loader's storage, so it feeds the CUDA backend and the
-    test oracle exactly like the programmatic scenes."""
-    return _load_scene_file(capi.lib().yk_pbrt_load, path, max_shapes_in_node, split_method)
+    test oracle exactly like the programmatic scenes. `with_lens`: also return the camera's D.ThinLens (its `lensradius`,
+    default 0, and `focaldistance`, default 1e6), which the reference ignores."""
+    return _load_scene_file(capi.lib().yk_pbrt_load, path, max_shapes_in_node, split_method, with_lens)
 
 
 def load_mitsuba(path: str, max_shapes_in_node: int = 1, split_method: int = D.SPLIT_SAH):
@@ -544,7 +557,7 @@ def load_mitsuba(path: str, max_shapes_in_node: int = 1, split_method: int = D.S
     return _load_scene_file(capi.lib().yk_mitsuba_load, path, max_shapes_in_node, split_method)
 
 
-def _load_scene_file(loader, path, max_shapes_in_node, split_method):
+def _load_scene_file(loader, path, max_shapes_in_node, split_method, with_lens=False):
     h = C.c_void_p()
     capi.check(loader(str(path).encode(), int(max_shapes_in_node), int(split_method), C.byref(h)))
     try:
@@ -588,9 +601,10 @@ def _load_scene_file(loader, path, max_shapes_in_node, split_method):
         cam = D.CameraParameters(tuple(float(v) for v in r.camera.position), tuple(float(v) for v in r.camera.target),
                                  tuple(float(v) for v in r.camera.up), int(r.camera.fov_axis), float(r.camera.fov_deg))
         film = D.FilmSettings((int(r.res_x), int(r.res_y)), 16)
+        lens = D.ThinLens(float(r.lens_radius), float(r.focal_distance)) if with_lens else None
     finally:
         capi.lib().yk_pbrt_destroy(h)
-    return sc, cam, film
+    return (sc, cam, film, lens) if with_lens else (sc, cam, film)
 
 
 def load_ply(path: str):
@@ -856,6 +870,9 @@ class Renderer:
         meta = {"spp": spp, "sampler": [sampler.kind, sampler.nx, sampler.ny, bool(sampler.jitter), int(sampler.seed)],
                 "integrator": [integrator.kind, integrator.max_depth, None if clamp is None else float(clamp)],
                 "camera": hashlib.sha256(cam_bytes).hexdigest()[:16], "scene": scene_id}
+        lens = render_kw.get("lens")
+        if lens is not None and float(lens.radius) > 0.0:   # (a radius-0 lens renders the pinhole's film: no key, as before)
+            meta["lens"] = [float(np.float32(lens.radius)), float(np.float32(lens.focal_distance))]
         if film.meta and film.meta != json_roundtrip(meta):
             raise ValueError(f"film was rendered with other settings: {film.meta}")
         film.meta = json_roundtrip(meta)
@@ -924,13 +941,15 @@ class Renderer:
                integrator: D.IntegratorType, tiles: Optional[np.ndarray] = None, want_hit_ids: bool = False,
                aux_sample: int = 0, wavefront_paths: int = 0, film_out: Optional[np.ndarray] = None,
                device_film_ptr: Optional[int] = None, progress=None, pipes: int = 0, ray_sort: int = 0, aovs=None,
-               aov_out: Optional[dict] = None, adaptive: Optional[D.Adaptive] = None, sample_counts_out=None) -> RenderResult:
+               aov_out: Optional[dict] = None, adaptive: Optional[D.Adaptive] = None, sample_counts_out=None,
+               lens: Optional[D.ThinLens] = None) -> RenderResult:
         """`aovs`: names of companion films (capi.AOV_NAMES) rendered from the same camera rays, returned in
         RenderResult.aovs as (res_y, res_x, 3) float32 arrays. `aov_out` maps names to the arrays to render into (accumulating
         or keep-film renders, like `film_out`), or, with `device_film_ptr`, to device pointers; its names are requested too.
         `adaptive` (D.Adaptive): stop each pixel once its mean is precise enough; RenderResult.sample_counts is then the
         (res_y, res_x) uint32 array of samples per pixel: `sample_counts_out` if given (pixels outside `tiles` keep their
-        values), or, with `device_film_ptr`, the device pointer `sample_counts_out` (None: no counts)."""
+        values), or, with `device_film_ptr`, the device pointer `sample_counts_out` (None: no counts).
+        `lens` (D.ThinLens): depth of field through a thin lens, with any integrator; None or radius 0 is the pinhole."""
         names = aov_names(aovs, aov_out)
         check_adaptive(adaptive, film, integrator)
         if sample_counts_out is not None and adaptive is None:
@@ -945,6 +964,7 @@ class Renderer:
         opts.aux_sample = aux_sample
         opts.pipes = pipes
         opts.ray_sort = ray_sort   # 0 default, 1 off, 2 leaf-slot key, 3 Morton key (yk_render_opts.ray_sort)
+        _set_lens(opts, lens)
         hit_ids = None
         if device_film_ptr is not None:
             opts.flags |= capi.RENDER_FILM_ON_DEVICE

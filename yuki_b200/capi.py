@@ -106,7 +106,8 @@ class HostSceneDesc(C.Structure):
 
 
 class PbrtResult(C.Structure):
-    _fields_ = [("scene", HostSceneDesc), ("camera", CameraParams), ("res_x", C.c_uint32), ("res_y", C.c_uint32)]
+    _fields_ = [("scene", HostSceneDesc), ("camera", CameraParams), ("res_x", C.c_uint32), ("res_y", C.c_uint32),
+                ("lens_radius", C.c_float), ("focal_distance", C.c_float)]
 
 
 class SphereDev(C.Structure):
@@ -154,10 +155,16 @@ class Adaptive(C.Structure):
                 ("sample_counts", C.c_void_p)]
 
 
+class ThinLens(C.Structure):
+    """yk_thin_lens: depth of field through a thin lens (YK_RENDER_THIN_LENS)."""
+    _fields_ = [("lens_radius", C.c_float), ("focal_distance", C.c_float)]
+
+
 class RenderOpts(C.Structure):
     _fields_ = [("flags", C.c_uint32), ("wavefront_paths", C.c_uint32), ("hit_ids", C.c_void_p), ("aux_sample", C.c_uint32),
                 ("pipes", C.c_uint32), ("progress", PROGRESS_FN), ("progress_user", C.c_void_p), ("ray_sort", C.c_uint32),
-                ("_reserved", C.c_uint32), ("aovs", C.POINTER(AovFilms)), ("adaptive", C.POINTER(Adaptive))]
+                ("_reserved", C.c_uint32), ("aovs", C.POINTER(AovFilms)), ("adaptive", C.POINTER(Adaptive)),
+                ("lens", C.POINTER(ThinLens))]
 
 
 class Stats(C.Structure):
@@ -174,6 +181,7 @@ class Stats(C.Structure):
 RENDER_FILM_ON_DEVICE = 1
 RENDER_AOVS = 4
 RENDER_ADAPTIVE = 8
+RENDER_THIN_LENS = 32
 QUERY_ON_DEVICE = 1
 DENOISE_ON_DEVICE = 1
 

@@ -781,6 +781,8 @@ extern "C" int yk_mitsuba_load(const char* path, uint32_t max_shapes_in_node, ui
     r.camera.fov_axis = YK_FOV_X;
     r.res_x = 640;
     r.res_y = 480;
+    r.lens_radius = 0.0f;  // a pinhole: the thinlens sensor is not read
+    r.focal_distance = 1e6f;
     if (!ld.top(root)) return yk_set_error(YK_ERR_INVALID, "mitsuba: " + ld.error);
     if (!ld.have_shapes) return yk_set_error(YK_ERR_INVALID, "mitsuba: the scene has no shapes (bvh.rs:68 needs at least one)");
     ld.retarget_camera();

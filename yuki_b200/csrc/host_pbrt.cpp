@@ -12,6 +12,8 @@
 //     converted with the Wyman-Sloan-Shirley CIE fits, cie.rs), point, normal, blackbody (dropped), texture;
 //   * materials glass / glossy / matte (sigma through to_radians twice, mod.rs:904-907) / metal (copper defaults);
 //     unknown types fall back to grey matte; fov is vertical unless the film is taller than wide (mod.rs:827-835).
+//   * Camera "perspective" also yields pbrt-v3's lensradius (default 0) and focaldistance (default 1e6), which the reference
+//     ignores; a caller renders with them through YK_RENDER_THIN_LENS.
 // Image textures are decoded here for PNG only (the reference uses the `image` crate, which is not vendored): 8/16-bit
 // RGB / RGBA / palette, non-interlaced; other layouts are the reference's "Unsupported image format".
 #include <zlib.h>
@@ -522,6 +524,7 @@ struct Parser {
         cam = yk_camera_params{{0, 0, 0}, {0, 0, 0}, {0, 1, 0}, YK_FOV_X, 0.0f};
         uint32_t res_x = 640, res_y = 480;  // FilmSettings::default, film.rs:25-38
         float fov = 0.0f;
+        float lens_radius = 0.0f, focal_distance = 1e6f;  // pbrt-v3's PerspectiveCamera defaults
         struct Graphics { int32_t material; };
         ParamSet none;
         if (!material("matte", none, &default_material)) return false;
@@ -572,6 +575,8 @@ struct Parser {
                     if (name != "perspective") return fail("Only perspective camera is supported");
                     if (!param_set(&ps)) return false;
                     fov = ParamSet::one(ps.f32s, "fov", 45.0f);
+                    lens_radius = ParamSet::one(ps.f32s, "lensradius", 0.0f);
+                    focal_distance = ParamSet::one(ps.f32s, "focaldistance", 1e6f);
                 } break;
                 case Tok::Film: {
                     std::string name;
@@ -743,6 +748,8 @@ struct Parser {
         cam.fov_deg = fov;
         out->result.res_x = res_x;
         out->result.res_y = res_y;
+        out->result.lens_radius = lens_radius;
+        out->result.focal_distance = focal_distance;
         std::memcpy(out->result.scene.background, background, 12);
         return true;
     }

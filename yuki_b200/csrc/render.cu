@@ -408,9 +408,9 @@ int retire_slot(Pipe* p, int k, Timers* tm, uint64_t* done_paths) {
 // One batch on one pipe: raygen, the bounce loop, and the per-batch film step, all asynchronous on the pipe's stream.
 // Path tracing runs exactly max_depth bounces (every queue length stays on the device); Whitted's tree walk has no
 // such bound, so it reads the next bounce's ray count back once per bounce.
-// `aov`: the companion films' sums (AovSums; all null = none requested).
+// `aov`: the companion films' sums (AovSums; all null = none requested). `lens`: a thin lens with a radius > 0, or null (pinhole).
 int run_batch(yk_context* c, Pipe* p, const yk_scene* sc, const RenderCfg& cfg, const Batch& bt, uint32_t first_sample, bool accumulate_film,
-              float* d_film, const AovSums& aov, Timers* tm, uint64_t* done_paths) {
+              float* d_film, const AovSums& aov, const yk_thin_lens* lens, Timers* tm, uint64_t* done_paths) {
     cudaStream_t s = p->stream;
     Wave& w = p->wave;
     const int k = (int)(p->n_batches % kRing);
@@ -439,7 +439,10 @@ int run_batch(yk_context* c, Pipe* p, const yk_scene* sc, const RenderCfg& cfg, 
     nvtxRangePushA("yk raygen");
     k_sample_jumps<<<1, kMaxBatchSamples, 0, s>>>(first_sample, bt.n_samples, p->d_jumps);
     tm->launches += 1;
-    k_raygen<<<(bt.n_paths + T - 1) / T, T, 0, s>>>(w, cfg, bt, first_sample, bt.n_samples, p->d_jumps, &p->d_ctr[0]);
+    if (lens)
+        k_raygen_lens<<<(bt.n_paths + T - 1) / T, T, 0, s>>>(w, cfg, bt, first_sample, bt.n_samples, p->d_jumps, &p->d_ctr[0],
+                                                             lens->lens_radius, lens->focal_distance);
+    else k_raygen<<<(bt.n_paths + T - 1) / T, T, 0, s>>>(w, cfg, bt, first_sample, bt.n_samples, p->d_jumps, &p->d_ctr[0]);
     nvtxRangePop();
     tm->launches += 1;
     const bool debug = cfg.integrator >= YK_INTEGRATOR_BVH_INTERSECTIONS;
@@ -1082,6 +1085,21 @@ static void aov_views(const yk_aov_films* a, float* (&v)[kAovViews]) {
     v[0] = a->bvh_intersections; v[1] = a->geometry_normals; v[2] = a->shading_normals; v[3] = a->shading_uvs; v[4] = a->radiance_sq;
 }
 
+// opts->lens when YK_RENDER_THIN_LENS is set, validated; *out = null for the pinhole (no flag, or a lens of radius 0: the plain
+// render, bit for bit)
+static int thin_lens_of(const yk_render_opts* opts, const char* fn, const yk_thin_lens** out) {
+    *out = nullptr;
+    if (!opts || !(opts->flags & YK_RENDER_THIN_LENS)) return YK_OK;
+    const yk_thin_lens* l = opts->lens;
+    if (!l) return yk_set_error(YK_ERR_INVALID, std::string(fn) + ": YK_RENDER_THIN_LENS without opts->lens");
+    if (!std::isfinite(l->lens_radius) || !(l->lens_radius >= 0.0f))
+        return yk_set_error(YK_ERR_INVALID, std::string(fn) + ": the lens radius must be finite and >= 0");
+    if (!std::isfinite(l->focal_distance) || !(l->focal_distance > 0.0f))
+        return yk_set_error(YK_ERR_INVALID, std::string(fn) + ": the focal distance must be finite and > 0");
+    if (l->lens_radius > 0.0f) *out = l;
+    return YK_OK;
+}
+
 // yk_render, and yk_debug_ray's single path (`debug_log` = device ray list, `debug_px` = the film pixel of its camera sample).
 static int render_impl(yk_context* c, const yk_scene* sc, const yk_camera* cam, const yk_film_settings* fs, const yk_sampler* sm,
                        const yk_integrator* in, const yk_tile* tiles, uint32_t n_tiles, const yk_render_opts* opts, float* film_rgb,
@@ -1121,6 +1139,8 @@ static int render_impl(yk_context* c, const yk_scene* sc, const yk_camera* cam, 
             return yk_set_error(YK_ERR_INVALID, "yk_render: adaptive sampling needs the Path or Whitted integrator");
         adaptive = a;
     }
+    const yk_thin_lens* lens = nullptr;
+    if (int rc = thin_lens_of(opts, "yk_render", &lens)) return rc;
     std::lock_guard<std::recursive_mutex> guard(c->mu);
     CUDA_TRY(cudaSetDevice(c->device));
     (void)cudaGetLastError();  // do not inherit a stale error from an unrelated earlier call
@@ -1432,10 +1452,11 @@ static int render_impl(yk_context* c, const yk_scene* sc, const yk_camera* cam, 
                     RenderCfg gcfg = cfg;
                     if (sm->kind == YK_SAMPLER_STRATIFIED) {
                         // tabulate the (pixel, dimension) hashes of this pixel group once for all of its samples
-                        uint64_t dims = 2;
-                        if (in->kind == YK_INTEGRATOR_PATH) dims = 2 + (uint64_t)in->max_depth * (2ull * sc->dev.n_lights + 3);
+                        const uint64_t camera_dims = lens ? 4 : 2;  // the film jitter, and the lens sample
+                        uint64_t dims = camera_dims;
+                        if (in->kind == YK_INTEGRATOR_PATH) dims = camera_dims + (uint64_t)in->max_depth * (2ull * sc->dev.n_lights + 3);
                         else if (in->kind == YK_INTEGRATOR_WHITTED)
-                            dims = 2 + 2ull * sc->dev.n_lights * ((1ull << std::min(in->max_depth, 8u)) - 1);
+                            dims = camera_dims + 2ull * sc->dev.n_lights * ((1ull << std::min(in->max_depth, 8u)) - 1);
                         dims = std::min<uint64_t>(dims, std::min<uint64_t>(4096, (256ull << 20) / (4ull * nj)));  // the rest is hashed on the fly
                         if (p.hash_group != group || p.rehash) {
                             const size_t need = (size_t)dims * nj;
@@ -1466,7 +1487,7 @@ static int render_impl(yk_context* c, const yk_scene* sc, const yk_camera* cam, 
                     bt.n_paths = nj * bt.n_samples;
                     // the batch's first sample index: s0, or the sample of the group's tiles (accumulating films: one per group)
                     const uint32_t first_sample = accumulate ? (uint32_t)tiles[groups[group].t_lo].sample : s0;
-                    rc = run_batch(c, &p, sc, gcfg, bt, first_sample, accumulate, d_film, aov_sums, &tm, &done);
+                    rc = run_batch(c, &p, sc, gcfg, bt, first_sample, accumulate, d_film, aov_sums, lens, &tm, &done);
                     if (rc != YK_OK) {  // nothing may stay in flight or marked busy behind an error return
                         cudaDeviceSynchronize();
                         for (Pipe& q : c->pipe)

@@ -67,6 +67,16 @@ __global__ void k_sample_jumps(uint32_t first_sample, uint32_t n, SampleJump* ju
     }
     jumps[k] = SampleJump{am, ap};
 }
+// sampling/mod.rs:68-87 (ConcentricSampleDisk), the map cosine_hemisphere inlines; restated here so that the shading kernels'
+// code stays as it is
+__device__ __forceinline__ V2 concentric_disk(V2 u) {
+    const float ox = u.x * 2.0f - 1.0f, oy = u.y * 2.0f - 1.0f;
+    if (ox == 0.0f && oy == 0.0f) return {0.0f, 0.0f};
+    float theta, r;
+    if (fabsf(ox) > fabsf(oy)) { theta = kPiOver4 * (oy / ox); r = ox; }
+    else { theta = kPiOver2 - kPiOver4 * (ox / oy); r = oy; }
+    return {cos_f32(theta) * r, sin_f32(theta) * r};
+}
 __global__ void k_raygen(Wave w, RenderCfg cfg, Batch bt, uint32_t first_sample, uint32_t n_jumps, const SampleJump* jumps, IterCounters* first) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= bt.n_paths) return;
@@ -93,6 +103,45 @@ __global__ void k_raygen(Wave w, RenderCfg cfg, Batch bt, uint32_t first_sample,
     const V3 d_cam = unit(p_cam);
     const V3 o = xf_point(cfg.c2w, mk(0.0f, 0.0f, 0.0f));
     const V3 d = xf_vec(cfg.c2w, d_cam);
+    st_once(&w.st[0].ray_o[i], make_float4(o.x, o.y, o.z, __int_as_float(0x7f800000)));
+    st_once(&w.st[0].ray_d[i], make_float4(d.x, d.y, d.z, 0.0f));
+    st_once(&w.st[0].rng[i], (unsigned long long)s.rng.state);
+    if (cfg.integrator == YK_INTEGRATOR_WHITTED) st_once(&w.st[0].beta[i], make_float4(__uint_as_float(s.dim), 1.0f, 1.0f, __uint_as_float(kFlagAlive)));
+    else st_once(&w.st[0].beta[i], make_float4(1.0f, 1.0f, 1.0f, __uint_as_float(kFlagAlive | (s.dim << kDimShift))));
+    st_once(&w.L[i], make_float4(0.0f, 0.0f, 0.0f, 0.0f));
+}
+
+// k_raygen for a thin lens of radius > 0 (yk_thin_lens, include/yuki_gpu.h: pbrt-v3's PerspectiveCamera::GenerateRay): the path's
+// second get_2d is the lens sample. A kernel of its own, so that the pinhole's code stays as it is.
+__global__ void k_raygen_lens(Wave w, RenderCfg cfg, Batch bt, uint32_t first_sample, uint32_t n_jumps, const SampleJump* jumps, IterCounters* first,
+                              float lens_radius, float focal_distance) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= bt.n_paths) return;
+    if (i == 0) first->n_active = bt.n_paths;
+    const uint32_t si = bt.div_jobs.div(i), ji = i - si * bt.n_jobs;
+    const Job job = bt.jobs[ji];
+    const uint32_t sample = job.sample_begin + bt.sample_off + si;
+    SamplerState s;
+    const uint32_t slot = sample - first_sample;
+    if (slot < n_jumps) {
+        s.px = job.x; s.py = job.y; s.index = sample; s.dim = 0; s.job = ji;
+        s.rng.inc = job.rng_inc;
+        const unsigned long long seeded = (cfg.sampler.seed + job.rng_inc) * kPcgMult + job.rng_inc;
+        const SampleJump j = jumps[slot];
+        s.rng.state = j.mult * seeded + job.rng_inc * j.plus;
+    } else {
+        s.start(cfg.sampler, job.x, job.y, sample, job.rng_inc, ji);
+    }
+    const V2 j = s.get_2d(cfg.sampler);
+    const V3 p_cam = xf_point(cfg.r2c, mk((float)job.x + j.x, (float)job.y + j.y, 0.0f));
+    const V3 d_cam = unit(p_cam);
+    const V2 l = concentric_disk(s.get_2d(cfg.sampler));
+    const float lx = lens_radius * l.x, ly = lens_radius * l.y;
+    const float ft = focal_distance / d_cam.z;
+    const V3 f = d_cam * ft;  // the point on the plane of focus
+    const V3 o_cam = mk(lx, ly, 0.0f);
+    const V3 o = xf_point(cfg.c2w, o_cam);
+    const V3 d = xf_vec(cfg.c2w, unit(f - o_cam));
     st_once(&w.st[0].ray_o[i], make_float4(o.x, o.y, o.z, __int_as_float(0x7f800000)));
     st_once(&w.st[0].ray_d[i], make_float4(d.x, d.y, d.z, 0.0f));
     st_once(&w.st[0].rng[i], (unsigned long long)s.rng.state);

@@ -180,6 +180,22 @@ class Adaptive:                             # yk_adaptive (include/yuki_gpu.h): 
 
 
 @dataclass(frozen=True)
+class ThinLens:                             # yk_thin_lens (include/yuki_gpu.h): pbrt-v3's lensradius / focaldistance
+    """Depth of field: camera rays leave from a disk of `radius` (scene units) around the camera position and meet on the
+    plane of focus at `focal_distance` along the view axis. Radius 0 is the pinhole."""
+    radius: float
+    focal_distance: float = 1e6
+
+    def __post_init__(self):
+        with np.errstate(over="ignore"):
+            r, f = float(np.float32(self.radius)), float(np.float32(self.focal_distance))
+        if not 0.0 <= r <= float(np.finfo(np.float32).max):   # (NaN fails the comparison)
+            raise ValueError(f"ThinLens.radius must be >= 0 and finite in float32, got {self.radius}")
+        if not 0.0 < f <= float(np.finfo(np.float32).max):
+            raise ValueError(f"ThinLens.focal_distance must be > 0 and finite in float32, got {self.focal_distance}")
+
+
+@dataclass(frozen=True)
 class Denoise:                              # yk_denoise_params (include/yuki_gpu.h): no counterpart in the reference
     """The a-trous denoiser's settings: `iterations` passes (1 ... 10) at steps 1, 2, 4, ...; colour weights
     (1 + |dc|^2 / (sigma^2 (var_p + var_q) + eps))^-2."""

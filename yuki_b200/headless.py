@@ -6,7 +6,8 @@ polling `check_status`, apply the selected tone map and write an uncompressed f3
 
 The reference takes integrator / sampler / film / tone-map choices from settings.yaml (app/mod.rs:17-25); here they are
 flags with the reference's defaults (Whitted depth 3, Stratified 1x1 jittered, the scene file's film settings, filmic
-tone map with exposure 1)."""
+tone map with exposure 1). The camera is the pinhole, as the reference's, unless --thin-lens (the pbrt file's `lensradius` /
+`focaldistance`) or --lens-radius asks for depth of field."""
 from __future__ import annotations
 
 import argparse
@@ -24,9 +25,14 @@ INTEGRATORS = {"whitted": D.INTEGRATOR_WHITTED, "path": D.INTEGRATOR_PATH, "bvh-
 SPLITS = {"sah": D.SPLIT_SAH, "middle": D.SPLIT_MIDDLE, "equal-counts": D.SPLIT_EQUAL_COUNTS}
 
 
-def try_load_scene(path: str, max_shapes_in_node: int = 1, split_method: int = D.SPLIT_SAH):
+def try_load_scene(path: str, max_shapes_in_node: int = 1, split_method: int = D.SPLIT_SAH, with_lens: bool = False):
     """app/util.rs:15-66: (SceneDesc, CameraParameters, FilmSettings) by file extension; an empty path is the built-in
-    Cornell box (`Scene::cornell`, scene/mod.rs:154-531)."""
+    Cornell box (`Scene::cornell`, scene/mod.rs:154-531). `with_lens`: also the file's D.ThinLens (a pbrt camera's
+    lensradius / focaldistance; radius 0 for the other formats)."""
+    if with_lens:
+        if os.path.splitext(path)[1] == ".pbrt" and os.path.exists(path):
+            return api.load_pbrt(path, max_shapes_in_node, split_method, with_lens=True)
+        return (*try_load_scene(path, max_shapes_in_node, split_method), D.ThinLens(0.0))
     if path == "":
         scene, cam = scenes.cornell(xf, light="rect", tall_box="glass", sphere=True, split_method=D.SPLIT_MIDDLE)
         return scene, cam, D.FilmSettings()
@@ -80,7 +86,19 @@ def parse_args(argv=None):
                          "radiance_sq and shading_normals companion films and, with --adaptive, its sample counts")
     ap.add_argument("--denoise-sigma", type=float, default=D.Denoise.sigma, metavar="S")
     ap.add_argument("--denoise-iterations", type=int, default=D.Denoise.iterations, metavar="K", help="1 ... 10")
+    ap.add_argument("--thin-lens", action="store_true",
+                    help="depth of field with the scene file's lens (pbrt: Camera lensradius / focaldistance); default: pinhole")
+    ap.add_argument("--lens-radius", type=float, default=None, metavar="R",
+                    help="depth of field through a thin lens of radius R (scene units); 0 = pinhole")
+    ap.add_argument("--focal-distance", type=float, default=None, metavar="F",
+                    help="with --lens-radius or --thin-lens: distance of the plane of focus (default: the scene file's, else 1e6)")
     args = ap.parse_args(argv)
+    if args.focal_distance is not None and args.lens_radius is None and not args.thin_lens:
+        ap.error("--focal-distance needs --lens-radius or --thin-lens")
+    try:
+        D.ThinLens(0.0 if args.lens_radius is None else args.lens_radius, 1e6 if args.focal_distance is None else args.focal_distance)
+    except ValueError as e:
+        ap.error(str(e))
     if args.sample_counts is not None and args.adaptive is None:
         ap.error("--sample-counts needs --adaptive")
     if args.denoise:
@@ -94,6 +112,15 @@ def parse_args(argv=None):
         if args.adaptive is None and sampler.samples_per_pixel() < 2:
             ap.error("--denoise needs at least 2 samples per pixel")
     return args
+
+
+def lens_from_args(args, file_lens: D.ThinLens):
+    """--thin-lens / --lens-radius R [--focal-distance F] -> D.ThinLens, each value the scene file's unless given; None
+    (the pinhole) without either."""
+    if not args.thin_lens and args.lens_radius is None:
+        return None
+    return D.ThinLens(file_lens.radius if args.lens_radius is None else args.lens_radius,
+                      file_lens.focal_distance if args.focal_distance is None else args.focal_distance)
 
 
 def denoise_from_args(args):
@@ -145,7 +172,8 @@ def settings_from_args(args):
 def render(args, out=sys.stdout) -> np.ndarray:
     sampler, integrator = settings_from_args(args)
     t0 = time.perf_counter()
-    scene, cam, film_settings = try_load_scene(args.scene, args.max_shapes_in_node, SPLITS[args.split])
+    scene, cam, film_settings, file_lens = try_load_scene(args.scene, args.max_shapes_in_node, SPLITS[args.split], with_lens=True)
+    lens = lens_from_args(args, file_lens)
     if args.res is not None or args.tile_dim != film_settings.tile_dim:
         film_settings = D.FilmSettings(tuple(args.res) if args.res is not None else tuple(film_settings.res), args.tile_dim)
     ctx = api.Context(args.device)
@@ -156,7 +184,9 @@ def render(args, out=sys.stdout) -> np.ndarray:
     start = time.perf_counter()
     denoise = denoise_from_args(args)
     aovs = [name for name, _ in args.aov] + (["radiance_sq", "shading_normals"] if denoise else [])
-    rn.launch(dev, cam, film, sampler, integrator, aovs=aovs, adaptive=adaptive_from_args(args))
+    if lens is not None:
+        print(f"Thin lens: radius {lens.radius:g}, focal distance {lens.focal_distance:g}", file=out)
+    rn.launch(dev, cam, film, sampler, integrator, aovs=aovs, adaptive=adaptive_from_args(args), lens=lens)
     width = 0
     while True:   # headless.rs:51-110
         st = rn.check_status()
