@@ -227,7 +227,8 @@ class Plane:
         return s, cam
 
     def hit(self, o, d):
-        """float64 hit of rays (o, d) with the plane: p, uv, inside, and distance of p to the outline."""
+        """float64 hit of rays (o, d) with the plane: p, uv, inside, the distance of p to the outline (edge), the geometric
+        normal n, the shading frame (ss, ts, ns) and the wo that Bsdf::f receives (-d, triangle.rs:179)."""
         o, d = np.asarray(o, np.float64), np.asarray(d, np.float64)
         t = ((self.v[0] - o) @ self.n) / (d @ self.n)
         p = o + t[..., None] * d
@@ -236,14 +237,98 @@ class Plane:
         v = (q @ self.ev) / (self.ev @ self.ev)
         inside = (t > 0) & (u > 0) & (u < 1) & (v > 0) & (v < 1)
         edge = 2.0 * np.minimum(np.minimum(u, 1 - u), np.minimum(v, 1 - v))   # the square's side is 2
-        return p, np.stack([u, v], axis=-1), inside, edge
+        each = lambda v3: np.broadcast_to(v3, p.shape)
+        return {"p": p, "uv": np.stack([u, v], axis=-1), "inside": inside, "edge": edge, "n": each(self.n), "ss": each(self.ss),
+                "ts": each(self.ts), "ns": each(self.n), "wo": -d, "frame_err": np.zeros(len(p))}
 
-    def local(self, w):
-        return np.stack([w @ self.ss, w @ self.ts, w @ self.n], axis=-1)
+    def self_shadow(self, p, n, target):
+        """A plane never occludes its own shadow rays: (occluded, within rounding)."""
+        return np.zeros(len(p), bool), np.zeros(len(p), bool)
+
+
+def _local(h, w):
+    """World to the shading frame (bsdfs/mod.rs:87-99): (w . ss, w . ts, w . ns)."""
+    return np.stack([(w * h["ss"]).sum(-1), (w * h["ts"]).sum(-1), (w * h["ns"]).sum(-1)], axis=-1)
+
+
+class SphereShape:
+    """A sphere (shapes/sphere.rs) in front of _quad_scene's camera. Geometry in float64 from the float32 object_to_world M,
+    its stored inverse W and the radius: the exact root of |W o + t W d|^2 = r^2, the object-space outward normal negated when M
+    swaps handedness and moved by W^T (interaction.rs:105-164; a mirrored sphere's normal points into it), sh_n = n,
+    ss = normalize(M (-2 pi p.y, 2 pi p.x, 0)), ts = cross(ns, ss), and wo = normalize(M (-d)) (sphere.rs:116): on a rotated or
+    non-uniformly scaled sphere that wo differs from -d."""
+
+    def __init__(self, name, to_world, radius):
+        self.name, self.to_world, self.r = name, to_world, float(F32(radius))
+        self.M = to_world.m.astype(np.float64).reshape(4, 4)
+        self.W = to_world.m_inv.astype(np.float64).reshape(4, 4)
+        self.swaps = np.linalg.det(self.M[:3, :3]) < 0
+
+    def scene(self, mat):
+        _, cam = _quad_scene()
+        s = D.SceneDesc(background=(0.0, 0.0, 0.0))
+        s.spheres.append(D.Sphere(self.to_world, self.r, mat.add_to(s)))
+        return s, cam
+
+    def _quadric(self, o, d):
+        oo = o @ self.W[:3, :3].T + self.W[:3, 3]
+        dd = d @ self.W[:3, :3].T
+        a, b, c = (dd * dd).sum(-1), 2.0 * (dd * oo).sum(-1), (oo * oo).sum(-1) - self.r * self.r
+        return oo, dd, a, b, c, b * b - 4.0 * a * c
+
+    def hit(self, o, d):
+        o, d = np.asarray(o, np.float64), np.asarray(d, np.float64)
+        oo, dd, a, b, c, disc = self._quadric(o, d)
+        t = (-b - np.sqrt(np.maximum(disc, 0.0))) / (2.0 * a)      # the camera is outside: the near root
+        inside = (disc > 0) & (t > 0)
+        p_obj = oo + t[:, None] * dd
+        p_obj *= self.r / np.linalg.norm(p_obj, axis=-1, keepdims=True)
+        p = p_obj @ self.M[:3, :3].T + self.M[:3, 3]
+        n = (p_obj / self.r * (-1.0 if self.swaps else 1.0)) @ self.W[:3, :3]
+        n /= np.linalg.norm(n, axis=-1, keepdims=True)
+        ss = np.stack([-p_obj[:, 1], p_obj[:, 0], np.zeros(len(p))], -1) @ self.M[:3, :3].T
+        ss /= np.linalg.norm(ss, axis=-1, keepdims=True)
+        wo = -d @ self.M[:3, :3].T
+        wo /= np.linalg.norm(wo, axis=-1, keepdims=True)
+        # the silhouette margin: r minus the object-space ray's distance from the centre, over r (the discriminant's margin)
+        rho = np.sqrt(np.maximum((oo * oo).sum(-1) - (oo * dd).sum(-1) ** 2 / a, 0.0))
+        edge = (self.r - rho) / self.r
+        # the float32 frame turns with the float32 hit point: the object-space ray carries ~8 roundings of |o'| + r, which the
+        # root moves along the surface by up to 1 / sqrt(1 - rho^2 / r^2) <= 1 / sqrt(2 edge) times; the inverse transpose
+        # amplifies the turn by W's condition number, the cross products and normalisations add ~16 roundings
+        cond = np.linalg.cond(self.W[:3, :3])
+        frame_err = 2.0 * cond * 8.0 * EPS32 * (np.linalg.norm(oo, axis=-1) / self.r + 1.0) / np.sqrt(2.0 * np.maximum(edge, 1e-12)) + 16.0 * EPS32
+        return {"p": p, "uv": np.zeros((len(p), 2)), "inside": inside, "edge": edge, "n": n, "ss": ss,
+                "ts": np.cross(n, ss), "ns": n, "wo": wo, "frame_err": frame_err}
+
+    def self_shadow(self, p, n, target):
+        """The shadow segment of spawn_ray_to (interaction.rs:41-59: origin p +- 0.001 n on the target's side, t_max 0.9999)
+        against the sphere itself: whether it is occluded in float64, and whether that decision is within rounding (the
+        discriminant within 1e-5 of its terms, or a root within 1e-5 r of either end)."""
+        off = 0.001 * n
+        o = np.where((((target - p) * n).sum(-1) > 0)[:, None], p + off, p - off)
+        oo, dd, a, b, c, disc = self._quadric(o, target - o)
+        sq = np.sqrt(np.maximum(disc, 0.0))
+        t0, t1 = (-b - sq) / (2.0 * a), (-b + sq) / (2.0 * a)
+        inr = lambda t: (t > 0) & (t < 0.9999)
+        occ = (disc >= 0) & (inr(t0) | inr(t1))
+        scale = b * b + 4.0 * a * np.abs(c)
+        dist = np.linalg.norm(target - o, axis=-1) / self.r      # a segment's t in units of r
+        near = (np.abs(disc) <= 1e-5 * scale) | np.any([np.abs(t) * dist < 1e-5 for t in (t0, t1, t0 - 0.9999, t1 - 0.9999)], axis=0)
+        return occ, near
 
 
 PLANES = {"flat": Plane("flat"),
           "tilted": Plane("tilted", xf.mul(xf.rotation(float(F32(0.5)), (0.0, 0.0, 1.0)), xf.rotation(float(F32(0.45)), (1.0, 0.6, 0.0))))}
+_C = xf.translation((0.1, 0.0, 0.0))
+SPHERES = {
+    "sphere-translated": SphereShape("sphere-translated", _C, 0.9),
+    "sphere-rotated": SphereShape("sphere-rotated", xf.mul(_C, xf.rotation(float(F32(1.1)), (0.4, 1.0, 0.3))), 0.9),
+    "sphere-scaled": SphereShape("sphere-scaled", xf.mul(_C, xf.mul(xf.rotation(float(F32(0.6)), (1.0, 0.0, 0.5)), xf.scale(1.2, 0.7, 0.95))), 0.85),
+    "sphere-scaled-mirrored": SphereShape("sphere-scaled-mirrored", xf.mul(_C, xf.mul(xf.rotation(float(F32(0.6)), (1.0, 0.0, 0.5)),
+                                                                                   xf.scale(1.2, -0.7, 0.95))), 0.85),
+}
+SHAPES = {**PLANES, **SPHERES}
 
 
 # ---- lights ------------------------------------------------------------------------------------------------------------
@@ -256,22 +341,23 @@ class Light:
         self.pos = self.m[:3, 3]
 
     def sample(self, p, n, u):
-        """sample_li at points p (geometric normal n) with draws u: wi, Li, pdf and whether a shadow ray exists."""
+        """sample_li at points p (geometric normal n) with draws u: wi, Li, pdf, whether a shadow ray exists, and the point
+        the shadow ray ends at."""
         k, N = self.desc.kind, p.shape[0]
         ones = np.ones(N)
         if k == D.LIGHT_POINT:   # point_light.rs:27-49: I / d^2
             to = self.pos - p
             d2 = (to * to).sum(axis=-1)
-            return to / np.sqrt(d2)[:, None], self.i / d2[:, None], ones, ones > 0
+            return to / np.sqrt(d2)[:, None], self.i / d2[:, None], ones, ones > 0, np.broadcast_to(self.pos, p.shape)
         if k == D.LIGHT_SPOT:    # spot_light.rs:38-80: I * falloff / d^2, falloff = delta^4 in the blend, no shadow ray at 0
             to = self.pos - p
             d2 = (to * to).sum(axis=-1)
             wi = to / np.sqrt(d2)[:, None]
             fall = self.falloff(p)
-            return wi, self.i * (fall / d2)[:, None], ones, fall > 0
+            return wi, self.i * (fall / d2)[:, None], ones, fall > 0, np.broadcast_to(self.pos, p.shape)
         if k == D.LIGHT_DISTANT:   # distant_light.rs:17-43: L along w as given, not normalised
             w = np.asarray(F32(self.desc.direction), np.float64)
-            return np.broadcast_to(w, p.shape), np.broadcast_to(self.i, p.shape), ones, ones > 0
+            return np.broadcast_to(w, p.shape), np.broadcast_to(self.i, p.shape), ones, ones > 0, p + 10000.0 * w
         # rectangular_light.rs:27-72: the point (u.x, 0, u.y) of the unit square scaled to `size`, one-sided radiance along the
         # transformed -y normal (not normalised), pdf = d^2 / (|cos_l| * area)
         sx, sz = (float(F32(v)) for v in self.desc.size)
@@ -284,7 +370,7 @@ class Light:
         cos_l = -(wi @ nl)
         li = np.where((cos_l > 0)[:, None], self.i, 0.0)
         area = float(F32(F32(sx) * F32(sz)))
-        return wi, li, d2 / (np.abs(cos_l) * area), ones > 0
+        return wi, li, d2 / (np.abs(cos_l) * area), ones > 0, lp
 
     def cos_spot(self, p):
         dl = (p - self.pos) @ self.m_inv[:3, :3].T      # world_to_light applied to -wi (the direction from the light)
@@ -327,6 +413,7 @@ def _light_descs(place):
 
 
 LIGHTS = {name: _light_descs(plane.to_world) for name, plane in PLANES.items()}
+SPHERE_LIGHT_SET = _light_descs(xf.translation((0.0, 0.0, 0.8)))   # the same lights raised above the spheres' tops
 LIGHT_NAMES = list(LIGHTS["flat"])
 
 
@@ -376,33 +463,57 @@ def _texel(mat, uv):
     return (iy, ix), safe
 
 
-def _shade(plane, mat, lights, o, d, u_lights):
+def _shade(shape, mat, lights, o, d, u_lights):
     """float64 radiance of Path / Whitted depth 1 for camera rays (o, d) (N, 3) and light draws (N, 2 * lights), plus masks and
-    per-ray relative tolerances. The fold of path.rs:102-119: sum_k f(wo, wi_k) * Li_k * clamp(n_s . wi_k, 0, 1) / pdf_k."""
-    p, uv, inside, edge = plane.hit(o, d)
-    texel, tex_safe = _texel(mat, uv)
-    wo_w = -np.asarray(d, np.float64)
-    wo = plane.local(wo_w)
+    per-ray relative tolerances. The fold of path.rs:102-119: sum_k f(wo, wi_k) * Li_k * clamp(n_s . wi_k, 0, 1) / pdf_k, with
+    the shape's wo (si.wo) and per-point frame."""
+    h = shape.hit(o, d)
+    p, n, inside = h["p"], h["n"], h["inside"]
+    texel, tex_safe = _texel(mat, h["uv"])
+    wo_w = h["wo"]
+    wo = _local(h, wo_w)
+    wo_neg_d = _local(h, -np.asarray(d, np.float64))   # the "obvious" wo, for the claim that the shape's own one is used
     L = np.zeros(p.shape)
-    keep = inside & (edge > EDGE) & tex_safe
+    keep = inside & (h["edge"] > EDGE) & tex_safe
     tol = np.full(len(p), RTOL)   # the sum of positive terms errs by at most its worst term's relative error
     abs_tol = np.zeros(p.shape)
-    info = {"cos": [], "fall": [], "li_nonzero": np.zeros(len(p), bool), "texel": texel}
+    info = {"cos": [], "fall": [], "li_nonzero": np.zeros(len(p), bool), "texel": texel, "wo_matters": np.zeros(len(p), bool),
+            "self_shadow": np.zeros(len(p), bool), "dark": np.ones(len(p), bool)}
     for k, desc in enumerate(lights):
         lt = Light(desc)
-        wi_w, li, pdf, vis = lt.sample(p, plane.n, u_lights[:, 2 * k:2 * k + 2].astype(np.float64))
+        wi_w, li, pdf, vis, target = lt.sample(p, n, u_lights[:, 2 * k:2 * k + 2].astype(np.float64))
+        wi_w = np.asarray(wi_w)
+        reaches = li.max(axis=-1) > 0
+        # the shape's own shadow ray (a sphere's, where the light is behind its horizon); within rounding of it: left out
+        occ, near = shape.self_shadow(p, n, np.asarray(target, np.float64))
+        vis = vis & ~occ
+        info["self_shadow"] |= inside & reaches & near
+        keep &= ~(reaches & near)
         # Bsdf::f (bsdfs/mod.rs:125-147): only reflection lobes, taken when wi and wo lie on the same side of n_g
-        refl = (wi_w @ plane.n) * (wo_w @ plane.n) > 0.0
-        f, f_err = mat.f(wo, plane.local(np.asarray(wi_w)), texel)
+        cos_g = (wi_w * n).sum(-1)
+        refl = cos_g * (wo_w * n).sum(-1) > 0.0
+        wi = _local(h, wi_w)
+        f, f_err = mat.f(wo, wi, texel)
         f = np.where(refl[:, None], f, 0.0)
-        cos = np.clip(np.asarray(wi_w) @ plane.n, 0.0, 1.0)
+        cos_s = (wi_w * h["ns"]).sum(-1)
+        cos = np.clip(cos_s, 0.0, 1.0)
+        # a per-point frame (spheres) that turns by frame_err moves cos by that over cos, GGX's D by up to 2 / alpha times it
+        # (its log-derivative in theta_h), the other factors by about twice it
+        slope = 2.0 / mat.alpha(mat.scalar(texel)) + 2.0 if mat.kind in (D.MAT_METAL, D.MAT_GLOSSY) else 2.0
+        f_err = f_err + h["frame_err"] * (slope + 1.0 / np.maximum(cos, COS_CUTOFF))
         term = np.where(vis[:, None], f * li * cos[:, None] / pdf[:, None], 0.0)
         L += term
-        info["li_nonzero"] |= (li.max(axis=-1) > 0) & refl
-        lit = refl & (li.max(axis=-1) > 0) & vis
+        info["li_nonzero"] |= reaches & refl
+        lit = refl & reaches & vis
         tol = np.maximum(tol, np.where(lit, RTOL + f_err, 0.0))
-        keep &= ~(lit & (cos < COS_CUTOFF))
+        keep &= ~(lit & (np.abs(cos_s) < COS_CUTOFF))
+        # where the light grazes the surface the side test and the clamp flip within rounding: left out
+        keep &= ~(reaches & vis & (np.abs(cos_g) < COS_CUTOFF))
         info["cos"].append(np.where(lit, cos, np.nan))
+        info["dark"] &= ~(lit & (cos > 0))
+        f_neg_d, _ = mat.f(wo_neg_d, wi, texel)
+        rtol = np.broadcast_to(np.asarray(RTOL + f_err, np.float64), lit.shape)
+        info["wo_matters"] |= lit & (np.abs(f - f_neg_d) > 10.0 * rtol[:, None] * np.abs(f)).any(axis=-1)
         if desc.kind == D.LIGHT_SPOT:
             # the falloff's rounding: d(delta^4)/d(cos_theta) = 4 delta^3 / (cos_falloff - cos_total), times SPOT_CT_ERR
             c_tot, c_fall = lt.cone()
@@ -416,7 +527,7 @@ def _shade(plane, mat, lights, o, d, u_lights):
     return np.where(inside[:, None], L, 0.0), keep, inside, tol, abs_tol, info
 
 
-def _reference(plane, mat, lights):
+def _reference(shape, mat, lights):
     """(want, keep, inside-but-not-kept pixels, per-pixel tolerances, info) at the film's resolution. Delta lights: pixel
     centres; rect lights: every (pixel, sample) from its exact draws, averaged as the film does."""
     from oracle import oracle as O
@@ -426,11 +537,12 @@ def _reference(plane, mat, lights):
         ys, xs = np.mgrid[0:h, 0:w]
         pf = np.stack([xs + 0.5, ys + 0.5], axis=-1).reshape(-1, 2).astype(np.float32)
         o, d = O.camera_rays(cam, DELTA_FILM, pf)
-        L, keep, inside, tol, abs_tol, info = _shade(plane, mat, lights, o, d, np.zeros((len(o), 2 * len(lights)), np.float32))
+        L, keep, inside, tol, abs_tol, info = _shade(shape, mat, lights, o, d, np.zeros((len(o), 2 * len(lights)), np.float32))
         sh = (h, w)
         info = {"cos": [c.reshape(sh) for c in info["cos"]], "fall": [tuple(np.reshape(a, sh) if np.ndim(a) else a for a in f) for f in info["fall"]],
                 "li_nonzero": info["li_nonzero"].reshape(sh),
-                "texel": None if mat.image is None else tuple(t.reshape(sh) for t in info["texel"])}
+                "texel": None if mat.image is None else tuple(t.reshape(sh) for t in info["texel"]),
+                **{k: info[k].reshape(sh) for k in ("wo_matters", "self_shadow", "dark")}, "covered": inside.reshape(sh)}
         return L.reshape(sh + (3,)), keep.reshape(sh), inside.reshape(sh), tol.reshape(sh), abs_tol.reshape(sh + (3,)), info
     w, h = RECT_FILM.res
     spp = RECT_SAMPLER.samples_per_pixel()
@@ -438,13 +550,15 @@ def _reference(plane, mat, lights):
     ys, xs = np.mgrid[0:h, 0:w]
     pf = np.stack([xs[..., None].astype(np.float32) + draws[..., 0], ys[..., None].astype(np.float32) + draws[..., 1]], axis=-1)
     o, d = O.camera_rays(cam, RECT_FILM, pf.reshape(-1, 2))
-    L, keep, inside, tol, abs_tol, info = _shade(plane, mat, lights, o, d, draws[..., 2:].reshape(-1, 2 * len(lights)))
+    L, keep, inside, tol, abs_tol, info = _shade(shape, mat, lights, o, d, draws[..., 2:].reshape(-1, 2 * len(lights)))
     sh = (h, w, spp)
     # a pixel is kept when all its samples are: the mean of the samples, within the largest of their tolerances
     keep_px = keep.reshape(sh).all(axis=-1) | ~inside.reshape(sh).any(axis=-1)
     keep_px &= inside.reshape(sh).all(axis=-1) | ~inside.reshape(sh).any(axis=-1)
     info = {"cos": [c.reshape(sh) for c in info["cos"]], "fall": [(f[0].reshape(sh),) + f[1:] for f in info["fall"]],
-            "li_nonzero": info["li_nonzero"].reshape(sh).any(axis=-1)}
+            "li_nonzero": info["li_nonzero"].reshape(sh).any(axis=-1), "wo_matters": info["wo_matters"].reshape(sh).any(axis=-1),
+            "self_shadow": info["self_shadow"].reshape(sh).any(axis=-1), "dark": info["dark"].reshape(sh).all(axis=-1),
+            "covered": inside.reshape(sh).all(axis=-1)}
     return (L.reshape(sh + (3,)).mean(axis=2), keep_px, inside.reshape(sh).any(axis=-1), tol.reshape(sh).max(axis=-1),
             abs_tol.reshape(sh + (3,)).max(axis=2), info)
 
@@ -465,8 +579,37 @@ def _film_sampler(lights):
     return (RECT_FILM, RECT_SAMPLER) if _has_rect(lights) else (DELTA_FILM, DELTA_SAMPLER)
 
 
+def _sphere_claims(shape, mat, light_name, lights, ref, img, st):
+    want, keep, inside, _, _, info = ref
+    lit = keep & (want.max(axis=-1) > 0)
+    rect = _has_rect(lights)
+    assert inside.sum() > (500 if rect else 2000) and st.shadow_rays > 0
+    # of the pixels the sphere covers (on a rect film: every sample; its outline's pixels mix sphere and background)
+    assert (keep & info["covered"]).sum() > 0.8 * info["covered"].sum(), "the masks leave out too much"
+    # shadow rays that pass within rounding of the sphere itself (spawn_ray_to's 0.001 n offset) are rare
+    assert info["self_shadow"].sum() <= 0.01 * inside.sum(), int(info["self_shadow"].sum())
+    if shape.swaps:
+        # the normal and shading normal point into a mirrored sphere: the lights reach it and the lobes' side test passes,
+        # but clamp(n_s . wi, 0, 1) is 0 on every visible point, so the film is exactly black
+        assert np.all(img == 0.0) and (info["li_nonzero"] & inside).sum() > 0.3 * inside.sum()
+        return
+    assert lit.sum() > (150 if rect else 600)
+    if light_name == "point-low":
+        # the terminator: lit kept pixels down to cos = 0.05 and the dark side beyond it, exactly 0
+        assert (lit & (info["cos"][0] < 0.2)).sum() > 200 and (keep & inside & info["dark"]).sum() > 500
+    if shape.name != "sphere-translated" and (mat.kind != D.MAT_MATTE or (mat.name != "matte" and light_name != "point-low")):
+        # si.wo = normalize(o2w (-d)) differs from -d: f differs by more than 10 tolerances on most lit pixels
+        assert (keep & info["wo_matters"]).sum() > 0.5 * lit.sum(), int((keep & info["wo_matters"]).sum())
+
+
+SPHERE_MATERIALS = ("matte", "oren-nayar-20", "copper-a0.3", "glossy-r0.2")
+SPHERE_LIGHTS = ("point-high", "point-low", "rect", "all-four")
+
+
 def _claims(plane, mat, light_name, lights, ref, img, st):
     """What the case names must occur in it, in enough pixels."""
+    if isinstance(plane, SphereShape):
+        return _sphere_claims(plane, mat, light_name, lights, ref, img, st)
     want, keep, inside, _, _, info = ref
     lit = keep & (want.max(axis=-1) > 0)
     min_px = 300 if _has_rect(lights) else 1500
@@ -507,6 +650,10 @@ def _cases():
         for mat in IMAGE_MATERIALS:
             for light in ("point-high", "point-low"):
                 out.append(f"{plane}-{mat}-{light}")
+    for sphere in SPHERES:
+        for light in SPHERE_LIGHTS:
+            for mat in SPHERE_MATERIALS:
+                out.append(f"{sphere}-{mat}-{light}")
     return out
 
 
@@ -514,12 +661,12 @@ CASES = _cases()
 
 
 def _case(case):
-    plane_name = next(p for p in PLANES if case.startswith(p + "-"))
-    rest = case[len(plane_name) + 1:]
+    shape_name = next(p for p in sorted(SHAPES, key=len, reverse=True) if case.startswith(p + "-"))
+    rest = case[len(shape_name) + 1:]
     light_name = next(l for l in sorted(LIGHT_NAMES, key=len, reverse=True) if rest.endswith("-" + l))
     mat_name = rest[:-(len(light_name) + 1)]
     mat = MATERIALS.get(mat_name) or IMAGE_MATERIALS[mat_name]
-    return PLANES[plane_name], mat, light_name, LIGHTS[plane_name][light_name]
+    return SHAPES[shape_name], mat, light_name, (LIGHTS[shape_name] if shape_name in PLANES else SPHERE_LIGHT_SET)[light_name]
 
 
 def _scene(plane, mat, lights):
