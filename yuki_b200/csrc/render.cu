@@ -54,6 +54,35 @@ constexpr int kMaxPipes = YK_MAX_PIPES;   // batches in flight on separate strea
 constexpr int kRing = 2;       // batches queued per pipe before the host waits for the oldest
 constexpr int kTimedStages = 5;  // events per bounce: before/after closest, after classify, after shading, after shadow
 
+// A device array that only grows: reserve() reallocates when the capacity is too small and keeps the allocation otherwise.
+// Plain cudaMalloc / cudaFree, not the stream-ordered pool (dev_alloc): cudaFree waits for the device, so a buffer that
+// reserve() replaces is not freed under work still reading it.
+template <class T>
+class DevArray {
+public:
+    DevArray() = default;
+    DevArray(DevArray&& o) noexcept { swap(o); }
+    DevArray& operator=(DevArray&& o) noexcept { swap(o); return *this; }
+    ~DevArray() { cudaFree(p_); }
+    // On failure the array is left empty, with capacity 0.
+    cudaError_t reserve(size_t count) {
+        if (cap_ >= count) return cudaSuccess;
+        cudaFree(p_);
+        p_ = nullptr;
+        cap_ = 0;
+        const cudaError_t e = cudaMalloc((void**)&p_, count * sizeof(T));
+        if (e != cudaSuccess) p_ = nullptr;
+        else cap_ = count;
+        return e;
+    }
+    T* get() const { return p_; }
+    size_t capacity() const { return cap_; }
+    void swap(DevArray& o) noexcept { std::swap(p_, o.p_); std::swap(cap_, o.cap_); }
+private:
+    T* p_ = nullptr;
+    size_t cap_ = 0;
+};
+
 // One asynchronous wavefront lane: its own stream, path state, bounce counters and timing events.
 struct Pipe {
     cudaStream_t stream = nullptr;
@@ -64,22 +93,18 @@ struct Pipe {
     bool wave_sort = false;          // the ray-sort arrays are allocated
     void* sort_scan_tmp = nullptr;   // cub scan workspace for the sort's bins
     size_t sort_scan_bytes = 0;
-    IterCounters* d_ctr = nullptr;   // two entries, alternating per bounce
+    DevArray<IterCounters> d_ctr;    // two entries, alternating per bounce
     IterCounters* h_ctr = nullptr;   // pinned: read-back for the integrators whose bounce count is unbounded (Whitted)
     Totals* h_totals = nullptr;      // pinned
-    SampleJump* d_jumps = nullptr;   // sampler seek table of the batch being queued (kMaxBatchSamples entries)
-    Job* d_jobs = nullptr;           // the pixel jobs of the pipe's current pixel group
-    size_t jobs_cap = 0;
-    uint32_t* d_dim_hash = nullptr;  // SamplerCfg::hash_table of the pipe's current pixel group
-    size_t dim_hash_cap = 0;
+    DevArray<SampleJump> d_jumps;    // sampler seek table of the batch being queued (kMaxBatchSamples entries)
+    DevArray<Job> d_jobs;            // the pixel jobs of the pipe's current pixel group
+    DevArray<uint32_t> d_dim_hash;   // SamplerCfg::hash_table of the pipe's current pixel group
     size_t hash_group = (size_t)-1;
     // adaptive sampling (wf_adaptive.cuh): the job list a check compacts into, its per-job keep flags and per-block survivor
     // counts, and the survivor count read back for the next batch's size
-    Job* d_jobs_next = nullptr;
-    size_t jobs_next_cap = 0;
-    uint8_t* d_keep = nullptr;
-    uint32_t* d_block_keep = nullptr;  // + 1 entry: the total
-    size_t keep_cap = 0;
+    DevArray<Job> d_jobs_next;
+    DevArray<uint8_t> d_keep;
+    DevArray<uint32_t> d_block_keep;   // + 1 entry: the total
     uint32_t* h_survivors = nullptr;   // pinned
     bool survivors_pending = false;    // a check's count is on its way to h_survivors
     bool rehash = false;               // the job list was compacted: SamplerCfg::hash_table is indexed by the old job slots
@@ -92,8 +117,10 @@ struct Pipe {
     } slot[kRing];
     uint64_t n_batches = 0;
     int timing = 2;  // the context's stage_timing when the queued batches were recorded
+    ~Pipe();
 };
 
+// Owns everything it holds: yk_context_destroy deletes it once the device is idle.
 struct yk_context {
     std::recursive_mutex mu;  // calls that use the context's pipes are serialised (SURVEY.md §8b: one context, many caller threads)
     int device = 0;
@@ -101,19 +128,15 @@ struct yk_context {
     cudaStream_t stream = nullptr;
     cudaEvent_t ev[4] = {};
     Pipe pipe[kMaxPipes];
-    yk_tile* d_tiles = nullptr;              // the tile list of the current render and the prefix sum of its tile areas
-    unsigned long long* d_tile_off = nullptr;
-    size_t tiles_cap = 0;
-    float* d_accum = nullptr;
-    float* d_film = nullptr;
-    int32_t* d_hit_ids = nullptr;
-    size_t film_cap = 0;
-    float* d_aov_sums[kAovViews] = {};  // per-pixel sums of the requested companion films (yk_render_opts.aovs), like d_accum
-    float* d_aov_film[kAovViews] = {};  // device copies of the companion films given as host buffers
-    size_t aov_sums_cap[kAovViews] = {}, aov_film_cap[kAovViews] = {};
-    float* d_adaptive_sq = nullptr;  // adaptive renders without radiance_sq: the per-pixel sums of li * li the stopping rule reads
-    uint32_t* d_counts = nullptr;    // device copy of yk_adaptive::sample_counts given as a host buffer
-    size_t adaptive_sq_cap = 0, counts_cap = 0;
+    DevArray<yk_tile> d_tiles;               // the tile list of the current render and the prefix sum of its tile areas
+    DevArray<unsigned long long> d_tile_off;
+    DevArray<float> d_accum;                 // film-sized (film_setup): the per-pixel sums, the film copy, the hit-id image
+    DevArray<float> d_film;
+    DevArray<int32_t> d_hit_ids;
+    DevArray<float> d_aov_sums[kAovViews];  // per-pixel sums of the requested companion films (yk_render_opts.aovs), like d_accum
+    DevArray<float> d_aov_film[kAovViews];  // device copies of the companion films given as host buffers
+    DevArray<float> d_adaptive_sq;  // adaptive renders without radiance_sq: the per-pixel sums of li * li the stopping rule reads
+    DevArray<uint32_t> d_counts;    // device copy of yk_adaptive::sample_counts given as a host buffer
     int occ_trace_closest = 0, occ_trace_any = 0, occ_trace_rays = 0;
     int wide_per_sm = 16;  // grid cap of the grid-stride kernels, blocks per SM (development override: YK_WIDE_PER_SM)
     int n_pipes_env = 0;  // YK_PIPES override (development)
@@ -131,7 +154,7 @@ struct yk_context {
     std::vector<void*> query_flag_alloc;
     int* q_nan = nullptr;  // device-resident rays: set by k_query_pack when a t_max is NaN
     // Ray sort between bounces (wf_sort.cuh). key: 0 = off, 1 = leaf slot of the shape the ray leaves + octant, 2 = Morton cell of
-    // the origin + octant, -1 = by scene size (render_impl). order: 1 = closest-hit kernel only, 2 = material sort too.
+    // the origin + octant, -1 = by scene size (render_cfg). order: 1 = closest-hit kernel only, 2 = material sort too.
     // Environment: YK_SORT_KEY, YK_SORT_ORDER; yk_render_opts.ray_sort overrides the key per render.
     int sort_key = -1, sort_order = 2;
     // Shadow rays: 1 = one ray per lane (k_trace_shadow_rays + k_shadow_fold), 0 = one path per lane with the fold fused
@@ -143,6 +166,7 @@ struct yk_context {
     int shade_phased = -1;  // k_shade<.., PHASED>: -1 = by scene (run_batch), 0 / 1 = environment YK_SHADE_PHASED
     int stage_timing = 1;  // CUDA events per bounce: 1 = around the closest-hit kernel (the roofline figure), 2 = every stage
                            // (costs ~1.5 % of a Cornell render), 0 = none; environment variable YK_STAGE_TIMING
+    ~yk_context();
 };
 
 struct yk_scene {
@@ -435,14 +459,14 @@ int run_batch(yk_context* c, Pipe* p, const yk_scene* sc, const RenderCfg& cfg, 
 #ifdef YK_CHECKED
     CUDA_TRY(cudaMemcpyToSymbolAsync(g_check_queue_cap, &w.cap, sizeof(uint32_t), 0, cudaMemcpyHostToDevice, s));
 #endif
-    CUDA_TRY(cudaMemsetAsync(p->d_ctr, 0, 2 * sizeof(IterCounters), s));
+    CUDA_TRY(cudaMemsetAsync(p->d_ctr.get(), 0, 2 * sizeof(IterCounters), s));
     nvtxRangePushA("yk raygen");
-    k_sample_jumps<<<1, kMaxBatchSamples, 0, s>>>(first_sample, bt.n_samples, p->d_jumps);
+    k_sample_jumps<<<1, kMaxBatchSamples, 0, s>>>(first_sample, bt.n_samples, p->d_jumps.get());
     tm->launches += 1;
     if (lens)
-        k_raygen_lens<<<(bt.n_paths + T - 1) / T, T, 0, s>>>(w, cfg, bt, first_sample, bt.n_samples, p->d_jumps, &p->d_ctr[0],
+        k_raygen_lens<<<(bt.n_paths + T - 1) / T, T, 0, s>>>(w, cfg, bt, first_sample, bt.n_samples, p->d_jumps.get(), p->d_ctr.get(),
                                                              lens->lens_radius, lens->focal_distance);
-    else k_raygen<<<(bt.n_paths + T - 1) / T, T, 0, s>>>(w, cfg, bt, first_sample, bt.n_samples, p->d_jumps, &p->d_ctr[0]);
+    else k_raygen<<<(bt.n_paths + T - 1) / T, T, 0, s>>>(w, cfg, bt, first_sample, bt.n_samples, p->d_jumps.get(), p->d_ctr.get());
     nvtxRangePop();
     tm->launches += 1;
     const bool debug = cfg.integrator >= YK_INTEGRATOR_BVH_INTERSECTIONS;
@@ -477,8 +501,8 @@ int run_batch(yk_context* c, Pipe* p, const yk_scene* sc, const RenderCfg& cfg, 
     const uint32_t* perm_classify = nullptr;
     for (uint32_t iter = 0; iter < max_iters; ++iter) {
         const int b = (int)(iter & 1);  // this bounce reads stream b and writes stream b ^ 1
-        IterCounters* cur = &p->d_ctr[iter & 1];
-        IterCounters* nxt = &p->d_ctr[(iter + 1) & 1];
+        IterCounters* cur = p->d_ctr.get() + (iter & 1);
+        IterCounters* nxt = p->d_ctr.get() + ((iter + 1) & 1);
         if (iter > 0) CUDA_TRY(cudaMemsetAsync(nxt, 0, sizeof(IterCounters), s));
         if (c->stage_timing > 0) CUDA_TRY(cudaEventRecord(stage_event(iter, 0), s));
         const bool spheres = sc->dev.spheres != nullptr || sc->dev.leaf_table != nullptr;  // the generic instantiations: sphere slots, leaf table
@@ -591,7 +615,7 @@ int run_batch(yk_context* c, Pipe* p, const yk_scene* sc, const RenderCfg& cfg, 
     if (accumulate_film) {
         k_film_add<<<(bt.n_paths + T - 1) / T, T, 0, s>>>(w, bt, d_film, cfg.res_x);
     } else {
-        k_film_accumulate<<<(bt.n_jobs + T - 1) / T, T, 0, s>>>(w, bt, c->d_accum, cfg.res_x);
+        k_film_accumulate<<<(bt.n_jobs + T - 1) / T, T, 0, s>>>(w, bt, c->d_accum.get(), cfg.res_x);
     }
     nvtxRangePop();
     tm->launches += 1;
@@ -614,42 +638,51 @@ int adaptive_check(Pipe* p, uint32_t nj, uint32_t count, bool last, const yk_ada
     cudaStream_t s = p->stream;
     const uint32_t nb = (nj + kAdaptiveThreads - 1) / kAdaptiveThreads;
     if (!last) {
-        if (p->jobs_next_cap < p->jobs_cap) {  // (cudaFree waits for the device: nothing in flight still reads the old buffer)
-            cudaFree(p->d_jobs_next);
-            p->d_jobs_next = nullptr;
-            p->jobs_next_cap = 0;
-            CUDA_TRY(cudaMalloc((void**)&p->d_jobs_next, p->jobs_cap * sizeof(Job)));
-            p->jobs_next_cap = p->jobs_cap;
-        }
-        if (p->keep_cap < nj) {
-            cudaFree(p->d_keep);
-            cudaFree(p->d_block_keep);
-            p->d_keep = nullptr;
-            p->d_block_keep = nullptr;
-            p->keep_cap = 0;
-            CUDA_TRY(cudaMalloc((void**)&p->d_keep, nj));
-            CUDA_TRY(cudaMalloc((void**)&p->d_block_keep, ((size_t)nb + 1) * sizeof(uint32_t)));
-            p->keep_cap = nj;
-        }
+        CUDA_TRY(p->d_jobs_next.reserve(p->d_jobs.capacity()));  // (cudaFree waits for the device: nothing in flight still reads the old buffer)
+        CUDA_TRY(p->d_keep.reserve(nj));
+        CUDA_TRY(p->d_block_keep.reserve((size_t)nb + 1));
         if (!p->h_survivors) CUDA_TRY(cudaMallocHost((void**)&p->h_survivors, sizeof(uint32_t)));
     }
-    k_adaptive_check<<<nb, kAdaptiveThreads, 0, s>>>(p->d_jobs, nj, res_x, count, last ? 1u : 0u, a.rel_error, a.abs_error, accum, sums,
-                                                      views, film, counts, last ? nullptr : p->d_keep, last ? nullptr : p->d_block_keep);
+    k_adaptive_check<<<nb, kAdaptiveThreads, 0, s>>>(p->d_jobs.get(), nj, res_x, count, last ? 1u : 0u, a.rel_error, a.abs_error, accum,
+                                                      sums, views, film, counts, last ? nullptr : p->d_keep.get(),
+                                                      last ? nullptr : p->d_block_keep.get());
     tm->launches += 1;
     if (last) return YK_OK;
-    uint32_t* d_total = p->d_block_keep + (p->keep_cap + kAdaptiveThreads - 1) / kAdaptiveThreads;
-    k_adaptive_scan<<<1, kAdaptiveScanThreads, 0, s>>>(p->d_block_keep, nb, d_total);
-    k_adaptive_compact<<<nb, kAdaptiveThreads, 0, s>>>(p->d_jobs, nj, p->d_keep, p->d_block_keep, p->d_jobs_next);
+    uint32_t* d_total = p->d_block_keep.get() + p->d_block_keep.capacity() - 1;
+    k_adaptive_scan<<<1, kAdaptiveScanThreads, 0, s>>>(p->d_block_keep.get(), nb, d_total);
+    k_adaptive_compact<<<nb, kAdaptiveThreads, 0, s>>>(p->d_jobs.get(), nj, p->d_keep.get(), p->d_block_keep.get(), p->d_jobs_next.get());
     CUDA_TRY(cudaMemcpyAsync(p->h_survivors, d_total, sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
     tm->launches += 2;
-    std::swap(p->d_jobs, p->d_jobs_next);
-    std::swap(p->jobs_cap, p->jobs_next_cap);
+    p->d_jobs.swap(p->d_jobs_next);
     p->survivors_pending = true;
     p->rehash = true;
     return YK_OK;
 }
 
 }  // namespace
+
+// The device must be current and idle (yk_context_destroy). Handles a partial yk_context_create left null are skipped.
+Pipe::~Pipe() {
+    free_bag(wave_allocs);
+    cudaFreeHost(h_survivors);
+    cudaFreeHost(h_ctr);
+    cudaFreeHost(h_totals);
+    for (auto& sl : slot) {
+        if (sl.done) cudaEventDestroy(sl.done);
+        for (cudaEvent_t e : sl.ev)
+            if (e) cudaEventDestroy(e);
+    }
+    if (owns_stream && stream) cudaStreamDestroy(stream);
+}
+
+yk_context::~yk_context() {
+    free_bag(query_allocs);
+    free_bag(query_surface_allocs);
+    free_bag(query_flag_alloc);
+    for (auto& e : ev)
+        if (e) cudaEventDestroy(e);
+    if (stream) cudaStreamDestroy(stream);
+}
 
 // Makes the context's device current on the calling thread (post.cu: the display passes may be called from any thread).
 int yk_context_activate(yk_context* c) {
@@ -680,7 +713,7 @@ int yk_context_create(int device_id, yk_context** out) {
                                              "); this backend has no CPU fallback");
     if (device_id < 0 || device_id >= n_dev) return yk_set_error(YK_ERR_INVALID, "yk_context_create: device id out of range");
     CUDA_TRY(cudaSetDevice(device_id));
-    auto* c = new yk_context();
+    auto c = std::make_unique<yk_context>();  // an error return releases what was created so far
     c->device = device_id;
     cudaDeviceProp prop;
     CUDA_TRY(cudaGetDeviceProperties(&prop, device_id));
@@ -692,9 +725,8 @@ int yk_context_create(int device_id, yk_context** out) {
         (void)cudaGetLastError();
     }
     CUDA_TRY(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
-    for (auto& ev : c->ev) CUDA_TRY(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
-    CUDA_TRY(cudaEventDestroy(c->ev[2]));
-    CUDA_TRY(cudaEventDestroy(c->ev[3]));
+    CUDA_TRY(cudaEventCreateWithFlags(&c->ev[0], cudaEventDisableTiming));
+    CUDA_TRY(cudaEventCreateWithFlags(&c->ev[1], cudaEventDisableTiming));
     CUDA_TRY(cudaEventCreate(&c->ev[2]));  // timing pair around the whole render
     CUDA_TRY(cudaEventCreate(&c->ev[3]));
     if (const char* np = getenv("YK_PIPES")) c->n_pipes_env = std::max(1, std::min(kMaxPipes, atoi(np)));
@@ -710,8 +742,8 @@ int yk_context_create(int device_id, yk_context** out) {
             CUDA_TRY(cudaStreamCreateWithFlags(&p.stream, cudaStreamNonBlocking));
             p.owns_stream = true;
         }
-        CUDA_TRY(cudaMalloc((void**)&p.d_ctr, 2 * sizeof(IterCounters)));
-        CUDA_TRY(cudaMalloc((void**)&p.d_jumps, kMaxBatchSamples * sizeof(SampleJump)));
+        CUDA_TRY(p.d_ctr.reserve(2));
+        CUDA_TRY(p.d_jumps.reserve(kMaxBatchSamples));
         CUDA_TRY(cudaMallocHost((void**)&p.h_ctr, sizeof(IterCounters)));
         CUDA_TRY(cudaMallocHost((void**)&p.h_totals, sizeof(Totals)));
     }
@@ -721,7 +753,7 @@ int yk_context_create(int device_id, yk_context** out) {
     // development overrides (A/B of co-resident kernels of two pipes): blocks per SM of the persistent / grid-stride kernels
     if (const char* e = getenv("YK_TRACE_PER_SM")) c->occ_trace_closest = c->occ_trace_any = c->occ_trace_rays = std::max(1, atoi(e));
     if (const char* e = getenv("YK_WIDE_PER_SM")) c->wide_per_sm = std::max(1, atoi(e));
-    *out = c;
+    *out = c.release();
     return YK_OK;
     });
 }
@@ -730,37 +762,6 @@ void yk_context_destroy(yk_context* c) {
     if (!c) return;
     cudaSetDevice(c->device);
     cudaDeviceSynchronize();
-    for (Pipe& p : c->pipe) {
-        free_bag(p.wave_allocs);
-        cudaFree(p.d_ctr);
-        cudaFree(p.d_dim_hash);
-        cudaFree(p.d_jobs);
-        cudaFree(p.d_jobs_next);
-        cudaFree(p.d_keep);
-        cudaFree(p.d_block_keep);
-        cudaFreeHost(p.h_survivors);
-        cudaFree(p.d_jumps);
-        cudaFreeHost(p.h_ctr);
-        cudaFreeHost(p.h_totals);
-        for (auto& sl : p.slot) {
-            if (sl.done) cudaEventDestroy(sl.done);
-            for (cudaEvent_t e : sl.ev) cudaEventDestroy(e);
-        }
-        if (p.owns_stream) cudaStreamDestroy(p.stream);
-    }
-    free_bag(c->query_allocs);
-    free_bag(c->query_surface_allocs);
-    free_bag(c->query_flag_alloc);
-    cudaFree(c->d_tiles);
-    cudaFree(c->d_tile_off);
-    cudaFree(c->d_accum);
-    cudaFree(c->d_film);
-    cudaFree(c->d_hit_ids);
-    for (int k = 0; k < kAovViews; ++k) { cudaFree(c->d_aov_sums[k]); cudaFree(c->d_aov_film[k]); }
-    cudaFree(c->d_adaptive_sq);
-    cudaFree(c->d_counts);
-    for (auto& ev : c->ev) cudaEventDestroy(ev);
-    cudaStreamDestroy(c->stream);
     delete c;
 }
 
@@ -1080,11 +1081,6 @@ void yk_scene_destroy(yk_scene* s) {
 // Internal yk_render_opts.flags bit (yk_multi_render's workers): the caller initialised the hit-id image, do not refill it.
 constexpr uint32_t kRenderAuxInitialised = 0x100u;
 
-// yk_aov_films' buffers in AovSums order
-static void aov_views(const yk_aov_films* a, float* (&v)[kAovViews]) {
-    v[0] = a->bvh_intersections; v[1] = a->geometry_normals; v[2] = a->shading_normals; v[3] = a->shading_uvs; v[4] = a->radiance_sq;
-}
-
 // opts->lens when YK_RENDER_THIN_LENS is set, validated; *out = null for the pinhole (no flag, or a lens of radius 0: the plain
 // render, bit for bit)
 static int thin_lens_of(const yk_render_opts* opts, const char* fn, const yk_thin_lens** out) {
@@ -1100,68 +1096,100 @@ static int thin_lens_of(const yk_render_opts* opts, const char* fn, const yk_thi
     return YK_OK;
 }
 
-// yk_render, and yk_debug_ray's single path (`debug_log` = device ray list, `debug_px` = the film pixel of its camera sample).
-static int render_impl(yk_context* c, const yk_scene* sc, const yk_camera* cam, const yk_film_settings* fs, const yk_sampler* sm,
-                       const yk_integrator* in, const yk_tile* tiles, uint32_t n_tiles, const yk_render_opts* opts, float* film_rgb,
-                       yk_stats* stats, DebugLog* debug_log, const float* debug_px) {
-    const auto wall0 = std::chrono::steady_clock::now();
-    if (!c || !sc || !cam || !fs || !sm || !in || !film_rgb) return yk_set_error(YK_ERR_INVALID, "yk_render: null argument");
-    if (sc->ctx != c) return yk_set_error(YK_ERR_INVALID, "yk_render: scene belongs to another context");
+// yk_render's and yk_multi_render's checks of the film and its tiles (`fn`: the entry point, for the messages)
+static int check_resolution(const yk_film_settings* fs, const char* fn) {
     if (!fs->res_x || !fs->res_y || fs->res_x > 0xffffu || fs->res_y > 0xffffu)
-        return yk_set_error(YK_ERR_INVALID, "yk_render: film resolution must fit u16 (integrators/mod.rs:140-141)");
-    if (in->kind > YK_INTEGRATOR_SHADING_UVS) return yk_set_error(YK_ERR_INVALID, "yk_render: unknown integrator");
-    if (sm->kind > YK_SAMPLER_STRATIFIED) return yk_set_error(YK_ERR_INVALID, "yk_render: unknown sampler");
-    const uint32_t spp = sm->kind == YK_SAMPLER_UNIFORM ? sm->nx : sm->nx * sm->ny;
-    if (spp == 0 || spp > 0x10000u) return yk_set_error(YK_ERR_INVALID, "yk_render: samples per pixel must be in 1..65536");
-    if (in->max_depth > 255) return yk_set_error(YK_ERR_INVALID, "yk_render: max_depth above 255");
-    if (in->kind == YK_INTEGRATOR_WHITTED && in->max_depth > 24)
-        return yk_set_error(YK_ERR_INVALID, "yk_render: whitted max_depth above 24 is not supported");
-    if (n_tiles && !tiles) return yk_set_error(YK_ERR_INVALID, "yk_render: null tile list");
-    const yk_aov_films* aovs = nullptr;
-    if (opts && (opts->flags & YK_RENDER_AOVS)) {
-        if (!opts->aovs) return yk_set_error(YK_ERR_INVALID, "yk_render: YK_RENDER_AOVS without opts->aovs");
-        if (in->kind >= YK_INTEGRATOR_BVH_INTERSECTIONS)
-            return yk_set_error(YK_ERR_INVALID, "yk_render: companion films need the Path or Whitted integrator (the debug integrators are the views)");
-        if (in->kind == YK_INTEGRATOR_PATH && in->max_depth == 0)
-            return yk_set_error(YK_ERR_INVALID, "yk_render: companion films need a traced primary ray (Path max_depth 0 traces none)");
-        aovs = opts->aovs;
-    }
-    const yk_adaptive* adaptive = nullptr;
-    if (opts && (opts->flags & YK_RENDER_ADAPTIVE)) {
-        const yk_adaptive* a = opts->adaptive;
-        if (!a) return yk_set_error(YK_ERR_INVALID, "yk_render: YK_RENDER_ADAPTIVE without opts->adaptive");
-        if (a->min_samples < 2 || a->step == 0)
-            return yk_set_error(YK_ERR_INVALID, "yk_render: adaptive sampling needs min_samples >= 2 and step >= 1");
-        if (!std::isfinite(a->rel_error) || !std::isfinite(a->abs_error) || !(a->rel_error >= 0.0f) || !(a->abs_error >= 0.0f))
-            return yk_set_error(YK_ERR_INVALID, "yk_render: adaptive tolerances must be finite and >= 0");
-        if (fs->accumulate) return yk_set_error(YK_ERR_INVALID, "yk_render: adaptive sampling needs an averaging film (not accumulate)");
-        if (in->kind >= YK_INTEGRATOR_BVH_INTERSECTIONS)
-            return yk_set_error(YK_ERR_INVALID, "yk_render: adaptive sampling needs the Path or Whitted integrator");
-        adaptive = a;
-    }
-    const yk_thin_lens* lens = nullptr;
-    if (int rc = thin_lens_of(opts, "yk_render", &lens)) return rc;
-    std::lock_guard<std::recursive_mutex> guard(c->mu);
-    CUDA_TRY(cudaSetDevice(c->device));
-    (void)cudaGetLastError();  // do not inherit a stale error from an unrelated earlier call
-    cudaStream_t s = c->stream;
-    const uint32_t flags = opts ? opts->flags : 0u;
-    const bool on_device = (flags & YK_RENDER_FILM_ON_DEVICE) != 0;
-    const bool accumulate = fs->accumulate != 0;
-
-    // Pixel jobs: tile order, row-major inside a tile. Only the tile list and the prefix sum of the tile areas go to the
-    // device; each pixel group's jobs are expanded there (k_jobs_expand).
-    std::vector<unsigned long long> tile_off((size_t)n_tiles + 1, 0ull);
+        return yk_set_error(YK_ERR_INVALID, std::string(fn) + ": film resolution must fit u16 (integrators/mod.rs:140-141)");
+    return YK_OK;
+}
+// Every tile inside the film; *tile_off = the prefix sum of the tile areas (n_tiles + 1 entries).
+static int check_tiles(const yk_tile* tiles, uint32_t n_tiles, const yk_film_settings* fs, const char* fn,
+                       std::vector<unsigned long long>* tile_off) {
+    tile_off->assign((size_t)n_tiles + 1, 0ull);
     for (uint32_t t = 0; t < n_tiles; ++t) {
         const yk_tile& tl = tiles[t];
         if (tl.x0 >= tl.x1 || tl.y0 >= tl.y1 || tl.x1 > fs->res_x || tl.y1 > fs->res_y)
-            return yk_set_error(YK_ERR_INVALID, "yk_render: tile outside the film (film.rs:224-231)");
-        tile_off[t + 1] = tile_off[t] + (unsigned long long)(tl.x1 - tl.x0) * (tl.y1 - tl.y0);
+            return yk_set_error(YK_ERR_INVALID, std::string(fn) + ": tile outside the film (film.rs:224-231)");
+        (*tile_off)[t + 1] = (*tile_off)[t] + (unsigned long long)(tl.x1 - tl.x0) * (tl.y1 - tl.y0);
     }
-    const unsigned long long n_jobs_total = tile_off[n_tiles], area = n_jobs_total;
-    const size_t n_pixels = (size_t)fs->res_x * fs->res_y;
-    const uint32_t samples_per_job = accumulate ? 1u : spp;
+    return YK_OK;
+}
 
+// A render's per-pixel outputs: the film, the primary-hit id image, the companion films (AovSums order) and the adaptive
+// sample counts. Null: not requested.
+struct FilmArrays {
+    float* film = nullptr;
+    int32_t* hit_ids = nullptr;
+    float* views[kAovViews] = {};
+    uint32_t* counts = nullptr;
+};
+
+static FilmArrays caller_arrays(float* film_rgb, const yk_render_opts* opts, const yk_aov_films* aovs, const yk_adaptive* adaptive) {
+    FilmArrays f;
+    f.film = film_rgb;
+    f.hit_ids = opts ? opts->hit_ids : nullptr;
+    if (aovs) {
+        f.views[0] = aovs->bvh_intersections;
+        f.views[1] = aovs->geometry_normals;
+        f.views[2] = aovs->shading_normals;
+        f.views[3] = aovs->shading_uvs;
+        f.views[4] = aovs->radiance_sq;
+    }
+    if (adaptive) f.counts = adaptive->sample_counts;
+    return f;
+}
+
+// The context's film-sized buffers: the per-pixel sums, the film copy and the hit-id image.
+static int reserve_film(yk_context* c, size_t n_pixels) {
+    CUDA_TRY(c->d_accum.reserve(n_pixels * 3));
+    CUDA_TRY(c->d_film.reserve(n_pixels * 3));
+    CUDA_TRY(c->d_hit_ids.reserve(n_pixels));
+    return YK_OK;
+}
+
+// One output on the device: the caller's array itself (on_device), or the context's copy of the caller's host array, zeroed
+// when the render's tiles cover the whole averaging film (full_cover) and uploaded otherwise.
+template <class T>
+static int film_target(T* caller, DevArray<T>& copy, size_t count, bool on_device, bool full_cover, cudaStream_t s, T** out) {
+    *out = caller;
+    if (on_device) return YK_OK;
+    CUDA_TRY(copy.reserve(count));
+    *out = copy.get();
+    if (full_cover) CUDA_TRY(cudaMemsetAsync(*out, 0, count * sizeof(T), s));
+    else CUDA_TRY(cudaMemcpyAsync(*out, caller, count * sizeof(T), cudaMemcpyHostToDevice, s));
+    return YK_OK;
+}
+
+// The device side of the caller's outputs `out`, queued on s (film_target); the hit-id image starts at -1 when fill_ids.
+static int film_setup(yk_context* c, const FilmArrays& out, size_t n_pixels, bool on_device, bool full_cover, bool fill_ids,
+                      cudaStream_t s, FilmArrays* dev) {
+    int rc = reserve_film(c, n_pixels);
+    if (rc == YK_OK) rc = film_target(out.film, c->d_film, n_pixels * 3, on_device, full_cover, s, &dev->film);
+    if (rc != YK_OK) return rc;
+    if (out.hit_ids) {
+        dev->hit_ids = on_device ? out.hit_ids : c->d_hit_ids.get();
+        if (fill_ids) k_fill_i32<<<(unsigned)((n_pixels + 255) / 256), 256, 0, s>>>(dev->hit_ids, n_pixels, -1);
+    }
+    for (int k = 0; k < kAovViews; ++k)
+        if (out.views[k] && (rc = film_target(out.views[k], c->d_aov_film[k], n_pixels * 3, on_device, full_cover, s, &dev->views[k])) != YK_OK)
+            return rc;
+    if (out.counts) return film_target(out.counts, c->d_counts, n_pixels, on_device, full_cover, s, &dev->counts);
+    return YK_OK;
+}
+
+// The rendered outputs back into the caller's host arrays, queued on s.
+static int film_readback(const FilmArrays& out, const FilmArrays& dev, size_t n_pixels, cudaStream_t s) {
+    CUDA_TRY(cudaMemcpyAsync(out.film, dev.film, n_pixels * 3 * sizeof(float), cudaMemcpyDeviceToHost, s));
+    if (out.hit_ids) CUDA_TRY(cudaMemcpyAsync(out.hit_ids, dev.hit_ids, n_pixels * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+    for (int k = 0; k < kAovViews; ++k)
+        if (out.views[k]) CUDA_TRY(cudaMemcpyAsync(out.views[k], dev.views[k], n_pixels * 3 * sizeof(float), cudaMemcpyDeviceToHost, s));
+    if (out.counts) CUDA_TRY(cudaMemcpyAsync(out.counts, dev.counts, n_pixels * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+    return YK_OK;
+}
+
+// The kernels' settings of a render: sampler, camera, integrator, shadow mode and ray sort (hit_ids is set with the film).
+static RenderCfg render_cfg(const yk_context* c, const yk_scene* sc, const yk_camera* cam, const yk_film_settings* fs, const yk_sampler* sm,
+                            const yk_integrator* in, const yk_render_opts* opts, DebugLog* debug_log, const float* debug_px) {
     RenderCfg cfg{};
     cfg.sampler = SamplerCfg{};
     cfg.sampler.kind = sm->kind;
@@ -1200,88 +1228,346 @@ static int render_impl(yk_context* c, const yk_scene* sc, const yk_camera* cam, 
             cfg.sort_cell_scale[a] = ext > 0.0f ? 32.0f / ext : 0.0f;
         }
     }
+    return cfg;
+}
 
-    // Device film / accumulators.
-    if (c->film_cap < n_pixels) {
-        cudaFree(c->d_accum); cudaFree(c->d_film); cudaFree(c->d_hit_ids);
-        c->d_accum = nullptr; c->d_film = nullptr; c->d_hit_ids = nullptr;
-        c->film_cap = 0;
-        CUDA_TRY(cudaMalloc((void**)&c->d_accum, n_pixels * 3 * sizeof(float)));
-        CUDA_TRY(cudaMalloc((void**)&c->d_film, n_pixels * 3 * sizeof(float)));
-        CUDA_TRY(cudaMalloc((void**)&c->d_hit_ids, n_pixels * sizeof(int32_t)));
-        c->film_cap = n_pixels;
+// How a render's jobs (pixels of the tiles) are cut into batches and spread over the pipes.
+struct RenderPlan {
+    struct Group { unsigned long long first; uint32_t count, t_lo, t_hi; };  // jobs [first, first + count) lie in tiles [t_lo, t_hi)
+    uint32_t stack_entries;  // Whitted's per-path stack
+    uint32_t m;              // samples of one pixel per batch
+    uint32_t jobs_per_batch;
+    uint32_t wave_cap;       // paths in flight per batch
+    int n_pipes;
+    uint64_t total_paths;
+    std::vector<Group> groups;
+};
+
+static RenderPlan plan_render(yk_context* c, const yk_scene* sc, const yk_integrator* in, const yk_render_opts* opts, const yk_tile* tiles,
+                              uint32_t n_tiles, const std::vector<unsigned long long>& tile_off, uint32_t samples_per_job, bool accumulate) {
+    const unsigned long long n_jobs_total = tile_off[n_tiles];
+    // Wavefront capacity: paths in flight per batch. Fewer, longer launches amortise the persistent kernels' tails and the
+    // launch gaps, and HBM is 180 GB: measured 4 Mi -> 8 Mi -> 16 Mi paths = +8 %, +12 % on the Cornell bench (round 1), and
+    // 16 Mi -> 32 Mi -> 64 Mi = +0.7 %, +0.8 % there with two pipes (+2.5 %, +3.9 % with one) and +4.1 %, +6.4 % on the
+    // 10 M-triangle scene (profiles/r02/capsweep_large_batches.txt). Default: as many as ~24 GB of wavefront state per pipe
+    // hold (~360 B per path with one light), at most 64 Mi, and never more than a sixth of the free device memory per pipe.
+    const uint32_t stack_entries = in->kind == YK_INTEGRATOR_WHITTED ? std::max(in->max_depth, 1u) : 0u;
+    uint32_t cap = opts ? opts->wavefront_paths : 0u;
+    if (!cap) {
+        const uint64_t bytes_per_path = 320ull + 40ull * std::max(sc->dev.n_lights, 1u) + (80ull * stack_entries + (stack_entries ? 8ull : 0ull));
+        if (!c->mem_budget) {  // asked once per context: cudaMemGetInfo can take milliseconds
+            size_t free_b = 0, total_b = 0;
+            c->mem_budget = 24ull << 30;
+            if (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess) c->mem_budget = std::min<uint64_t>(c->mem_budget, (uint64_t)free_b / 6);
+        }
+        cap = (uint32_t)std::min<uint64_t>(1u << 26, std::max<uint64_t>(1u << 20, c->mem_budget / bytes_per_path));
     }
-    float* d_film = on_device ? film_rgb : c->d_film;
-    const bool full_cover = !accumulate && area == n_pixels;
-    if (!on_device) {
-        if (full_cover) CUDA_TRY(cudaMemsetAsync(d_film, 0, n_pixels * 3 * sizeof(float), s));
-        else CUDA_TRY(cudaMemcpyAsync(d_film, film_rgb, n_pixels * 3 * sizeof(float), cudaMemcpyHostToDevice, s));
+    const uint64_t total_paths = (uint64_t)n_jobs_total * samples_per_job;
+    if (cap > total_paths) cap = (uint32_t)total_paths;
+    cap = std::max(cap, 32u);
+    // Samples of one pixel per batch: enough to amortise per-batch fixed costs, few enough that many pixels
+    // (>= 64 Ki when available) share a batch.
+    uint32_t m = std::min(samples_per_job, kMaxBatchSamples);
+    if (const char* e = getenv("YK_MAX_BATCH_SAMPLES")) m = std::min<uint32_t>(m, (uint32_t)std::max(1, atoi(e)));  // development: A/B of the batch shape
+    while (m > 1 && (uint64_t)m * std::min<uint64_t>(n_jobs_total, 65536) > cap) m >>= 1;
+    uint32_t jobs_per_batch = std::max(1u, cap / m);
+    // Pipes: pixel groups alternate between the streams, so one group's latency-bound shading overlaps the other's
+    // issue-bound traversal. A pixel's samples stay on one pipe, in order (the film sum is order-dependent).
+    // The accumulating film adds with atomics across tiles, so it keeps to one stream.
+    // Default: two pipes. Measured on one box with the current kernels (profiles/r01/README.md): Cornell +5 %, config-4
+    // room +6 %, 1 M-triangle heightfield +10 %, 10 M-triangle terrain +12 %. Whitted's bounce loop waits for the host
+    // once per bounce, which would serialise the pipes, so it keeps one. YK_PIPES / opts->pipes override (bench.py
+    // times its device-resident leg on one pipe so that the event-bracketed kernel times stay exclusive).
+    int n_pipes = c->n_pipes_env > 0 ? c->n_pipes_env : (in->kind == YK_INTEGRATOR_WHITTED ? 1 : 2);
+    if (opts && opts->pipes) n_pipes = (int)opts->pipes;
+    n_pipes = std::max(1, std::min(kMaxPipes, n_pipes));
+    if (accumulate) n_pipes = 1;
+    // Pixel groups of equal size, their number a multiple of the pipe count: a ragged tail (a last group of a fraction of a
+    // batch, or an odd group that runs on one pipe with nothing beside it) cost a 2-GPU yk_multi_render whose runs are
+    // not multiples of a group 8 ms per run. Fewer pixel groups than pipes: split the jobs evenly if that leaves decent
+    // batches, else use fewer pipes.
+    if (!accumulate) {
+        for (;;) {
+            unsigned long long n_g = (n_jobs_total + jobs_per_batch - 1) / jobs_per_batch;
+            n_g = (n_g + n_pipes - 1) / n_pipes * n_pipes;
+            const unsigned long long per = (n_jobs_total + n_g - 1) / n_g;
+            if (n_pipes == 1 || per * m >= (1u << 20) || n_g > (unsigned long long)n_pipes) {
+                jobs_per_batch = (uint32_t)std::max<unsigned long long>(1, per);
+                break;
+            }
+            n_pipes -= 1;
+        }
     }
-    int32_t* d_ids = nullptr;
-    if (opts && opts->hit_ids) {
-        d_ids = on_device ? opts->hit_ids : c->d_hit_ids;
-        if (!(flags & kRenderAuxInitialised)) k_fill_i32<<<(unsigned)((n_pixels + 255) / 256), 256, 0, s>>>(d_ids, n_pixels, -1);
-    }
-    cfg.hit_ids = d_ids;
-    // Companion films: each requested view on the device (the caller's buffer, or a copy of the host buffer made like d_film's),
-    // and the per-pixel sums its kernels add into (accumulating films: the view itself).
-    float* d_aov[kAovViews] = {};
-    AovSums aov_sums{};
-    auto ensure = [&](float** buf, size_t* cap) -> int {
-        if (*cap >= n_pixels) return YK_OK;
-        cudaFree(*buf);
-        *buf = nullptr;
-        *cap = 0;
-        CUDA_TRY(cudaMalloc((void**)buf, n_pixels * 3 * sizeof(float)));
-        *cap = n_pixels;
-        return YK_OK;
+    const uint32_t wave_cap = (uint32_t)std::min<uint64_t>(cap, (uint64_t)jobs_per_batch * m);
+    // Pixel groups: consecutive runs of at most jobs_per_batch jobs. The accumulating film adds every batch into the
+    // film in stream order, so a group never spans a change of `tile.sample`: within one sample index the reference's
+    // tiles are disjoint, each pixel appears once per batch and the per-pixel sum runs in tile-list order exactly
+    // like the reference's `*fc += c` (film.rs:260-272).
+    std::vector<RenderPlan::Group> groups;
+    uint32_t seg_t0 = 0;
+    auto flush = [&](uint32_t seg_t1) {  // the jobs of tiles [seg_t0, seg_t1)
+        uint32_t t = seg_t0;
+        for (unsigned long long j = tile_off[seg_t0]; j < tile_off[seg_t1]; j += jobs_per_batch) {
+            const unsigned long long end = std::min<unsigned long long>(j + jobs_per_batch, tile_off[seg_t1]);
+            while (tile_off[t + 1] <= j) ++t;
+            uint32_t t_hi = t + 1;
+            while (tile_off[t_hi] < end) ++t_hi;
+            groups.push_back(RenderPlan::Group{j, (uint32_t)(end - j), t, t_hi});
+        }
+        seg_t0 = seg_t1;
     };
-    if (aovs) {
-        float* views[kAovViews];
-        aov_views(aovs, views);
-        for (int k = 0; k < kAovViews; ++k) {
-            if (!views[k]) continue;
-            int rc = YK_OK;
-            if (on_device) d_aov[k] = views[k];
-            else {
-                if ((rc = ensure(&c->d_aov_film[k], &c->aov_film_cap[k])) != YK_OK) return rc;
-                d_aov[k] = c->d_aov_film[k];
-                if (full_cover) CUDA_TRY(cudaMemsetAsync(d_aov[k], 0, n_pixels * 3 * sizeof(float), s));
-                else CUDA_TRY(cudaMemcpyAsync(d_aov[k], views[k], n_pixels * 3 * sizeof(float), cudaMemcpyHostToDevice, s));
+    if (accumulate)
+        for (uint32_t t = 1; t < n_tiles; ++t)
+            if (tiles[t].sample != tiles[t - 1].sample) flush(t);
+    flush(n_tiles);
+    return RenderPlan{stack_entries, m, jobs_per_batch, wave_cap, n_pipes, total_paths, std::move(groups)};
+}
+
+// What the batch loop of one render reads besides its plan.
+struct RenderCall {
+    const yk_scene* sc;
+    const yk_render_opts* opts;
+    const yk_tile* tiles;
+    uint32_t n_tiles;
+    const std::vector<unsigned long long>* tile_off;
+    const yk_adaptive* adaptive;
+    const yk_thin_lens* lens;
+    bool accumulate;
+    uint32_t spp, samples_per_job;
+    RenderCfg cfg;
+    FilmArrays dev;          // the outputs on the device (film_setup)
+    AovSums aov_sums;        // the per-pixel sums the companion films (and the adaptive li * li) add into
+    AovSums adaptive_views;  // the companion films k_adaptive_check stores a stopped pixel into
+};
+
+// The plan's pixel groups, batch by batch on the pipes, and the wait for all of them: the counters into *totals, the paths
+// finished into *done, *cancelled when the progress callback asked to stop. On an error return batches may still be queued
+// or marked busy (render_impl clears them).
+static int run_groups(yk_context* c, const RenderCall& r, const RenderPlan& plan, Timers* tm, Totals* totals, uint64_t* done,
+                      bool* cancelled) {
+    const yk_scene* sc = r.sc;
+    const yk_adaptive* adaptive = r.adaptive;
+    const uint32_t res_x = r.cfg.res_x, samples_per_job = r.samples_per_job, n_tiles = r.n_tiles;
+    const int n_pipes = plan.n_pipes;
+    cudaStream_t s = c->stream;
+    CUDA_TRY(c->d_tiles.reserve(n_tiles));
+    CUDA_TRY(c->d_tile_off.reserve((size_t)n_tiles + 1));
+    CUDA_TRY(cudaMemcpyAsync(c->d_tiles.get(), r.tiles, (size_t)n_tiles * sizeof(yk_tile), cudaMemcpyHostToDevice, s));
+    CUDA_TRY(cudaMemcpyAsync(c->d_tile_off.get(), r.tile_off->data(), r.tile_off->size() * sizeof(unsigned long long), cudaMemcpyHostToDevice, s));
+    int rc = YK_OK;
+    CUDA_TRY(cudaEventRecord(c->ev[0], s));
+    for (int pi = 0; pi < n_pipes; ++pi) {
+        Pipe& p = c->pipe[pi];
+        if ((rc = ensure_wave(&p, plan.wave_cap, sc->dev.n_lights, plan.stack_entries, r.cfg.sort_key_mode != 0)) != YK_OK) return rc;
+        if (pi > 0) CUDA_TRY(cudaStreamWaitEvent(p.stream, c->ev[0], 0));
+        CUDA_TRY(cudaMemsetAsync(p.wave.totals, 0, sizeof(Totals), p.stream));
+        p.hash_group = (size_t)-1;
+        p.survivors_pending = false;
+        p.rehash = false;
+    }
+    const size_t n_groups = plan.groups.size();
+    // The samples [s0, s1) of a batch: at most m, and, with adaptive sampling, never past the next check point (min_samples,
+    // min_samples + step, ...), so that the stopping decisions do not depend on the batch shape.
+    auto batch_end = [&](uint32_t s0) -> uint32_t {
+        uint32_t s1 = std::min(samples_per_job, s0 + plan.m);
+        if (adaptive) {
+            const uint32_t lo = adaptive->min_samples, st_ = adaptive->step;
+            const uint64_t check = s0 < lo ? lo : lo + ((uint64_t)(s0 - lo) / st_ + 1) * st_;
+            s1 = (uint32_t)std::min<uint64_t>(s1, check);
+        }
+        return s1;
+    };
+    for (size_t g0 = 0; g0 < n_groups && !*cancelled; g0 += n_pipes) {
+        uint32_t active[kMaxPipes] = {};  // adaptive: the jobs of each pipe's group still sampling (its job list's length)
+        for (uint32_t s0 = 0, s1 = 0; s0 < samples_per_job && !*cancelled; s0 = s1) {
+            s1 = batch_end(s0);
+            bool any = false;
+            for (int pi = 0; pi < n_pipes && g0 + pi < n_groups && !*cancelled; ++pi) {
+                Pipe& p = c->pipe[pi];
+                const size_t group = g0 + pi;
+                const RenderPlan::Group& gr = plan.groups[group];
+                uint32_t nj = gr.count;
+                if (adaptive && p.hash_group == group) {
+                    if (p.survivors_pending) {  // the last check's survivors: the other pipe keeps running meanwhile
+                        CUDA_TRY(cudaStreamSynchronize(p.stream));
+                        active[pi] = *p.h_survivors;
+                        p.survivors_pending = false;
+                    }
+                    nj = active[pi];
+                    if (!nj) continue;  // every pixel of the group has stopped
+                }
+                any = true;
+                active[pi] = nj;
+                if (p.hash_group != group) {  // a new pixel group on this pipe: its jobs, and a zeroed accumulator
+                    if (p.d_jobs.capacity() < nj) {
+                        CUDA_TRY(cudaStreamSynchronize(p.stream));
+                        CUDA_TRY(p.d_jobs.reserve(std::max(nj, plan.jobs_per_batch)));
+                    }
+                    k_jobs_expand<<<(nj + 255) / 256, 256, 0, p.stream>>>(c->d_tiles.get(), c->d_tile_off.get(), gr.t_lo, gr.t_hi, gr.first, nj,
+                                                                           r.accumulate ? 1u : 0u, p.d_jobs.get());
+                    tm->launches += 1;
+                    if (!r.accumulate) {
+                        k_zero_jobs<<<(nj + 255) / 256, 256, 0, p.stream>>>(p.d_jobs.get(), nj, c->d_accum.get(), res_x);
+                        tm->launches += 1;
+                        for (float* sums : r.aov_sums.v) {
+                            if (!sums) continue;
+                            k_zero_jobs<<<(nj + 255) / 256, 256, 0, p.stream>>>(p.d_jobs.get(), nj, sums, res_x);
+                            tm->launches += 1;
+                        }
+                    }
+                    if (r.cfg.debug_log) {
+                        k_debug_job<<<1, 1, 0, p.stream>>>(p.d_jobs.get());
+                        tm->launches += 1;
+                    }
+                }
+                RenderCfg gcfg = r.cfg;
+                if (r.cfg.sampler.kind == YK_SAMPLER_STRATIFIED) {
+                    // tabulate the (pixel, dimension) hashes of this pixel group once for all of its samples
+                    const uint64_t camera_dims = r.lens ? 4 : 2;  // the film jitter, and the lens sample
+                    uint64_t dims = camera_dims;
+                    if (r.cfg.integrator == YK_INTEGRATOR_PATH) dims = camera_dims + (uint64_t)r.cfg.max_depth * (2ull * sc->dev.n_lights + 3);
+                    else if (r.cfg.integrator == YK_INTEGRATOR_WHITTED)
+                        dims = camera_dims + 2ull * sc->dev.n_lights * ((1ull << std::min(r.cfg.max_depth, 8u)) - 1);
+                    dims = std::min<uint64_t>(dims, std::min<uint64_t>(4096, (256ull << 20) / (4ull * nj)));  // the rest is hashed on the fly
+                    if (p.hash_group != group || p.rehash) {
+                        const size_t need = (size_t)dims * nj;
+                        if (p.d_dim_hash.capacity() < need) {
+                            CUDA_TRY(cudaStreamSynchronize(p.stream));
+                            CUDA_TRY(p.d_dim_hash.reserve(need));
+                        }
+                        k_dim_hashes<<<dim3((nj + 255) / 256, (unsigned)std::min<uint64_t>(dims, 64)), 256, 0, p.stream>>>(
+                            p.d_jobs.get(), nj, (uint32_t)dims, r.cfg.sampler.seed, p.d_dim_hash.get());
+                        tm->launches += 1;
+                    }
+                    gcfg.sampler.hash_table = p.d_dim_hash.get();
+                    gcfg.sampler.n_hash_dims = (uint32_t)dims;
+                    gcfg.sampler.hash_stride = nj;
+                }
+                p.hash_group = group;
+                p.rehash = false;
+                Batch bt;
+                bt.jobs = p.d_jobs.get();
+                bt.n_jobs = nj;
+                bt.div_jobs = FastDiv::make(nj);
+                bt.sample_off = s0;
+                bt.n_samples = s1 - s0;
+                bt.n_paths = nj * bt.n_samples;
+                // the batch's first sample index: s0, or the sample of the group's tiles (accumulating films: one per group)
+                const uint32_t first_sample = r.accumulate ? (uint32_t)r.tiles[gr.t_lo].sample : s0;
+                if ((rc = run_batch(c, &p, sc, gcfg, bt, first_sample, r.accumulate, r.dev.film, r.aov_sums, r.lens, tm, done)) != YK_OK) return rc;
+                if (adaptive) {
+                    const bool last = s1 >= samples_per_job;
+                    if (last || (s1 >= adaptive->min_samples && (s1 - adaptive->min_samples) % adaptive->step == 0))
+                        if ((rc = adaptive_check(&p, nj, s1, last, *adaptive, res_x, c->d_accum.get(), r.aov_sums, r.adaptive_views, r.dev.film,
+                                                 r.dev.counts, tm)) != YK_OK)
+                            return rc;
+                } else if (!r.accumulate && s1 >= samples_per_job) {
+                    // the group's last samples are queued: `color /= sample_count` + Film::update_tile for its pixels
+                    k_film_store<<<(nj + 255) / 256, 256, 0, p.stream>>>(p.d_jobs.get(), nj, c->d_accum.get(), r.dev.film, res_x, (float)r.spp);
+                    tm->launches += 1;
+                    for (int k = 0; k < kAovViews; ++k) {
+                        if (!r.dev.views[k]) continue;
+                        k_film_store<<<(nj + 255) / 256, 256, 0, p.stream>>>(p.d_jobs.get(), nj, r.aov_sums.v[k], r.dev.views[k], res_x, (float)r.spp);
+                        tm->launches += 1;
+                    }
+                }
+                const yk_render_opts* opts = r.opts;
+                if (opts && opts->progress && opts->progress(opts->progress_user, *done, plan.total_paths)) *cancelled = true;
             }
-            if (accumulate) aov_sums.v[k] = d_aov[k];
-            else {
-                if ((rc = ensure(&c->d_aov_sums[k], &c->aov_sums_cap[k])) != YK_OK) return rc;
-                aov_sums.v[k] = c->d_aov_sums[k];
-            }
+            if (!any) break;
         }
     }
-    // Adaptive sampling: the sums of li * li the stopping rule reads (radiance_sq's, else a scratch accumulator that the
-    // render zeroes and sums like a companion film), and the per-pixel counts on the device (kept outside `tiles`, like d_film).
-    uint32_t* d_counts = nullptr;
-    AovSums adaptive_views{};
+    for (int pi = 0; pi < n_pipes; ++pi) {
+        Pipe& p = c->pipe[pi];
+        CUDA_TRY(cudaMemcpyAsync(p.h_totals, p.wave.totals, sizeof(Totals), cudaMemcpyDeviceToHost, p.stream));
+        for (int k = 0; k < kRing; ++k)
+            if ((rc = retire_slot(&p, k, tm, done)) != YK_OK) return rc;
+        CUDA_TRY(cudaStreamSynchronize(p.stream));
+        const Totals& t = *p.h_totals;
+        totals->closest_nodes += t.closest_nodes; totals->closest_tris += t.closest_tris;
+        totals->any_nodes += t.any_nodes; totals->any_tris += t.any_tris;
+        totals->hit_hash += t.hit_hash; totals->shadow_rays += t.shadow_rays; totals->closest_rays += t.closest_rays;
+    }
+    return YK_OK;
+}
+
+// yk_render, and yk_debug_ray's single path (`debug_log` = device ray list, `debug_px` = the film pixel of its camera sample).
+static int render_impl(yk_context* c, const yk_scene* sc, const yk_camera* cam, const yk_film_settings* fs, const yk_sampler* sm,
+                       const yk_integrator* in, const yk_tile* tiles, uint32_t n_tiles, const yk_render_opts* opts, float* film_rgb,
+                       yk_stats* stats, DebugLog* debug_log, const float* debug_px) {
+    const auto wall0 = std::chrono::steady_clock::now();
+    if (!c || !sc || !cam || !fs || !sm || !in || !film_rgb) return yk_set_error(YK_ERR_INVALID, "yk_render: null argument");
+    if (sc->ctx != c) return yk_set_error(YK_ERR_INVALID, "yk_render: scene belongs to another context");
+    if (int rc = check_resolution(fs, "yk_render")) return rc;
+    if (in->kind > YK_INTEGRATOR_SHADING_UVS) return yk_set_error(YK_ERR_INVALID, "yk_render: unknown integrator");
+    if (sm->kind > YK_SAMPLER_STRATIFIED) return yk_set_error(YK_ERR_INVALID, "yk_render: unknown sampler");
+    const uint32_t spp = sm->kind == YK_SAMPLER_UNIFORM ? sm->nx : sm->nx * sm->ny;
+    if (spp == 0 || spp > 0x10000u) return yk_set_error(YK_ERR_INVALID, "yk_render: samples per pixel must be in 1..65536");
+    if (in->max_depth > 255) return yk_set_error(YK_ERR_INVALID, "yk_render: max_depth above 255");
+    if (in->kind == YK_INTEGRATOR_WHITTED && in->max_depth > 24)
+        return yk_set_error(YK_ERR_INVALID, "yk_render: whitted max_depth above 24 is not supported");
+    if (n_tiles && !tiles) return yk_set_error(YK_ERR_INVALID, "yk_render: null tile list");
+    const yk_aov_films* aovs = nullptr;
+    if (opts && (opts->flags & YK_RENDER_AOVS)) {
+        if (!opts->aovs) return yk_set_error(YK_ERR_INVALID, "yk_render: YK_RENDER_AOVS without opts->aovs");
+        if (in->kind >= YK_INTEGRATOR_BVH_INTERSECTIONS)
+            return yk_set_error(YK_ERR_INVALID, "yk_render: companion films need the Path or Whitted integrator (the debug integrators are the views)");
+        if (in->kind == YK_INTEGRATOR_PATH && in->max_depth == 0)
+            return yk_set_error(YK_ERR_INVALID, "yk_render: companion films need a traced primary ray (Path max_depth 0 traces none)");
+        aovs = opts->aovs;
+    }
+    const yk_adaptive* adaptive = nullptr;
+    if (opts && (opts->flags & YK_RENDER_ADAPTIVE)) {
+        const yk_adaptive* a = opts->adaptive;
+        if (!a) return yk_set_error(YK_ERR_INVALID, "yk_render: YK_RENDER_ADAPTIVE without opts->adaptive");
+        if (a->min_samples < 2 || a->step == 0)
+            return yk_set_error(YK_ERR_INVALID, "yk_render: adaptive sampling needs min_samples >= 2 and step >= 1");
+        if (!std::isfinite(a->rel_error) || !std::isfinite(a->abs_error) || !(a->rel_error >= 0.0f) || !(a->abs_error >= 0.0f))
+            return yk_set_error(YK_ERR_INVALID, "yk_render: adaptive tolerances must be finite and >= 0");
+        if (fs->accumulate) return yk_set_error(YK_ERR_INVALID, "yk_render: adaptive sampling needs an averaging film (not accumulate)");
+        if (in->kind >= YK_INTEGRATOR_BVH_INTERSECTIONS)
+            return yk_set_error(YK_ERR_INVALID, "yk_render: adaptive sampling needs the Path or Whitted integrator");
+        adaptive = a;
+    }
+    const yk_thin_lens* lens = nullptr;
+    if (int rc = thin_lens_of(opts, "yk_render", &lens)) return rc;
+    // Pixel jobs: tile order, row-major inside a tile. Only the tile list and the prefix sum of the tile areas go to the
+    // device; each pixel group's jobs are expanded there (k_jobs_expand).
+    std::vector<unsigned long long> tile_off;
+    if (int rc = check_tiles(tiles, n_tiles, fs, "yk_render", &tile_off)) return rc;
+    std::lock_guard<std::recursive_mutex> guard(c->mu);
+    CUDA_TRY(cudaSetDevice(c->device));
+    (void)cudaGetLastError();  // do not inherit a stale error from an unrelated earlier call
+    cudaStream_t s = c->stream;
+    const uint32_t flags = opts ? opts->flags : 0u;
+    const bool on_device = (flags & YK_RENDER_FILM_ON_DEVICE) != 0;
+    const bool accumulate = fs->accumulate != 0;
+    const unsigned long long n_jobs_total = tile_off[n_tiles];
+    const size_t n_pixels = (size_t)fs->res_x * fs->res_y;
+    RenderCall r{sc, opts, tiles, n_tiles, &tile_off, adaptive, lens, accumulate, spp, accumulate ? 1u : spp};
+    r.cfg = render_cfg(c, sc, cam, fs, sm, in, opts, debug_log, debug_px);
+
+    // The outputs on the device, and the per-pixel sums their kernels add into (accumulating films: the views themselves).
+    // Adaptive sampling reads the sums of li * li (radiance_sq's, else a scratch accumulator that the render zeroes and sums
+    // like a companion film).
+    const FilmArrays out = caller_arrays(film_rgb, opts, aovs, adaptive);
+    int rc = film_setup(c, out, n_pixels, on_device, !accumulate && n_jobs_total == n_pixels, !(flags & kRenderAuxInitialised), s, &r.dev);
+    if (rc != YK_OK) return rc;
+    r.cfg.hit_ids = r.dev.hit_ids;
+    for (int k = 0; k < kAovViews; ++k) {
+        if (!r.dev.views[k]) continue;
+        if (accumulate) r.aov_sums.v[k] = r.dev.views[k];
+        else {
+            CUDA_TRY(c->d_aov_sums[k].reserve(n_pixels * 3));
+            r.aov_sums.v[k] = c->d_aov_sums[k].get();
+        }
+    }
     if (adaptive) {
-        if (!aov_sums.v[kAovRadianceSq]) {
-            int rc = ensure(&c->d_adaptive_sq, &c->adaptive_sq_cap);
-            if (rc != YK_OK) return rc;
-            aov_sums.v[kAovRadianceSq] = c->d_adaptive_sq;
+        if (!r.aov_sums.v[kAovRadianceSq]) {
+            CUDA_TRY(c->d_adaptive_sq.reserve(n_pixels * 3));
+            r.aov_sums.v[kAovRadianceSq] = c->d_adaptive_sq.get();
         }
-        for (int k = 0; k < kAovViews; ++k) adaptive_views.v[k] = d_aov[k];
-        if (adaptive->sample_counts) {
-            if (on_device) d_counts = adaptive->sample_counts;
-            else {
-                if (c->counts_cap < n_pixels) {
-                    cudaFree(c->d_counts);
-                    c->d_counts = nullptr;
-                    c->counts_cap = 0;
-                    CUDA_TRY(cudaMalloc((void**)&c->d_counts, n_pixels * sizeof(uint32_t)));
-                    c->counts_cap = n_pixels;
-                }
-                d_counts = c->d_counts;
-                if (full_cover) CUDA_TRY(cudaMemsetAsync(d_counts, 0, n_pixels * sizeof(uint32_t), s));
-                else CUDA_TRY(cudaMemcpyAsync(d_counts, adaptive->sample_counts, n_pixels * sizeof(uint32_t), cudaMemcpyHostToDevice, s));
-            }
-        }
+        for (int k = 0; k < kAovViews; ++k) r.adaptive_views.v[k] = r.dev.views[k];
     }
 
     yk_stats st{};
@@ -1289,267 +1575,24 @@ static int render_impl(yk_context* c, const yk_scene* sc, const yk_camera* cam, 
     Totals totals{};
     CUDA_TRY(cudaEventRecord(c->ev[2], s));
     if (n_jobs_total) {
-        if (c->tiles_cap < n_tiles) {
-            cudaFree(c->d_tiles);
-            cudaFree(c->d_tile_off);
-            c->d_tiles = nullptr;
-            c->d_tile_off = nullptr;
-            c->tiles_cap = 0;
-            CUDA_TRY(cudaMalloc((void**)&c->d_tiles, (size_t)n_tiles * sizeof(yk_tile)));
-            CUDA_TRY(cudaMalloc((void**)&c->d_tile_off, ((size_t)n_tiles + 1) * sizeof(unsigned long long)));
-            c->tiles_cap = n_tiles;
-        }
-        CUDA_TRY(cudaMemcpyAsync(c->d_tiles, tiles, (size_t)n_tiles * sizeof(yk_tile), cudaMemcpyHostToDevice, s));
-        CUDA_TRY(cudaMemcpyAsync(c->d_tile_off, tile_off.data(), tile_off.size() * sizeof(unsigned long long), cudaMemcpyHostToDevice, s));
-        // Wavefront capacity: paths in flight per batch. Fewer, longer launches amortise the persistent kernels' tails and the
-        // launch gaps, and HBM is 180 GB: measured 4 Mi -> 8 Mi -> 16 Mi paths = +8 %, +12 % on the Cornell bench (round 1), and
-        // 16 Mi -> 32 Mi -> 64 Mi = +0.7 %, +0.8 % there with two pipes (+2.5 %, +3.9 % with one) and +4.1 %, +6.4 % on the
-        // 10 M-triangle scene (profiles/r02/capsweep_large_batches.txt). Default: as many as ~24 GB of wavefront state per pipe
-        // hold (~360 B per path with one light), at most 64 Mi, and never more than a sixth of the free device memory per pipe.
-        const uint32_t stack_entries = in->kind == YK_INTEGRATOR_WHITTED ? std::max(in->max_depth, 1u) : 0u;
-        uint32_t cap = opts ? opts->wavefront_paths : 0u;
-        if (!cap) {
-            const uint64_t bytes_per_path = 320ull + 40ull * std::max(sc->dev.n_lights, 1u) + (80ull * stack_entries + (stack_entries ? 8ull : 0ull));
-            if (!c->mem_budget) {  // asked once per context: cudaMemGetInfo can take milliseconds
-                size_t free_b = 0, total_b = 0;
-                c->mem_budget = 24ull << 30;
-                if (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess) c->mem_budget = std::min<uint64_t>(c->mem_budget, (uint64_t)free_b / 6);
-            }
-            cap = (uint32_t)std::min<uint64_t>(1u << 26, std::max<uint64_t>(1u << 20, c->mem_budget / bytes_per_path));
-        }
-        const uint64_t total_paths = (uint64_t)n_jobs_total * samples_per_job;
-        if (cap > total_paths) cap = (uint32_t)total_paths;
-        cap = std::max(cap, 32u);
-        // Samples of one pixel per batch: enough to amortise per-batch fixed costs, few enough that many pixels
-        // (>= 64 Ki when available) share a batch.
-        uint32_t m = std::min(samples_per_job, kMaxBatchSamples);
-        if (const char* e = getenv("YK_MAX_BATCH_SAMPLES")) m = std::min<uint32_t>(m, (uint32_t)std::max(1, atoi(e)));  // development: A/B of the batch shape
-        while (m > 1 && (uint64_t)m * std::min<uint64_t>(n_jobs_total, 65536) > cap) m >>= 1;
-        uint32_t jobs_per_batch = std::max(1u, cap / m);
-        // Pipes: pixel groups alternate between the streams, so one group's latency-bound shading overlaps the other's
-        // issue-bound traversal. A pixel's samples stay on one pipe, in order (the film sum is order-dependent).
-        // The accumulating film adds with atomics across tiles, so it keeps to one stream.
-        // Default: two pipes. Measured on one box with the current kernels (profiles/r01/README.md): Cornell +5 %, config-4
-        // room +6 %, 1 M-triangle heightfield +10 %, 10 M-triangle terrain +12 %. Whitted's bounce loop waits for the host
-        // once per bounce, which would serialise the pipes, so it keeps one. YK_PIPES / opts->pipes override (bench.py
-        // times its device-resident leg on one pipe so that the event-bracketed kernel times stay exclusive).
-        int n_pipes = c->n_pipes_env > 0 ? c->n_pipes_env : (in->kind == YK_INTEGRATOR_WHITTED ? 1 : 2);
-        if (opts && opts->pipes) n_pipes = (int)opts->pipes;
-        n_pipes = std::max(1, std::min(kMaxPipes, n_pipes));
-        if (accumulate) n_pipes = 1;
-        // Pixel groups of equal size, their number a multiple of the pipe count: a ragged tail (a last group of a fraction of a
-        // batch, or an odd group that runs on one pipe with nothing beside it) cost a 2-GPU yk_multi_render whose runs are
-        // not multiples of a group 8 ms per run. Fewer pixel groups than pipes: split the jobs evenly if that leaves decent
-        // batches, else use fewer pipes.
-        if (!accumulate) {
-            for (;;) {
-                unsigned long long n_g = (n_jobs_total + jobs_per_batch - 1) / jobs_per_batch;
-                n_g = (n_g + n_pipes - 1) / n_pipes * n_pipes;
-                const unsigned long long per = (n_jobs_total + n_g - 1) / n_g;
-                if (n_pipes == 1 || per * m >= (1u << 20) || n_g > (unsigned long long)n_pipes) {
-                    jobs_per_batch = (uint32_t)std::max<unsigned long long>(1, per);
-                    break;
-                }
-                n_pipes -= 1;
-            }
-        }
-        const uint32_t wave_cap = (uint32_t)std::min<uint64_t>(cap, (uint64_t)jobs_per_batch * m);
-        int rc = YK_OK;
-        CUDA_TRY(cudaEventRecord(c->ev[0], s));
-        for (int pi = 0; pi < n_pipes; ++pi) {
-            Pipe& p = c->pipe[pi];
-            if ((rc = ensure_wave(&p, wave_cap, sc->dev.n_lights, stack_entries, cfg.sort_key_mode != 0)) != YK_OK) return rc;
-            if (pi > 0) CUDA_TRY(cudaStreamWaitEvent(p.stream, c->ev[0], 0));
-            CUDA_TRY(cudaMemsetAsync(p.wave.totals, 0, sizeof(Totals), p.stream));
-            p.hash_group = (size_t)-1;
-            p.survivors_pending = false;
-            p.rehash = false;
-        }
-        // Pixel groups: consecutive runs of at most jobs_per_batch jobs. The accumulating film adds every batch into the
-        // film in stream order, so a group never spans a change of `tile.sample`: within one sample index the reference's
-        // tiles are disjoint, each pixel appears once per batch and the per-pixel sum runs in tile-list order exactly
-        // like the reference's `*fc += c` (film.rs:260-272).
-        struct Group { unsigned long long first; uint32_t count, t_lo, t_hi; };  // jobs [first, first + count) lie in tiles [t_lo, t_hi)
-        std::vector<Group> groups;
-        {
-            uint32_t seg_t0 = 0;
-            auto flush = [&](uint32_t seg_t1) {  // the jobs of tiles [seg_t0, seg_t1)
-                uint32_t t = seg_t0;
-                for (unsigned long long j = tile_off[seg_t0]; j < tile_off[seg_t1]; j += jobs_per_batch) {
-                    const unsigned long long end = std::min<unsigned long long>(j + jobs_per_batch, tile_off[seg_t1]);
-                    while (tile_off[t + 1] <= j) ++t;
-                    uint32_t t_hi = t + 1;
-                    while (tile_off[t_hi] < end) ++t_hi;
-                    groups.push_back(Group{j, (uint32_t)(end - j), t, t_hi});
-                }
-                seg_t0 = seg_t1;
-            };
-            if (accumulate)
-                for (uint32_t t = 1; t < n_tiles; ++t)
-                    if (tiles[t].sample != tiles[t - 1].sample) flush(t);
-            flush(n_tiles);
-        }
-        const size_t n_groups = groups.size();
+        const RenderPlan plan = plan_render(c, sc, in, opts, tiles, n_tiles, tile_off, r.samples_per_job, accumulate);
         uint64_t done = 0;
         bool cancelled = false;
-        // The samples [s0, s1) of a batch: at most m, and, with adaptive sampling, never past the next check point (min_samples,
-        // min_samples + step, ...), so that the stopping decisions do not depend on the batch shape.
-        auto batch_end = [&](uint32_t s0) -> uint32_t {
-            uint32_t s1 = std::min(samples_per_job, s0 + m);
-            if (adaptive) {
-                const uint32_t lo = adaptive->min_samples, st_ = adaptive->step;
-                const uint64_t check = s0 < lo ? lo : lo + ((uint64_t)(s0 - lo) / st_ + 1) * st_;
-                s1 = (uint32_t)std::min<uint64_t>(s1, check);
-            }
-            return s1;
-        };
-        for (size_t g0 = 0; g0 < n_groups && !cancelled; g0 += n_pipes) {
-            uint32_t active[kMaxPipes] = {};  // adaptive: the jobs of each pipe's group still sampling (its job list's length)
-            for (uint32_t s0 = 0, s1 = 0; s0 < samples_per_job && !cancelled; s0 = s1) {
-                s1 = batch_end(s0);
-                bool any = false;
-                for (int pi = 0; pi < n_pipes && g0 + pi < n_groups && !cancelled; ++pi) {
-                    Pipe& p = c->pipe[pi];
-                    const size_t group = g0 + pi;
-                    uint32_t nj = groups[group].count;
-                    if (adaptive && p.hash_group == group) {
-                        if (p.survivors_pending) {  // the last check's survivors: the other pipe keeps running meanwhile
-                            CUDA_TRY(cudaStreamSynchronize(p.stream));
-                            active[pi] = *p.h_survivors;
-                            p.survivors_pending = false;
-                        }
-                        nj = active[pi];
-                        if (!nj) continue;  // every pixel of the group has stopped
-                    }
-                    any = true;
-                    active[pi] = nj;
-                    if (p.hash_group != group) {  // a new pixel group on this pipe: its jobs, and a zeroed accumulator
-                        if (p.jobs_cap < nj) {
-                            CUDA_TRY(cudaStreamSynchronize(p.stream));
-                            cudaFree(p.d_jobs);
-                            p.d_jobs = nullptr;
-                            p.jobs_cap = 0;
-                            CUDA_TRY(cudaMalloc((void**)&p.d_jobs, (size_t)std::max(nj, jobs_per_batch) * sizeof(Job)));
-                            p.jobs_cap = std::max(nj, jobs_per_batch);
-                        }
-                        k_jobs_expand<<<(nj + 255) / 256, 256, 0, p.stream>>>(c->d_tiles, c->d_tile_off, groups[group].t_lo, groups[group].t_hi,
-                                                                               groups[group].first, nj, accumulate ? 1u : 0u, p.d_jobs);
-                        tm.launches += 1;
-                        if (!accumulate) {
-                            k_zero_jobs<<<(nj + 255) / 256, 256, 0, p.stream>>>(p.d_jobs, nj, c->d_accum, fs->res_x);
-                            tm.launches += 1;
-                            for (float* sums : aov_sums.v) {
-                                if (!sums) continue;
-                                k_zero_jobs<<<(nj + 255) / 256, 256, 0, p.stream>>>(p.d_jobs, nj, sums, fs->res_x);
-                                tm.launches += 1;
-                            }
-                        }
-                        if (debug_log) {
-                            k_debug_job<<<1, 1, 0, p.stream>>>(p.d_jobs);
-                            tm.launches += 1;
-                        }
-                    }
-                    RenderCfg gcfg = cfg;
-                    if (sm->kind == YK_SAMPLER_STRATIFIED) {
-                        // tabulate the (pixel, dimension) hashes of this pixel group once for all of its samples
-                        const uint64_t camera_dims = lens ? 4 : 2;  // the film jitter, and the lens sample
-                        uint64_t dims = camera_dims;
-                        if (in->kind == YK_INTEGRATOR_PATH) dims = camera_dims + (uint64_t)in->max_depth * (2ull * sc->dev.n_lights + 3);
-                        else if (in->kind == YK_INTEGRATOR_WHITTED)
-                            dims = camera_dims + 2ull * sc->dev.n_lights * ((1ull << std::min(in->max_depth, 8u)) - 1);
-                        dims = std::min<uint64_t>(dims, std::min<uint64_t>(4096, (256ull << 20) / (4ull * nj)));  // the rest is hashed on the fly
-                        if (p.hash_group != group || p.rehash) {
-                            const size_t need = (size_t)dims * nj;
-                            if (p.dim_hash_cap < need) {
-                                CUDA_TRY(cudaStreamSynchronize(p.stream));
-                                cudaFree(p.d_dim_hash);
-                                p.d_dim_hash = nullptr;
-                                p.dim_hash_cap = 0;
-                                CUDA_TRY(cudaMalloc((void**)&p.d_dim_hash, need * sizeof(uint32_t)));
-                                p.dim_hash_cap = need;
-                            }
-                            k_dim_hashes<<<dim3((nj + 255) / 256, (unsigned)std::min<uint64_t>(dims, 64)), 256, 0, p.stream>>>(
-                                p.d_jobs, nj, (uint32_t)dims, sm->seed, p.d_dim_hash);
-                            tm.launches += 1;
-                        }
-                        gcfg.sampler.hash_table = p.d_dim_hash;
-                        gcfg.sampler.n_hash_dims = (uint32_t)dims;
-                        gcfg.sampler.hash_stride = nj;
-                    }
-                    p.hash_group = group;
-                    p.rehash = false;
-                    Batch bt;
-                    bt.jobs = p.d_jobs;
-                    bt.n_jobs = nj;
-                    bt.div_jobs = FastDiv::make(nj);
-                    bt.sample_off = s0;
-                    bt.n_samples = s1 - s0;
-                    bt.n_paths = nj * bt.n_samples;
-                    // the batch's first sample index: s0, or the sample of the group's tiles (accumulating films: one per group)
-                    const uint32_t first_sample = accumulate ? (uint32_t)tiles[groups[group].t_lo].sample : s0;
-                    rc = run_batch(c, &p, sc, gcfg, bt, first_sample, accumulate, d_film, aov_sums, lens, &tm, &done);
-                    if (rc != YK_OK) {  // nothing may stay in flight or marked busy behind an error return
-                        cudaDeviceSynchronize();
-                        for (Pipe& q : c->pipe)
-                            for (auto& slot : q.slot) slot.busy = false;
-                        return rc;
-                    }
-                    if (adaptive) {
-                        const bool last = s1 >= samples_per_job;
-                        if (last || (s1 >= adaptive->min_samples && (s1 - adaptive->min_samples) % adaptive->step == 0)) {
-                            rc = adaptive_check(&p, nj, s1, last, *adaptive, fs->res_x, c->d_accum, aov_sums, adaptive_views, d_film, d_counts, &tm);
-                            if (rc != YK_OK) {
-                                cudaDeviceSynchronize();
-                                for (Pipe& q : c->pipe)
-                                    for (auto& slot : q.slot) slot.busy = false;
-                                return rc;
-                            }
-                        }
-                    } else if (!accumulate && s1 >= samples_per_job) {
-                        // the group's last samples are queued: `color /= sample_count` + Film::update_tile for its pixels
-                        k_film_store<<<(nj + 255) / 256, 256, 0, p.stream>>>(p.d_jobs, nj, c->d_accum, d_film, fs->res_x, (float)spp);
-                        tm.launches += 1;
-                        for (int k = 0; k < kAovViews; ++k) {
-                            if (!d_aov[k]) continue;
-                            k_film_store<<<(nj + 255) / 256, 256, 0, p.stream>>>(p.d_jobs, nj, aov_sums.v[k], d_aov[k], fs->res_x, (float)spp);
-                            tm.launches += 1;
-                        }
-                    }
-                    if (opts && opts->progress && opts->progress(opts->progress_user, done, total_paths)) cancelled = true;
-                }
-                if (!any) break;
-            }
-        }
-        for (int pi = 0; pi < n_pipes; ++pi) {
-            Pipe& p = c->pipe[pi];
-            CUDA_TRY(cudaMemcpyAsync(p.h_totals, p.wave.totals, sizeof(Totals), cudaMemcpyDeviceToHost, p.stream));
-            for (int k = 0; k < kRing; ++k)
-                if ((rc = retire_slot(&p, k, &tm, &done)) != YK_OK) return rc;
-            CUDA_TRY(cudaStreamSynchronize(p.stream));
-            const Totals& t = *p.h_totals;
-            totals.closest_nodes += t.closest_nodes; totals.closest_tris += t.closest_tris;
-            totals.any_nodes += t.any_nodes; totals.any_tris += t.any_tris;
-            totals.hit_hash += t.hit_hash; totals.shadow_rays += t.shadow_rays; totals.closest_rays += t.closest_rays;
+        if ((rc = run_groups(c, r, plan, &tm, &totals, &done, &cancelled)) != YK_OK) {
+            // nothing may stay in flight, or marked busy for the next render to retire, behind an error return
+            cudaDeviceSynchronize();
+            for (Pipe& q : c->pipe)
+                for (auto& slot : q.slot) slot.busy = false;
+            return rc;
         }
         if (cancelled) return yk_set_error(YK_ERR_CANCELLED, "yk_render: cancelled by the progress callback");
         // (adaptive: the samples taken, each pixel's count, of at most total_paths)
-        const uint64_t taken = adaptive ? done : total_paths;
+        const uint64_t taken = adaptive ? done : plan.total_paths;
         if (opts && opts->progress) opts->progress(opts->progress_user, taken, taken);
         st.samples = taken;
     }
     CUDA_TRY(cudaEventRecord(c->ev[3], s));
-    if (!on_device) {
-        CUDA_TRY(cudaMemcpyAsync(film_rgb, d_film, n_pixels * 3 * sizeof(float), cudaMemcpyDeviceToHost, s));
-        if (opts && opts->hit_ids)
-            CUDA_TRY(cudaMemcpyAsync(opts->hit_ids, d_ids, n_pixels * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
-        if (aovs) {
-            float* views[kAovViews];
-            aov_views(aovs, views);
-            for (int k = 0; k < kAovViews; ++k)
-                if (views[k]) CUDA_TRY(cudaMemcpyAsync(views[k], d_aov[k], n_pixels * 3 * sizeof(float), cudaMemcpyDeviceToHost, s));
-        }
-        if (d_counts) CUDA_TRY(cudaMemcpyAsync(adaptive->sample_counts, d_counts, n_pixels * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
-    }
+    if (!on_device && (rc = film_readback(out, r.dev, n_pixels, s)) != YK_OK) return rc;
     CUDA_TRY(cudaStreamSynchronize(s));
     CUDA_TRY(cudaGetLastError());
     if (stats) {
@@ -1768,7 +1811,7 @@ int query_run(yk_context* c, const yk_scene* sc, const QueryCall& q) {
         IterCounters ctr{};
         if (q.hits) ctr.n_active = m;
         else ctr.mat[0] = m;  // all segments in the first material queue's range of shading positions
-        CUDA_TRY(cudaMemcpyAsync(&p.d_ctr[0], &ctr, sizeof(ctr), cudaMemcpyHostToDevice, s));
+        CUDA_TRY(cudaMemcpyAsync(p.d_ctr.get(), &ctr, sizeof(ctr), cudaMemcpyHostToDevice, s));
         CUDA_TRY(cudaMemsetAsync(p.wave.totals, 0, sizeof(Totals), s));
         // where an output of this chunk goes: the caller's array itself, or the staging buffer it is copied back from
         auto out = [&](auto* caller, auto* staged, size_t per) -> decltype(caller) {
@@ -1783,8 +1826,8 @@ int query_run(yk_context* c, const yk_scene* sc, const QueryCall& q) {
         if (q.hits) {
             k_query_pack<<<(m + T - 1) / T, T, 0, s>>>(p.wave, o, d, tm, m, check_nan ? c->q_nan : nullptr);
             const int blocks = grid_for(m, kTraceThreads, c->sm_count * std::max(1, c->occ_trace_closest));
-            if (generic) k_trace_closest<true, true><<<blocks, kTraceThreads, 0, s>>>(sc->dev, p.wave, 0, &p.d_ctr[0], nullptr);
-            else k_trace_closest<true, false><<<blocks, kTraceThreads, 0, s>>>(sc->dev, p.wave, 0, &p.d_ctr[0], nullptr);
+            if (generic) k_trace_closest<true, true><<<blocks, kTraceThreads, 0, s>>>(sc->dev, p.wave, 0, p.d_ctr.get(), nullptr);
+            else k_trace_closest<true, false><<<blocks, kTraceThreads, 0, s>>>(sc->dev, p.wave, 0, p.d_ctr.get(), nullptr);
             if (h.t || h.orig_id || h.counts)
                 k_query_unpack<<<(m + T - 1) / T, T, 0, s>>>(sc->dev, p.wave, m, out(h.t, c->q_t, 1), out(h.orig_id, c->q_id, 1),
                                                              out(h.counts, c->q_cnt, 2));
@@ -1810,12 +1853,12 @@ int query_run(yk_context* c, const yk_scene* sc, const QueryCall& q) {
             const bool per_ray = c->shadow_mode != 0;  // one segment per lane either way; the per-ray kernel needs no fold
             if (per_ray) {
                 const int blocks = grid_for(m, kTraceThreads, c->sm_count * std::max(1, c->occ_trace_rays));
-                if (generic) k_trace_shadow_rays<true><<<blocks, kTraceThreads, 0, s>>>(sc->dev, p.wave, 1u, &p.d_ctr[0]);
-                else k_trace_shadow_rays<false><<<blocks, kTraceThreads, 0, s>>>(sc->dev, p.wave, 1u, &p.d_ctr[0]);
+                if (generic) k_trace_shadow_rays<true><<<blocks, kTraceThreads, 0, s>>>(sc->dev, p.wave, 1u, p.d_ctr.get());
+                else k_trace_shadow_rays<false><<<blocks, kTraceThreads, 0, s>>>(sc->dev, p.wave, 1u, p.d_ctr.get());
             } else {
                 const int blocks = grid_for(m, kTraceThreads, c->sm_count * std::max(1, c->occ_trace_any));
-                if (generic) k_trace_shadow<true><<<blocks, kTraceThreads, 0, s>>>(sc->dev, p.wave, cfg, &p.d_ctr[0]);
-                else k_trace_shadow<false><<<blocks, kTraceThreads, 0, s>>>(sc->dev, p.wave, cfg, &p.d_ctr[0]);
+                if (generic) k_trace_shadow<true><<<blocks, kTraceThreads, 0, s>>>(sc->dev, p.wave, cfg, p.d_ctr.get());
+                else k_trace_shadow<false><<<blocks, kTraceThreads, 0, s>>>(sc->dev, p.wave, cfg, p.d_ctr.get());
             }
             k_query_unpack_segments<<<(m + T - 1) / T, T, 0, s>>>(p.wave, m, per_ray ? 1 : 0, out(q.occluded, c->q_occ, 1));
             if ((rc = back(q.occluded, c->q_occ, 1)) != YK_OK) return rc;
